@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json's metric for the NUBOMEDIA-VCA detection hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 3, "Full-resolution 1920x1080 face detection (processing
 width 1920, min window 24x24, scale 1.1)" — the configuration the metric's first half ("1080p face-cascade
@@ -425,6 +425,8 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-aux", action="store_true", help="skip the cfg5 720p-streams auxiliary measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rectangles of the last timed step, one DIR/faces_frame<i>.npy "
+                                                           "(float64, rows x y w h) per frame of rank 0's batch")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -528,6 +530,10 @@ def main():
     barrier()
     clocks = sampler.stop()                       # sampled across both timed regions
     assert all((a == b).all() for a, b in zip(out_d, out))
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for i, o in enumerate(out):
+            np.save(os.path.join(args.dump_outputs, f"faces_frame{i}.npy"), np.asarray(o, np.float64).reshape(-1, 4))
     # (a) the GPU's rectangles for this rank's frames against the CPU arm's (cv2, the reference's call sequence) in this run
     parity = None
     if rank == 0:

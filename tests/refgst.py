@@ -7,13 +7,37 @@
 
 Test infrastructure only."""
 import ctypes as C
+import hashlib
+import json
 import os
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 FACTORIES = ["nubofacedetector", "nuboeyedetector", "nubomouthdetector", "nubonosedetector", "nuboeardetector", "nubotracker"]
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+
+
+def load_golden(name):
+    """What the reference elements answered in a test, as tests/golden/make_ref_golden.py recorded it."""
+    with open(os.path.join(GOLDEN_DIR, name)) as f:
+        return json.load(f)
+
+
+GOLDEN = load_golden("ref_elements.json") if os.path.exists(os.path.join(GOLDEN_DIR, "ref_elements.json")) else {}
+
+
+def plain(x):
+    """x as it reads back from JSON (tuples become lists)."""
+    return json.loads(json.dumps(x))
+
+
+def frame_digest(frame):
+    """First 16 hex digits of the SHA-256 of a frame's pixels: how the recorded answers hold the frames an element drew into."""
+    return hashlib.sha256(np.ascontiguousarray(frame).tobytes()).hexdigest()[:16]
 FMT = {"BGR": 0, "BGRA": 1, "I420": 2, "NV12": 3}
 
 

@@ -1,5 +1,6 @@
-"""Randomised element-level parity run against the REFERENCE'S OWN ELEMENTS (oracle/_ref/libnubo_ref_elements.so: the six
-kms*detect.cpp / gstnubotracker.cpp sources compiled unmodified, computing through the CPU oracle):
+"""Randomised element-level parity run against what the REFERENCE'S OWN ELEMENTS (the six kms*detect.cpp /
+gstnubotracker.cpp sources compiled unmodified by oracle/build_ref.py, computing through the CPU oracle) answered on the
+same sequences, recorded in tests/golden/ref_elements_gpu.json:
 
   target "mirror": the nv_element C ABI of libnubovca.so (CUDA),
   target "shell":  this repo's GStreamer shells (nubomedia-vca_b200/gst/) built against the mock GStreamer, driven through
@@ -7,11 +8,11 @@ kms*detect.cpp / gstnubotracker.cpp sources compiled unmodified, computing throu
 
 Random frame sizes, face layouts, stand-in feature models, property values (including out-of-range ones, view-*,
 detect-event with random upstream event streams — face messages, motion messages, foreign messages, messages without a
-timestamp —, activate-events / events-ms under an injected wall clock), frame sequences with noise and empty frames.
-Compared per frame: the pushed downstream event (structure name, timestamp, every sub-structure field by field), the
-emitted signal payload, and the frame's pixels after the element drew into it (the reference's recorded cvRectangle /
-cv::circle calls replayed with the real cv2).  Needs a CUDA device.
-Usage: python tools/fuzz_ref_elements.py [seconds] [seed] [mirror|shell|both]"""
+timestamp —, activate-events / events-ms under an injected wall clock), frame sequences with noise and empty frames, all
+drawn from the recorded seed.  Compared per frame: the pushed downstream event (structure name, timestamp, every
+sub-structure field by field), the emitted signal payload, and a digest of the frame's pixels after the element drew into
+it.  Needs a CUDA device.
+Usage: python tools/fuzz_ref_elements.py [mirror|shell|both]"""
 import os
 import shutil
 import sys
@@ -110,11 +111,13 @@ class ShellTarget:
         self.e.close()
 
 
-def run(budget, seed, targets):
+def run(nseq, seed, targets, expected=None):
+    """nseq random sequences from `seed` through `targets`.  With `expected` (the recorded sequences) every target is compared
+    with it; without, the first target's answers are returned as the record."""
     rng = np.random.default_rng(seed)
-    R = refgst.ref()
     t0 = time.time()
-    stats = dict(sequences=0, frames=0, rects=0, signals=0, drawn_frames=0, ref_threw=0, events_sent=0, rejected_sets=0, mismatches=0)
+    stats = dict(sequences=0, frames=0, rects=0, signals=0, drawn_frames=0, events_sent=0, rejected_sets=0, mismatches=0)
+    record = []
     # ONE set of stand-in models per process: the reference's nose element keeps its cascades in file-static objects that
     # only the first instance loads (kmsnosedetect.cpp:151-152,1049-1051), so the models cannot change between sequences
     d = tempfile.mkdtemp(prefix="nubovca_fzr_")
@@ -123,10 +126,11 @@ def run(budget, seed, targets):
     for name, (w, h) in STANDINS.items():
         permissive_cascade(os.path.join(d, name), np.random.default_rng(int(rng.integers(1 << 30))), w, h,
                            bias=float(rng.choice([0.2, 0.35, 0.5])))
-    R.register_cascade_dir(d)
-    while time.time() - t0 < budget:
+    for q in range(nseq):
         els = []
-        ref = None
+        exp = expected[q] if expected is not None else None
+        rec = {"sets": [], "gets": [], "frames": []}
+        record.append(rec)
         try:
             factory = refgst.FACTORIES[int(rng.integers(6))]
             trk = factory == "nubotracker"
@@ -141,7 +145,6 @@ def run(budget, seed, targets):
                         frames.append(np.full((H, W, 3), 90, np.uint8))
                     else:
                         frames.append(np.clip(base.astype(np.int16) + rng.integers(-3, 4, base.shape, dtype=np.int16), 0, 255).astype(np.uint8))
-            ref = R.element(factory)
             els = [t(factory, d) for t in targets]
             props = {}
             if trk:
@@ -157,15 +160,18 @@ def run(budget, seed, targets):
             props["activate-events"] = int(rng.choice([0, 1, 1]))
             props["events-ms"] = int(rng.choice([0, 50, 1000]))
             wall = 1e12
-            R.set_time(0, wall)
             nv._lib.nv_debug_set_wall_clock_ms(wall)
             for k, v in props.items():
-                oks = [ref.set(k, v)] + [e.set(k, v) for e in els]
+                oks = [e.set(k, v) for e in els]
                 assert len(set(oks)) == 1, (factory, k, v, oks)
+                rec["sets"].append(oks[0])
                 stats["rejected_sets"] += not oks[0]
             for k in props:
-                vals = [ref.get(k)] + [e.get(k) for e in els]
+                vals = [e.get(k) for e in els]
                 assert len(set(vals)) == 1, (factory, k, vals)
+                rec["gets"].append(vals[0])
+            if exp is not None:
+                assert (rec["sets"], rec["gets"]) == (exp["sets"], exp["gets"]), (factory, props, rec, exp)
             for i, f in enumerate(frames):
                 pts = i * 33_333_000
                 wall += float(rng.choice([5, 40, 700]))
@@ -174,61 +180,53 @@ def run(budget, seed, targets):
                         kind = str(rng.choice(["faces", "faces", "motion", "other"]))
                         ts = bool(rng.random() < 0.85)
                         faces = [(int(rng.integers(0, W - 80)), int(rng.integers(0, H - 80)), int(s), int(s)) for s in rng.integers(40, min(H, 260), int(rng.integers(0, 3)))]
-                        if kind == "faces":
-                            ref.send_event(R.faces_message(faces, timestamp=ts))
-                        elif kind == "motion":
-                            ref.send_event(R.motion_message(timestamp=ts))
-                        else:
-                            ref.send_event(R.structure("message", ([("timestamp", "struct", R.structure("time", [("pts", "uint64", 0)]))] if ts else []) +
-                                                       [("x", "struct", R.structure("thing", [("type", "string", "thing")]))]))
                         for e in els:
                             e.event(kind, faces, ts)
                         stats["events_sent"] += 1
-                R.set_time(pts / 1e6, wall)
-                fr = f.copy()
-                threw, events, sig = ref.process(fr, pts_ns=pts, fmt="BGRA" if trk else "BGR")
-                if threw:                            # ROI outside the image: cv::Mat::operator() throws in the reference (streaming thread dies);
-                    stats["ref_threw"] += 1          # the replacement clamps instead (documented) — nothing to compare from here on
-                    break
-                assert len(events) <= 1 and (fr == f).all()
-                exp_msg = exp_event = None
-                if events:
-                    name, epts, rows = exp_event = events[0]
-                    assert [r[0] for r in rows] == [str(j) for j in range(len(rows))]
-                    assert (name, epts) == (("noses", 2 ** 64 - 1) if factory == "nubonosedetector" else ("message", pts))
-                    exp_msg = [tuple(r[1:]) for r in rows]
-                exp_sig = sig[0][1] if sig else None
-                exp_frame = refgst.replay_draws(f.copy(), ref.draws(fr))
-                stats["frames"] += 1
-                stats["rects"] += len(exp_msg or [])
-                stats["signals"] += exp_sig is not None
-                stats["drawn_frames"] += bool((exp_frame != f).any())
+                outs = []
                 for e in els:
                     g = f.copy()
                     msg, s = e.process(g, pts, wall)
+                    outs.append((e, refgst.plain(msg), s, refgst.frame_digest(g), int((g != f).any(axis=-1).sum())))
+                if exp is None:
+                    _, event, sig, pixels, drawn = outs[0]
+                    rec["frames"].append({"event": event, "signal": sig, "pixels": pixels, "drawn": drawn})
+                    continue
+                x = exp["frames"][i]
+                exp_event, exp_sig = x["event"], x["signal"]
+                exp_msg = None
+                if exp_event is not None:
+                    name, epts, rows = exp_event
+                    assert [r[0] for r in rows] == [str(j) for j in range(len(rows))]
+                    assert (name, epts) == (("noses", 2 ** 64 - 1) if factory == "nubonosedetector" else ("message", pts))
+                    exp_msg = [r[1:] for r in rows]
+                stats["frames"] += 1
+                stats["rects"] += len(exp_msg or [])
+                stats["signals"] += exp_sig is not None
+                stats["drawn_frames"] += bool(x["drawn"])
+                for e, msg, s, pixels, drawn in outs:
                     if e.name == "mirror" and (trk or factory == "nuboeardetector"):
                         msg = None                   # the mirror reports the message it built; neither element pushes one
-                    if msg != (exp_event if e.name == "shell" else exp_msg) or s != exp_sig or not (g == exp_frame).all():
+                    if msg != (exp_event if e.name == "shell" else exp_msg) or s != exp_sig or pixels != x["pixels"]:
                         stats["mismatches"] += 1
-                        print("MISMATCH", e.name, factory, (W, H), props, "frame", i, "\n  msg", msg, "\n  exp", exp_msg, "\n  sig", s, "\n  exp", exp_sig,
-                              "\n  pixels differ:", int((g != exp_frame).sum()), flush=True)
+                        print("MISMATCH", e.name, factory, (W, H), props, "sequence", q, "frame", i, "\n  msg", msg, "\n  exp", exp_msg,
+                              "\n  sig", s, "\n  exp", exp_sig, "\n  drawn pixels", drawn, "expected", x["drawn"], flush=True)
                         raise StopIteration
             stats["sequences"] += 1
         except StopIteration:
             pass
         finally:
-            for e in els + ([ref] if ref else []):
+            for e in els:
                 e.close()
     shutil.rmtree(d, ignore_errors=True)
     nv._lib.nv_debug_set_wall_clock_ms(-1.0)
-    return stats, time.time() - t0
+    return stats, time.time() - t0, record
 
 
 if __name__ == "__main__":
-    budget = float(sys.argv[1]) if len(sys.argv) > 1 else 60.0
-    seed = int(sys.argv[2]) if len(sys.argv) > 2 else 0
-    which = sys.argv[3] if len(sys.argv) > 3 else "mirror"
+    which = sys.argv[1] if len(sys.argv) > 1 else "both"
     targets = {"mirror": [MirrorTarget], "shell": [ShellTarget], "both": [MirrorTarget, ShellTarget]}[which]
-    stats, dt = run(budget, seed, targets)
-    print(f"fuzz_ref_elements[{which}]: " + ", ".join(f"{v} {k}" for k, v in stats.items()) + f", seed {seed}, {dt:.0f} s")
-    sys.exit(1 if stats["mismatches"] else 0)
+    golden = refgst.load_golden("ref_elements_gpu.json")["fuzz"]
+    stats, dt, _ = run(len(golden["sequences"]), golden["seed"], targets, golden["sequences"])
+    print(f"fuzz_ref_elements[{which}]: " + ", ".join(f"{v} {k}" for k, v in stats.items()) + f", seed {golden['seed']}, {dt:.0f} s")
+    sys.exit(1 if stats["mismatches"] or stats["sequences"] < len(golden["sequences"]) else 0)
