@@ -95,6 +95,21 @@ typedef struct {
 NV_API int nv_detect_multiscale(nv_ctx *ctx, const nv_cascade *c, const uint8_t *gray, int width, int height,
                                 int stride_bytes, const nv_detect_params *p, nv_rect *out, int cap, int *n);
 
+/* ---- detection scores: cv::CascadeClassifier::detectMultiScale2 / detectMultiScale3 (OpenCV 4.13).
+ *      on != 0: every detect call on this ctx (nv_detect_multiscale, nv_face_detect / _submit / _submit_device /
+ *      _detect_yuv / _submit_yuv) also yields, per output rectangle, detectMultiScale2's numDetections and
+ *      detectMultiScale3(outputRejectLevels = true)'s levelWeights:
+ *        - min_neighbors > 0: numDetections is the number of raw windows grouped into the rectangle (the count compared
+ *          with min_neighbors), levelWeight the largest last-stage sum among them;
+ *        - min_neighbors <= 0: numDetections is 1, levelWeight the window's own last-stage sum.
+ *      A window's last-stage sum is the double sum of its last stage's leaves in XML order, which is at or above that
+ *      stage's threshold.  detectMultiScale3's rejectLevels is always the cascade's stage count and is not returned.
+ *      The setting applies from the next submit; a ctx keeps separate graphs for both settings.  Rectangles do not change. */
+NV_API int nv_ctx_set_scores(nv_ctx *ctx, int on);
+/* Scores of the last collected call, parallel to its rectangles (same order, same clip); either output may be NULL.
+ * NV_ERR_STATE if that call ran with scores off; NV_ERR_CAPACITY (and the first cap entries) if cap is too small. */
+NV_API int nv_get_scores(nv_ctx *ctx, int *neighbors, double *level_weights, int cap, int *n);
+
 /* ---- the nubofacedetector hot block, kmsfacedetect.cpp:770-811:
  *      scale = width / width_to_process (integer), cv::resize(BGR, INTER_LINEAR), BGR2GRAY,
  *      equalizeHist, detectMultiScale(scale_factor, min_neighbors, 0, Size(min_w, min_h)).

@@ -235,23 +235,27 @@ static int ensure(T **p, size_t *cap, size_t need, bool zero = false)
     return NV_OK;
 }
 
-// candidate-side buffers: ids, sorted ids, rects, similarity bit-matrix (+ group scratch), result block
+// candidate-side buffers: ids, sorted ids, rects, weights, similarity bit-matrix (+ group scratch), result block
 static int alloc_candidates(nv_ctx *c, int cap, bool with_adj)
 {
     cudaFree(c->d_cand); cudaFree(c->d_cand_sorted); cudaFree(c->d_cand_rects); cudaFree(c->d_adj); cudaFree(c->d_result);
+    cudaFree(c->d_cand_w); cudaFree(c->d_cls_wmax);
     cudaFreeHost(c->h_result);
     c->d_cand = c->d_cand_sorted = nullptr; c->d_cand_rects = nullptr; c->d_adj = nullptr; c->d_result = c->h_result = nullptr;
+    c->d_cand_w = nullptr; c->d_cls_wmax = nullptr;
     c->cand_cap = cap; c->result_cap = cap; c->adj_cap = 0; c->epoch++;
     NV_CUDA(cudaMalloc(&c->d_cand, (size_t)cap * sizeof(uint32_t)));
     NV_CUDA(cudaMalloc(&c->d_cand_sorted, (size_t)cap * sizeof(uint32_t)));
     NV_CUDA(cudaMalloc(&c->d_cand_rects, (size_t)cap * sizeof(int4)));
+    NV_CUDA(cudaMalloc(&c->d_cand_w, (size_t)cap * sizeof(double)));
+    NV_CUDA(cudaMalloc(&c->d_cls_wmax, (size_t)cap * sizeof(unsigned long long)));
     // the similarity bit-matrix only serves frames with at most NV_GROUP_UF_MIN candidates (kernels_group.cu)
     const size_t acap = std::min<size_t>((size_t)cap, NV_GROUP_UF_MIN);
     size_t adj_words = (with_adj ? acap * ((acap + 31) / 32) : 0) + 8 * (size_t)cap;
     NV_CUDA(cudaMalloc(&c->d_adj, adj_words * sizeof(uint32_t)));
     c->adj_cap = with_adj ? cap : 0;
     c->d_grp = reinterpret_cast<int *>(c->d_adj + (adj_words - 8 * (size_t)cap));
-    size_t rbytes = sizeof(ResultHeader) + (size_t)c->result_cap * sizeof(nv_rect);
+    size_t rbytes = sizeof(ResultHeader) + (size_t)c->result_cap * (sizeof(nv_rect) + sizeof(double) + sizeof(int));
     NV_CUDA(cudaMalloc(&c->d_result, rbytes));
     NV_CUDA(cudaMallocHost(&c->h_result, rbytes));
     memset(c->h_result, 0, sizeof(ResultHeader));
@@ -321,6 +325,7 @@ extern "C" void nv_ctx_destroy(nv_ctx *c)
     cudaFree(c->d_sq); cudaFree(c->d_pyr); cudaFree(c->d_tilt); cudaFree(c->d_vnf); cudaFree(c->d_depth);
     cudaFree(c->d_bits_ok); cudaFree(c->d_queue); cudaFree(c->d_queue2); cudaFree(c->d_deepq); cudaFree(c->d_counters); cudaFree(c->d_cand);
     cudaFree(c->d_cand_sorted); cudaFree(c->d_cand_rects); cudaFree(c->d_adj); cudaFree(c->d_result);
+    cudaFree(c->d_cand_w); cudaFree(c->d_cls_wmax);
     cudaFreeHost(c->h_result);
     cudaFree(c->d_trk_prev); cudaFree(c->d_trk_hist); cudaFree(c->d_trk_scratch); cudaFreeHost(c->h_trk);
     if (c->gexec) cudaGraphExecDestroy(c->gexec);
@@ -331,6 +336,28 @@ extern "C" void nv_ctx_destroy(nv_ctx *c)
     if (c->stream) cudaStreamDestroy(c->stream);
     cudaGetLastError();
     delete c;
+}
+
+extern "C" int nv_ctx_set_scores(nv_ctx *ctx, int on)
+{
+    if (!ctx) { nv_set_error("null ctx"); return NV_ERR_ARG; }
+    ctx->scores = on ? 1 : 0;
+    return NV_OK;
+}
+
+// scores of the last collected call, parallel to its rectangles (result block: rects | weights | neighbour counts)
+extern "C" int nv_get_scores(nv_ctx *ctx, int *neighbors, double *level_weights, int cap, int *n)
+{
+    if (!ctx) { nv_set_error("null ctx"); return NV_ERR_ARG; }
+    if (!ctx->scores_ready) { nv_set_error("no collected call with scores on"); return NV_ERR_STATE; }
+    const int total = reinterpret_cast<const ResultHeader *>(ctx->h_result)->n_out, m = std::min(total, std::max(cap, 0));
+    const uint8_t *w = ctx->h_result + sizeof(ResultHeader) + (size_t)ctx->result_cap * sizeof(nv_rect);
+    const uint8_t *nb = w + (size_t)ctx->result_cap * sizeof(double);
+    if (level_weights && m > 0) memcpy(level_weights, w, (size_t)m * sizeof(double));
+    if (neighbors && m > 0) memcpy(neighbors, nb, (size_t)m * sizeof(int));
+    if (n) *n = m;
+    if (total > cap) { nv_set_error("%d rectangles, caller capacity %d", total, cap); return NV_ERR_CAPACITY; }
+    return NV_OK;
 }
 
 extern "C" int nv_ctx_set_debug(nv_ctx *ctx, int debug)
@@ -871,16 +898,25 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
     // small plans: sort + similarity matrix + grouping in one launch of one block (k_group_fused)
     static const bool group_fused = [] { const char *e = getenv("NUBOVCA_GROUP_FUSED"); return !e || atoi(e) != 0; }();
     static const int small_limit_g = [] { const char *e = getenv("NUBOVCA_SMALL_PLAN"); return e ? atoi(e) : NV_SMALL_PLAN_WINDOWS; }();
+    const ScoreArgs sa = {ctx->cur_meta, ctx->cur_stumps, ctx->use_gen ? ctx->cur_gen : GenModel{}, ctx->use_gen ? 1 : 0, ctx->d_sum, ctx->d_sq,
+                          ctx->use_gen && ctx->cur_tilted ? ctx->d_tilt : nullptr, ctx->d_cand_w, ctx->d_cls_wmax};
     NV_CUDA(launch_group(ctx->ps->d_plan, ctx->d_counters, ctx->d_cand, ctx->cand_cap, ctx->d_cand_sorted, ctx->d_cand_rects,
                          ctx->d_adj, ctx->d_grp, p->min_neighbors, 0.2, W, H, ctx->d_result, ctx->result_cap, 148 * 2, st, &nl,
-                         group_fused && P.total_windows <= small_limit_g, host_writes ? ctx->h_result : nullptr));
+                         group_fused && P.total_windows <= small_limit_g, host_writes ? ctx->h_result : nullptr,
+                         ctx->scores ? &sa : nullptr));
     prof_mark(ctx, 8);
     // the grouping kernel writes header and rectangles into the page-locked result block itself (mapped memory, posted
     // writes over PCIe, visible once the stream has been waited for): no device-to-host copy behind it.
     // NUBOVCA_HOST_WRITES=0: the copy (what every call did before).
-    if (!host_writes)
+    if (!host_writes) {
         NV_CUDA(cudaMemcpyAsync(ctx->h_result, ctx->d_result, sizeof(ResultHeader) + NV_RESULT_INLINE * sizeof(nv_rect),
                                 cudaMemcpyDeviceToHost, st));
+        if (ctx->scores) {
+            const size_t wofs = sizeof(ResultHeader) + (size_t)ctx->result_cap * sizeof(nv_rect), nofs = wofs + (size_t)ctx->result_cap * sizeof(double);
+            NV_CUDA(cudaMemcpyAsync(ctx->h_result + wofs, ctx->d_result + wofs, NV_RESULT_INLINE * sizeof(double), cudaMemcpyDeviceToHost, st));
+            NV_CUDA(cudaMemcpyAsync(ctx->h_result + nofs, ctx->d_result + nofs, NV_RESULT_INLINE * sizeof(int), cudaMemcpyDeviceToHost, st));
+        }
+    }
     *nlaunch += nl;
     counters_guard.done = true;
     return NV_OK;
@@ -892,6 +928,7 @@ static void detect_bookkeeping(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_g
     ctx->last_min_neighbors = p->min_neighbors;
     ctx->last_casc = casc; ctx->last_params = *p; ctx->last_W = W; ctx->last_H = H;
     ctx->tap_gray = d_gray; ctx->tap_lut = d_lut; ctx->tap_stride = gstride;
+    ctx->last_scores = ctx->scores != 0; ctx->scores_ready = false;
     ctx->pending = true;
 }
 
@@ -906,7 +943,7 @@ int nv_detect_device(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, int W
     PlanSlot *sl = ctx->ps;
     DetGraphKey key;
     key.gray = d_gray; key.gstride = gstride; key.lut = d_lut; key.casc = casc->uid; key.sf = p->scale_factor; key.mn = p->min_neighbors;
-    key.epoch = ctx->epoch;
+    key.epoch = ctx->epoch; key.scores = ctx->scores;
     bool graphable = !ctx->debug && !ctx->profile && !ctx->no_graph;
     int nl = 0;
     if (graphable && sl->dexec && key == sl->dkey) {
@@ -956,7 +993,10 @@ int nv_collect(nv_ctx *ctx, nv_rect *out, int cap, int *n)
         int rc = alloc_candidates(ctx, std::min(lim, need + need / 4 + 64), ctx->last_min_neighbors > 0);
         if (rc != NV_OK) return rc;
         nv_detect_params p = ctx->last_params;
+        const int scores = ctx->scores;
+        ctx->scores = ctx->last_scores;                      // the call as it was submitted
         rc = nv_detect_device(ctx, ctx->last_casc, ctx->tap_gray, ctx->last_W, ctx->last_H, ctx->tap_stride, ctx->tap_lut, &p);
+        ctx->scores = scores;
         if (rc != NV_OK) return rc;
         NV_CUDA(cudaStreamSynchronize(ctx->stream));
         ctx->pending = false;
@@ -967,7 +1007,15 @@ int nv_collect(nv_ctx *ctx, nv_rect *out, int cap, int *n)
         NV_CUDA(cudaMemcpy(ctx->h_result + sizeof(ResultHeader) + NV_RESULT_INLINE * sizeof(nv_rect),
                            ctx->d_result + sizeof(ResultHeader) + NV_RESULT_INLINE * sizeof(nv_rect),
                            (size_t)(total - NV_RESULT_INLINE) * sizeof(nv_rect), cudaMemcpyDeviceToHost));
+        if (ctx->last_scores) {
+            const size_t wofs = sizeof(ResultHeader) + (size_t)ctx->result_cap * sizeof(nv_rect), nofs = wofs + (size_t)ctx->result_cap * sizeof(double);
+            NV_CUDA(cudaMemcpy(ctx->h_result + wofs + NV_RESULT_INLINE * sizeof(double), ctx->d_result + wofs + NV_RESULT_INLINE * sizeof(double),
+                               (size_t)(total - NV_RESULT_INLINE) * sizeof(double), cudaMemcpyDeviceToHost));
+            NV_CUDA(cudaMemcpy(ctx->h_result + nofs + NV_RESULT_INLINE * sizeof(int), ctx->d_result + nofs + NV_RESULT_INLINE * sizeof(int),
+                               (size_t)(total - NV_RESULT_INLINE) * sizeof(int), cudaMemcpyDeviceToHost));
+        }
     }
+    ctx->scores_ready = ctx->last_scores;
     int m = std::min(total, cap);
     if (out && m > 0) memcpy(out, ctx->h_result + sizeof(ResultHeader), (size_t)m * sizeof(nv_rect));
     if (n) *n = m;
@@ -1206,7 +1254,8 @@ static int face_submit_impl(nv_ctx *ctx, const nv_cascade *c, const FaceSrc &src
     // state of an element); debug / profiling runs keep individual launches so that their events and taps work.
     nv_ctx::GraphKey key = {d_src, width, height, stride, cols, rows, d_rtab, casc->uid, dp.scale_factor, dp.min_neighbors,
                             dp.min_w, dp.min_h, ctx->epoch, ctx->ps, ctx->ps->gen,
-                            src.fmt, yuv ? planes.p1 : nullptr, yuv ? planes.p2 : nullptr, yuv ? planes.s1 : 0, yuv ? planes.s2 : 0};
+                            src.fmt, yuv ? planes.p1 : nullptr, yuv ? planes.p2 : nullptr, yuv ? planes.s1 : 0, yuv ? planes.s2 : 0,
+                            ctx->scores};
     bool graphable = !ctx->debug && !ctx->no_graph;
     int nl = 0;
     if (graphable && ctx->gexec && key == ctx->gkey) {

@@ -265,7 +265,8 @@ struct Stage0Params {
 };
 static_assert(sizeof(Stage0Params) <= 32000, "kernel parameter space is 32764 bytes");
 
-// header of the device result block (then rects follow)
+// header of the device result block; then rects[result_cap], level weights (double)[result_cap], neighbour counts
+// (int)[result_cap] — the last two are written by calls with scores on only
 struct ResultHeader {
     int n_out;          // rects written after grouping + clipping
     int n_cand;         // raw candidates (before the cap)
@@ -278,9 +279,10 @@ struct ResultHeader {
 // frame, and re-deriving + re-uploading a plan costs more than the detection itself on such small images.
 struct DetGraphKey {
     const void *gray = nullptr; int gstride = 0; const void *lut = nullptr; unsigned long long casc = 0;     // nv_cascade::uid
-    double sf = 0; int mn = 0; unsigned long long epoch = 0;
+    double sf = 0; int mn = 0; unsigned long long epoch = 0; int scores = 0;
     bool operator==(const DetGraphKey &o) const {
-        return gray == o.gray && gstride == o.gstride && lut == o.lut && casc == o.casc && sf == o.sf && mn == o.mn && epoch == o.epoch;
+        return gray == o.gray && gstride == o.gstride && lut == o.lut && casc == o.casc && sf == o.sf && mn == o.mn && epoch == o.epoch &&
+               scores == o.scores;
     }
 };
 struct PlanSlot {
@@ -340,8 +342,11 @@ struct nv_ctx {
     uint32_t *d_cand_sorted = nullptr;
     int4 *d_cand_rects = nullptr;
     uint32_t *d_adj = nullptr;   size_t adj_cap = 0;  int *d_grp = nullptr;   // similarity bit-matrix, group scratch
-    uint8_t *d_result = nullptr; uint8_t *h_result = nullptr;   // ResultHeader + rects
+    uint8_t *d_result = nullptr; uint8_t *h_result = nullptr;   // ResultHeader + rects (+ scores)
     int result_cap = 0;                                     // rects
+    // detection scores (nv_ctx_set_scores): last-stage sum per sorted candidate, per-class maximum (order-preserving uint64)
+    int scores = 0;  bool last_scores = false, scores_ready = false;
+    double *d_cand_w = nullptr;  unsigned long long *d_cls_wmax = nullptr;
 
     // CUDA graph of the steady-state face pipeline (one launch per frame once a call shape repeats)
     struct GraphKey {
@@ -349,8 +354,9 @@ struct nv_ctx {
         unsigned long long casc = 0; double sf = 0; int mn = 0, min_w = 0, min_h = 0; unsigned long long epoch = 0;
         const PlanSlot *slot = nullptr; unsigned long long slot_gen = 0;
         int fmt = 0; const void *p1 = nullptr, *p2 = nullptr; int s1 = 0, s2 = 0;      // 4:2:0 input: chroma planes
+        int scores = 0;
         bool operator==(const GraphKey &o) const {
-            return fmt == o.fmt && p1 == o.p1 && p2 == o.p2 && s1 == o.s1 && s2 == o.s2 && src == o.src && w == o.w && h == o.h && stride == o.stride && cols == o.cols && rows == o.rows &&
+            return scores == o.scores && fmt == o.fmt && p1 == o.p1 && p2 == o.p2 && s1 == o.s1 && s2 == o.s2 && src == o.src && w == o.w && h == o.h && stride == o.stride && cols == o.cols && rows == o.rows &&
                    rtab == o.rtab && casc == o.casc && sf == o.sf && mn == o.mn && min_w == o.min_w && min_h == o.min_h &&
                    epoch == o.epoch && slot == o.slot && slot_gen == o.slot_gen;
         }
@@ -470,9 +476,21 @@ int nv_h2d(nv_ctx *ctx, const uint8_t *src, size_t bytes);
 int nv_get_rtab(nv_ctx *ctx, int sw, int sh, int dw, int dh, const int **d_tab, const nv_ctx::RtabEntry **entry = nullptr);
 
 // kernels_group.cu
+// What the candidate sort needs to evaluate each candidate's last stage (detectMultiScale3's levelWeights) and what the
+// grouping needs to pass the scores on.  w == nullptr: scores off.
+struct ScoreArgs {
+    const DevCascade *meta;
+    const DevStump *stumps;       // stump cascades (general == 0)
+    GenModel g;                   // general cascades; g.subset != nullptr: LBP (no variance factor)
+    int general;
+    const uint32_t *sum, *sq, *tilt;
+    double *w;                    // [cand_cap] weight of the candidate of rank i
+    unsigned long long *cls_wmax; // [cand_cap] per class: maximum member weight, order-preserving map
+};
 cudaError_t launch_group(const PlanDev *plan, int *counters, const uint32_t *cand, int cand_cap, uint32_t *cand_sorted,
                          int4 *cand_rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h,
-                         uint8_t *result, int result_cap, int nblocks, cudaStream_t st, int *nlaunch, bool fused = false, uint8_t *host_result = nullptr);
+                         uint8_t *result, int result_cap, int nblocks, cudaStream_t st, int *nlaunch, bool fused = false, uint8_t *host_result = nullptr,
+                         const ScoreArgs *scores = nullptr);
 
 // kernels_tracker.cu
 size_t tracker_scratch_bytes(int w, int h, TrkLayout *lo);

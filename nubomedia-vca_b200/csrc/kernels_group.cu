@@ -14,7 +14,14 @@
 // 2 delta, i.e. sit on a few neighbouring levels, and in rows within delta — and links them with a lock-free union-find
 // whose root is the smallest index (uf_link inside k_adj, many blocks).  Same components, same labels (first member), so the rest
 // of k_group is shared.
-#include "internal.h"
+//
+// Scores (SCORES = true, nv_ctx_set_scores): the warp that ranks a candidate also evaluates the candidate's LAST stage —
+// detectMultiScale3's levelWeights is that stage's sum — and the grouping passes on, per output rectangle, the class size
+// (detectMultiScale2's numDetections) and the largest member weight.  The bulk cascade kernels keep no stage sums, so the
+// stage is evaluated again here, in the reference's arithmetic whatever kernel produced the candidate: the variance
+// factor as in stage 0, one lane per weak classifier, and the double sum formed in XML order by one shuffle per
+// classifier, so it is exact for every cascade without the order-free certificate.
+#include "cascade_eval.cuh"
 
 
 #define GROUP_SMEM_LABELS NV_GROUP_UF_MIN      // the matrix path keeps its labels in shared memory
@@ -26,9 +33,55 @@ __device__ __forceinline__ bool similar_rects(const int4 &a, const int4 &b, doub
            (double)abs(a.x + a.z - b.x - b.z) <= delta && (double)abs(a.y + a.w - b.y - b.w) <= delta;
 }
 
+// sum of the last stage at candidate `key`, evaluated by the whole warp (every lane returns it)
+__device__ __forceinline__ double last_stage_weight(const ScoreArgs &sa, const PlanDev *__restrict__ plan, uint32_t key, int lane)
+{
+    const int l = key >> 26, iy = (key >> 13) & 8191, ix = key & 8191;
+    const LevelDesc &L = plan->lv[l];
+    LevelView v{sa.sum + L.iofs, L.ipitch, L.iplane, L.ystep};
+    const size_t rowbase = (size_t)iy * L.ystep * L.ipitch;
+    const uint32_t *wb = v.sum + rowbase + ix;
+    float vnf = 0.f;
+    if (!sa.g.subset) {                                           // Haar: the variance factor exactly as stage 0 forms it
+        const int ww = plan->win_w, wh = plan->win_h;
+        const int c00 = corner(v, 1, 1), c10 = corner(v, ww - 1, 1), c01 = corner(v, 1, wh - 1), c11 = corner(v, ww - 1, wh - 1);
+        const uint32_t *qb = sa.sq + L.iofs + rowbase + ix;
+        const double area = (double)((ww - 2) * (wh - 2));
+        const int valsum = (int)(__ldg(wb + c00) - __ldg(wb + c10) - __ldg(wb + c01) + __ldg(wb + c11));
+        const uint32_t valsq = __ldg(qb + c00) - __ldg(qb + c10) - __ldg(qb + c01) + __ldg(qb + c11);
+        const double nf = __dsub_rn(__dmul_rn(area, (double)valsq), __dmul_rn((double)valsum, (double)valsum));
+        vnf = __double2float_rn(__ddiv_rn(1.0, __dsqrt_rn(nf)));  // nf > 0: the candidate passed the variance test
+    }
+    const uint32_t *tb = sa.tilt ? sa.tilt + L.iofs + rowbase + ix * L.ystep : nullptr;
+    const int st = sa.meta->nstages - 1, t0 = sa.meta->stage_first[st], t1 = sa.meta->stage_first[st + 1];
+    double w = 0.;
+    for (int t = t0; t < t1; t += 32) {
+        const int k = t + lane;
+        double leaf = 0.;
+        if (k < t1)
+            leaf = sa.general ? gen_stage_sum(sa.g, k, k + 1, wb, v, tb, L.ipitch, vnf)
+                              : (double)stump_leaf(wb, v, load_stump(sa.stumps + k), vnf);
+        const int m = min(32, t1 - t);
+        for (int j = 0; j < m; j++) w = __dadd_rn(w, __shfl_sync(0xffffffffu, leaf, j));     // XML order
+    }
+    return w;
+}
+
+// order-preserving map of a double onto uint64 (atomicMax over class members) and back
+__device__ __forceinline__ unsigned long long weight_key(double w)
+{
+    const unsigned long long u = (unsigned long long)__double_as_longlong(w);
+    return (u >> 63) ? ~u : u | 0x8000000000000000ull;
+}
+__device__ __forceinline__ double weight_of_key(unsigned long long k)
+{
+    return __longlong_as_double((long long)((k >> 63) ? k & 0x7fffffffffffffffull : ~k));
+}
+
 // rank sort + candidate rectangles (A.6: cvRound of FLOAT products)
+template <bool SCORES>
 __device__ __forceinline__ void cand_sort_body(const PlanDev *__restrict__ plan, int n, const uint32_t *__restrict__ cand,
-                                               uint32_t *sorted, int4 *rects, int *label)
+                                               uint32_t *sorted, int4 *rects, int *label, const ScoreArgs &sa)
 {
     // one WARP per candidate: its rank is counted 32 keys at a time and summed by a warp reduction (a thread per candidate
     // walked all n keys alone — n threads busy, each for n dependent iterations)
@@ -38,6 +91,8 @@ __device__ __forceinline__ void cand_sort_body(const PlanDev *__restrict__ plan,
         int rank = 0;
         for (int j = lane; j < n; j += 32) rank += __ldg(cand + j) < key;
         rank = __reduce_add_sync(0xffffffffu, rank);
+        double wt = 0.;
+        if (SCORES) wt = last_stage_weight(sa, plan, key, lane);
         if (lane) continue;
         int l = key >> 26, iy = (key >> 13) & 8191, ix = key & 8191;
         const LevelDesc &L = plan->lv[l];
@@ -49,15 +104,17 @@ __device__ __forceinline__ void cand_sort_body(const PlanDev *__restrict__ plan,
         r.w = __float2int_rn(__fmul_rn(__int2float_rn(plan->win_h), sc));
         sorted[rank] = key;
         rects[rank] = r;
+        if (SCORES) sa.w[rank] = wt;
         if (label) label[rank] = rank;                            // union-find forest of the large-n path
     }
 }
 
+template <bool SCORES>
 __global__ void __launch_bounds__(256)
 k_cand_sort(const PlanDev *__restrict__ plan, const int *__restrict__ counters, const uint32_t *__restrict__ cand,
-            int cand_cap, uint32_t *__restrict__ sorted, int4 *__restrict__ rects, int *__restrict__ label)
+            int cand_cap, uint32_t *__restrict__ sorted, int4 *__restrict__ rects, int *__restrict__ label, const ScoreArgs sa)
 {
-    cand_sort_body(plan, min(counters[1], cand_cap), cand, sorted, rects, label);
+    cand_sort_body<SCORES>(plan, min(counters[1], cand_cap), cand, sorted, rects, label, sa);
 }
 
 __device__ __forceinline__ int uf_find(int *L, int a)
@@ -158,10 +215,11 @@ __device__ __forceinline__ int block_flag_rank(bool flag, int &carry, int *s_war
 }
 
 // grp scratch layout (ints): label[cap] | cls[cap] | acc[5*cap] (x,y,w,h,count) | keep[cap]
-template <int NT>
+// SCORES: output i also gets its neighbour count and level weight, in the result block after the rectangles
+template <int NT, bool SCORES>
 __device__ __forceinline__ void group_body(int *counters, int cand_cap, const int4 *rects, const uint32_t *adj, int *grp,
                                            int min_neighbors, double eps, int img_w, int img_h, uint8_t *result, int result_cap,
-                                           uint8_t *host_result)
+                                           uint8_t *host_result, const ScoreArgs &sa)
 {
     __shared__ int s_warp[32];
     int tid = threadIdx.x;
@@ -172,6 +230,12 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
     // NV_RESULT_INLINE rectangles are written there as well, straight over PCIe, so that no device-to-host copy follows
     // the launch (one node less in every call's graph).
     int4 *hout = host_result ? reinterpret_cast<int4 *>(host_result + sizeof(ResultHeader)) : nullptr;
+    double *out_w = reinterpret_cast<double *>(out + result_cap), *hout_w = hout ? reinterpret_cast<double *>(hout + result_cap) : nullptr;
+    int *out_n = reinterpret_cast<int *>(out_w + result_cap), *hout_n = hout ? reinterpret_cast<int *>(hout_w + result_cap) : nullptr;
+    auto put_scores = [&](int pos, int nb, double w) {
+        out_w[pos] = w; out_n[pos] = nb;
+        if (hout && pos < NV_RESULT_INLINE) { hout_w[pos] = w; hout_n[pos] = nb; }
+    };
     extern __shared__ int s_label[];                 // min(n, GROUP_SMEM_LABELS) labels; global scratch beyond that
     __shared__ int s_changed;
     const bool uf = n > NV_GROUP_UF_MIN;                          // labels already final in grp (uf_link in k_adj, flattened below)
@@ -193,7 +257,10 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
                 r = make_int4(x0, y0, x1 - x0, y1 - y0);
             }
             int pos = block_flag_rank<NT>(k, carry, s_warp);
-            if (k && pos < result_cap) { out[pos] = r; if (hout && pos < NV_RESULT_INLINE) hout[pos] = r; }
+            if (k && pos < result_cap) {
+                out[pos] = r; if (hout && pos < NV_RESULT_INLINE) hout[pos] = r;
+                if (SCORES) put_scores(pos, 1, sa.w[i]);
+            }
         }
         nout = carry;
     } else {
@@ -248,6 +315,7 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
         }
         int ncls = carry;
         for (int i = tid; i < 5 * ncls; i += NT) acc[i] = 0;
+        if (SCORES) for (int c = tid; c < ncls; c += NT) sa.cls_wmax[c] = 0ull;     // below the key of any finite weight
         __syncthreads();
         for (int i = tid; i < n; i += NT) {
             int c = cls[label[i]];
@@ -255,6 +323,7 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
             atomicAdd(&acc[5 * c + 0], r.x); atomicAdd(&acc[5 * c + 1], r.y);
             atomicAdd(&acc[5 * c + 2], r.z); atomicAdd(&acc[5 * c + 3], r.w);
             atomicAdd(&acc[5 * c + 4], 1);
+            if (SCORES) atomicMax(&sa.cls_wmax[c], weight_key(sa.w[i]));
         }
         __syncthreads();
         for (int c = tid; c < ncls; c += NT) {
@@ -303,7 +372,10 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
                 r = make_int4(x0, y0, x1 - x0, y1 - y0);
             }
             int pos = block_flag_rank<NT>(k, carry, s_warp);
-            if (k && pos < result_cap) { out[pos] = r; if (hout && pos < NV_RESULT_INLINE) hout[pos] = r; }
+            if (k && pos < result_cap) {
+                out[pos] = r; if (hout && pos < NV_RESULT_INLINE) hout[pos] = r;
+                if (SCORES) { const int i = keep[a]; put_scores(pos, acc[5 * i + 4], weight_of_key(sa.cls_wmax[i])); }
+            }
         }
         nout = carry;
     }
@@ -318,12 +390,14 @@ __device__ __forceinline__ void group_body(int *counters, int cand_cap, const in
     }
 }
 
+template <bool SCORES>
 __global__ void __launch_bounds__(NV_GROUP_THREADS)
 k_group(int *__restrict__ counters, int cand_cap, const int4 *__restrict__ rects, const uint32_t *__restrict__ adj,
         int *__restrict__ grp, int min_neighbors, double eps, int img_w, int img_h, uint8_t *__restrict__ result,
-        int result_cap, uint8_t *__restrict__ host_result)
+        int result_cap, uint8_t *__restrict__ host_result, const ScoreArgs sa)
 {
-    group_body<NV_GROUP_THREADS>(counters, cand_cap, rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap, host_result);
+    group_body<NV_GROUP_THREADS, SCORES>(counters, cand_cap, rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap,
+                                         host_result, sa);
 }
 
 // Small plans (a config-1 frame, a nested ROI: a few dozen candidates): canonical order, similarity matrix and grouping by
@@ -333,39 +407,57 @@ k_group(int *__restrict__ counters, int cand_cap, const int4 *__restrict__ rects
 // control and barriers.  (Keeping keys, rectangles, matrix and class tables of up to 256 candidates in shared memory was
 // measured too: no change, 19 us under ncu either way — the launch is a chain of short dependent phases of one block.)
 #define NV_GROUP_FUSED_THREADS 256
+template <bool SCORES>
 __global__ void __launch_bounds__(NV_GROUP_FUSED_THREADS)
 k_group_fused(const PlanDev *__restrict__ plan, int *counters, const uint32_t *__restrict__ cand, int cand_cap, uint32_t *sorted,
               int4 *rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h, uint8_t *result,
-              int result_cap, uint8_t *host_result)
+              int result_cap, uint8_t *host_result, const ScoreArgs sa)
 {
     const int n = min(counters[1], cand_cap);
-    cand_sort_body(plan, n, cand, sorted, rects, min_neighbors > 0 ? grp : nullptr);
+    cand_sort_body<SCORES>(plan, n, cand, sorted, rects, min_neighbors > 0 ? grp : nullptr, sa);
     __syncthreads();
     if (min_neighbors > 0) {
         adj_body(plan, n, sorted, rects, adj, grp, eps);
         __syncthreads();
     }
-    group_body<NV_GROUP_FUSED_THREADS>(counters, cand_cap, rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap, host_result);
+    group_body<NV_GROUP_FUSED_THREADS, SCORES>(counters, cand_cap, rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap,
+                                               host_result, sa);
 }
 
-cudaError_t launch_group(const PlanDev *plan, int *counters, const uint32_t *cand, int cand_cap, uint32_t *cand_sorted,
-                         int4 *cand_rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h,
-                         uint8_t *result, int result_cap, int nblocks, cudaStream_t st, int *nlaunch, bool fused, uint8_t *host_result)
+template <bool SCORES>
+static cudaError_t launch_group_t(const PlanDev *plan, int *counters, const uint32_t *cand, int cand_cap, uint32_t *cand_sorted,
+                                  int4 *cand_rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h,
+                                  uint8_t *result, int result_cap, int nblocks, cudaStream_t st, int *nlaunch, bool fused,
+                                  uint8_t *host_result, const ScoreArgs &sa)
 {
     if (fused) {
-        k_group_fused<<<1, NV_GROUP_FUSED_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj,
-                                                                                  grp, min_neighbors, eps, img_w, img_h, result, result_cap, host_result);
+        k_group_fused<SCORES><<<1, NV_GROUP_FUSED_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(
+            plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap,
+            host_result, sa);
         (*nlaunch)++;
         return cudaGetLastError();
     }
-    k_cand_sort<<<nblocks, 256, 0, st>>>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, min_neighbors > 0 ? grp : nullptr);
+    k_cand_sort<SCORES><<<nblocks, 256, 0, st>>>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, min_neighbors > 0 ? grp : nullptr,
+                                                 sa);
     (*nlaunch)++;
     if (min_neighbors > 0) {
         k_adj<<<nblocks, 256, 0, st>>>(plan, counters, cand_cap, cand_sorted, cand_rects, adj, grp, eps);
         (*nlaunch)++;
     }
-    k_group<<<1, NV_GROUP_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(counters, cand_cap, cand_rects, adj, grp, min_neighbors, eps,
-                                                              img_w, img_h, result, result_cap, host_result);
+    k_group<SCORES><<<1, NV_GROUP_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(counters, cand_cap, cand_rects, adj, grp, min_neighbors,
+                                                                                  eps, img_w, img_h, result, result_cap, host_result, sa);
     (*nlaunch)++;
     return cudaGetLastError();
+}
+
+cudaError_t launch_group(const PlanDev *plan, int *counters, const uint32_t *cand, int cand_cap, uint32_t *cand_sorted,
+                         int4 *cand_rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h,
+                         uint8_t *result, int result_cap, int nblocks, cudaStream_t st, int *nlaunch, bool fused, uint8_t *host_result,
+                         const ScoreArgs *scores)
+{
+    if (scores)
+        return launch_group_t<true>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h,
+                                    result, result_cap, nblocks, st, nlaunch, fused, host_result, *scores);
+    return launch_group_t<false>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h,
+                                 result, result_cap, nblocks, st, nlaunch, fused, host_result, ScoreArgs{});
 }

@@ -83,6 +83,8 @@ _SIGS = {
     "nv_ctx_create": (_i, [_i, _i, _i, C.POINTER(_vp)]),
     "nv_ctx_destroy": (None, [_vp]),
     "nv_ctx_set_debug": (_i, [_vp, _i]),
+    "nv_ctx_set_scores": (_i, [_vp, _i]),
+    "nv_get_scores": (_i, [_vp, _ip, C.POINTER(C.c_double), _i, _ip]),
     "nv_detect_multiscale": (_i, [_vp, _vp, _vp, _i, _i, _i, C.POINTER(DetectParams), _vp, _i, _ip]),
     "nv_face_detect": (_i, [_vp, _vp, _vp, _i, _i, _i, C.POINTER(FaceParams), _vp, _i, _ip]),
     "nv_face_submit": (_i, [_vp, _vp, _vp, _i, _i, _i, C.POINTER(FaceParams)]),
@@ -392,6 +394,7 @@ class Context:
         _check(_lib.nv_ctx_create(gpu, max_width, max_height, C.byref(self.handle)), "nv_ctx_create")
         self._cap = 131072
         self._out = (Rect * self._cap)()
+        self._scores_on = False
         if debug:
             self.set_debug(True)
 
@@ -418,6 +421,29 @@ class Context:
     def record(self, ev: "Event"):
         _check(_lib.nv_event_record(self.handle, ev.handle), "nv_event_record")
 
+    # ---- detection scores (cv::CascadeClassifier::detectMultiScale2 / 3) ---------------------------
+    def set_scores(self, on: bool):
+        """Every later detect call on this context also yields per-rectangle neighbour counts and level weights."""
+        _check(_lib.nv_ctx_set_scores(self.handle, int(on)), "nv_ctx_set_scores")
+        self._scores_on = bool(on)
+
+    def scores(self):
+        """(num_detections int32 [n], level_weights float64 [n]) of the last collected call, parallel to its rectangles."""
+        nb = np.empty(self._cap, np.int32); wt = np.empty(self._cap, np.float64); n = C.c_int(0)
+        _check(_lib.nv_get_scores(self.handle, nb.ctypes.data_as(_ip), wt.ctypes.data_as(C.POINTER(C.c_double)), self._cap,
+                                  C.byref(n)), "nv_get_scores")
+        return nb[:n.value].copy(), wt[:n.value].copy()
+
+    def _with_scores(self, fn):
+        """fn() run with scores on; the context's own setting is restored afterwards."""
+        was = self._scores_on
+        self.set_scores(True)
+        try:
+            rects = fn()
+            return (rects,) + self.scores()
+        finally:
+            self.set_scores(was)
+
     # ---- detection -------------------------------------------------------------------------
     def detect_multiscale(self, casc: Cascade, gray, scale_factor=1.1, min_neighbors=3, min_size=(0, 0), max_size=(0, 0)):
         gray = _u8(gray); h, w = gray.shape
@@ -427,12 +453,27 @@ class Context:
                                          self._out, self._cap, C.byref(n)), "nv_detect_multiscale")
         return _rects(self._out, n.value)
 
+    def detect_multiscale2(self, casc: Cascade, gray, scale_factor=1.1, min_neighbors=3, min_size=(0, 0), max_size=(0, 0)):
+        """cv2.CascadeClassifier.detectMultiScale2: (rects, num_detections)."""
+        r, nb, _ = self._with_scores(lambda: self.detect_multiscale(casc, gray, scale_factor, min_neighbors, min_size, max_size))
+        return r, nb
+
+    def detect_multiscale3(self, casc: Cascade, gray, scale_factor=1.1, min_neighbors=3, min_size=(0, 0), max_size=(0, 0)):
+        """cv2.CascadeClassifier.detectMultiScale3(..., outputRejectLevels=True): (rects, reject_levels, level_weights).
+        reject_levels is always the cascade's stage count, as in OpenCV 4.13."""
+        r, _, wt = self._with_scores(lambda: self.detect_multiscale(casc, gray, scale_factor, min_neighbors, min_size, max_size))
+        return r, np.full(len(r), casc.info.nstages, np.int32), wt
+
     @staticmethod
     def _face_params(width_to_process, scale_factor, min_neighbors, min_size):
         mw, mh = (-1, -1) if min_size is None else min_size
         return FaceParams(width_to_process, scale_factor, min_neighbors, mw, mh)
 
-    def face_detect(self, casc: Cascade, bgr, width_to_process=160, scale_factor=1.25, min_neighbors=3, min_size=None):
+    def face_detect(self, casc: Cascade, bgr, width_to_process=160, scale_factor=1.25, min_neighbors=3, min_size=None,
+                    scores=False):
+        """scores=True: (rects, num_detections, level_weights), see set_scores."""
+        if scores:
+            return self._with_scores(lambda: self.face_detect(casc, bgr, width_to_process, scale_factor, min_neighbors, min_size))
         bgr = _u8(bgr); h, w, _ = bgr.shape
         p = self._face_params(width_to_process, scale_factor, min_neighbors, min_size)
         n = C.c_int(0)
@@ -490,10 +531,12 @@ class Context:
         _check(_lib.nv_yuv2bgr(self.handle, C.byref(f), _p(out), 3 * f.width), "nv_yuv2bgr")
         return out
 
-    def face_collect(self):
+    def face_collect(self, scores=False):
+        """scores=True: (rects, num_detections, level_weights) of a call submitted with set_scores(True)."""
         n = C.c_int(0)
         _check(_lib.nv_face_collect(self.handle, self._out, self._cap, C.byref(n)), "nv_face_collect")
-        return _rects(self._out, n.value)
+        rects = _rects(self._out, n.value)
+        return (rects,) + self.scores() if scores else rects
 
     # ---- tracker ---------------------------------------------------------------------------
     def tracker_process(self, bgra, ts_ms, threshold=20, min_area=50, max_area=30000, distance=35):

@@ -1,6 +1,7 @@
 """Randomised parity run (not part of the test suite): random frame sizes, strides, processing widths, scale factors,
 minNeighbors and input formats through a few long-lived contexts (plan cache, graph replay, format switches) against the
-CPU oracle, for a wall-clock budget.  Usage: python tools/fuzz_parity.py [seconds] [seed]"""
+CPU oracle, for a wall-clock budget.  --scores: every context runs with detection scores on, and each call's neighbour
+counts and level weights are checked too.  Usage: python tools/fuzz_parity.py [seconds] [seed] [--scores]"""
 import os
 import sys
 import time
@@ -8,17 +9,22 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path[:0] = [os.path.join(ROOT, "nubomedia-vca_b200", "python"), os.path.join(ROOT, "oracle")]
+sys.path[:0] = [os.path.join(ROOT, "nubomedia-vca_b200", "python"), os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")]
 import nubovca as nv  # noqa: E402
 import oracle as O  # noqa: E402
+import scores_ref as S  # noqa: E402
 from nubovca import synth  # noqa: E402
 
-budget = float(sys.argv[1]) if len(sys.argv) > 1 else 120.0
-seed = int(sys.argv[2]) if len(sys.argv) > 2 else 0
+scores = "--scores" in sys.argv
+args = [a for a in sys.argv[1:] if a != "--scores"]
+budget = float(args[0]) if len(args) > 0 else 120.0
+seed = int(args[1]) if len(args) > 1 else 0
 rng = np.random.default_rng(seed)
 xml = os.path.join(ROOT, "nubomedia-vca_b200", "cascades", "haarcascade_frontalface_alt.xml")
 ncasc, ocasc = nv.Cascade(xml), O.Cascade(xml)
 ctxs = [nv.Context(0, 1920, 1080, debug=False) for _ in range(3)] + [nv.Context(0, 1920, 1080, debug=True)]
+for c in ctxs:
+    c.set_scores(scores)
 t0 = time.time()
 n = bad = 0
 shapes = []
@@ -59,6 +65,11 @@ while time.time() - t0 < budget:
     ok = got.shape == exp.shape and (got == exp).all()
     if c is ctxs[-1]:
         ok = ok and (c.gray() == eq).all()
+    if scores:
+        rows, cols = eq.shape
+        _, enb, ewt = S.detect_multiscale_scores(eq, ocasc, sf, mn, (cols // 20, rows // 20) if ms is None else ms)
+        nb, wt = c.scores()
+        ok = ok and nb.shape == enb.shape and (nb == enb).all() and (wt == ewt).all()
     n += 1
     if not ok:
         bad += 1
