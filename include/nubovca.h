@@ -152,6 +152,42 @@ NV_API void nv_host_free(void *p);
 NV_API int nv_host_register(void *p, size_t bytes);
 NV_API int nv_host_unregister(void *p);
 
+/* ---- batches: N images of one size per call, through one chain of kernel launches ---------------------------------------
+ *      frames: N pointers to N images (8-bit gray for nv_detect_multiscale_batch, BGR for the face calls), each `height`
+ *      rows of `stride_bytes`.  on_device == 0: host memory, copied like the single calls' frames (page-locked frames are
+ *      read by the DMA engine in place and must stay untouched until collect, pageable ones are staged before submit
+ *      returns; for the face calls only the row pairs the resize reads travel, as in nv_face_submit).  on_device != 0:
+ *      device pointers (a CUDA uint8 tensor [N, H, W(, 3)]: data_ptr() + i * stride(0)), read in place until collect.
+ *      Image i's rectangles are exactly those of the single call on that image (nv_detect_multiscale / nv_face_detect,
+ *      same nv_face_params rules, min_w < 0 included).  out holds image 0's rectangles, then image 1's, ...; counts[i] is
+ *      always image i's true count and *total (if given) the number written; when the counts add up to more than cap, the
+ *      first cap rectangles are written and the call returns NV_ERR_CAPACITY.
+ *      Route: when the image size makes a small plan (at most 16384 windows) of a stump cascade with the order-free
+ *      exactness certificates whose weak classifiers fit in shared memory (haarcascade_frontalface_alt on a 160x120 or
+ *      96x64 image: the face element's default shape), the whole batch runs as ONE chain of six kernel launches (five for
+ *      gray images), replayed as one CUDA graph once the shape (N, size, cascade, parameters) repeats — new frame addresses
+ *      on every call do not prevent the replay.  An image with more than 1024 raw candidates is detected again alone in
+ *      collect.  Every other case (larger images, tree / tilted / LBP models, models without the certificates) runs the
+ *      single-image pipeline once per image inside submit: the same results, no gain in throughput.
+ *      The context grows its per-image buffers to the largest batch it has seen and keeps them.  A batch shares the
+ *      context's cache of plans with the single calls: a batch shape that is not cached takes the least recently used
+ *      plan (and that plan's single-call graph) and may grow the single-call integral buffers, so a single call after it
+ *      can re-plan once; results never depend on it.
+ *      Refused: N < 1 or N > NV_BATCH_MAX (NV_ERR_ARG); a context with scores on (NV_ERR_STATE).  After a batch,
+ *      nv_debug_get_counters reports [0..2] summed over its images, [3] the kernel launches of the whole call and [4] 1 when
+ *      the batched chain was replayed from a CUDA graph captured by an earlier call (0 otherwise); the other
+ *      parity taps, nv_get_scores and nv_ctx_get_stage_times return NV_ERR_STATE (they describe single calls); a pending
+ *      batch is collected with nv_face_collect_batch only. ---------------------------------------------------------------- */
+#define NV_BATCH_MAX 256
+NV_API int nv_detect_multiscale_batch(nv_ctx *ctx, const nv_cascade *c, const uint8_t *const *frames, int n, int width, int height,
+                                      int stride_bytes, int on_device, const nv_detect_params *p, nv_rect *out, int cap, int *counts);
+NV_API int nv_face_submit_batch(nv_ctx *ctx, const nv_cascade *c, const uint8_t *const *frames, int n, int width, int height,
+                                int stride_bytes, int on_device, const nv_face_params *p);
+NV_API int nv_face_collect_batch(nv_ctx *ctx, nv_rect *out, int cap, int *counts, int *total);
+NV_API int nv_face_detect_batch(nv_ctx *ctx, const nv_cascade *c, const uint8_t *const *frames, int n, int width, int height,
+                                int stride_bytes, int on_device, const nv_face_params *p, nv_rect *out, int cap, int *counts,
+                                int *total);
+
 /* ---- 4:2:0 ingest (extension, SURVEY §8f rank 4).  The reference elements negotiate BGR only
  *      (kmsfacedetect.cpp:129-133,1025-1031), so a decoder's I420 / NV12 output passes through a CPU videoconvert
  *      and twice the bytes cross PCIe.  These entry points take the decoder's planes as they are: the result is

@@ -23,6 +23,10 @@
 #define NV_MAX_LEVELS 64          // level index is packed in 6 bits of a window id
 #define NV_MAX_STAGES 64
 #define NV_RESULT_INLINE 1024     // rects copied back with the header in one D2H
+#define NV_HIST_STRIDE 260        // ints per histogram: 256 bins + the prep kernels' last-block ticket
+// batched route (nv_detect_multiscale_batch, nv_face_submit_batch): raw candidates and rectangles grouped on the device per
+// image; an image with more is re-run through the single-image path in collect
+#define NV_BATCH_GROUP_CAP NV_RESULT_INLINE
 
 // ----------------------------------------------------------------------------------------------
 // error plumbing
@@ -262,6 +266,8 @@ struct Stage0Params {
     int16_t *depth;
     uint2 *queue;                                    // small plans: (window id, vnf) of every alive window goes straight to the
     int queue_cap, queue_cidx;                       // warp-per-window kernel's queue (count in counters[queue_cidx]); else nullptr
+    size_t integ_stride;                             // batched launch (k_stage0_rows_p<true>): per-image strides of sum / sq,
+    int win_stride, bits_stride;                     // vnf and alive bits
 };
 static_assert(sizeof(Stage0Params) <= 32000, "kernel parameter space is 32764 bytes");
 
@@ -379,6 +385,40 @@ struct nv_ctx {
     int last_min_neighbors = 0;
     long long launches = 0;
 
+    // batched route (nv_detect_multiscale_batch / nv_face_submit_batch): per-image buffers, grow-only, sized for bcap images
+    struct Batch {
+        int cap = 0;                                        // images the per-image buffers below hold
+        size_t frame_bytes = 0, gray_bytes = 0, integ = 0, wins = 0, bits = 0;   // per-image sizes the buffers were made for
+        uint8_t *d_frame = nullptr, *h_stage = nullptr;     // uploaded frames / pinned staging of pageable ones
+        uint8_t *d_gray = nullptr, *d_lut = nullptr;  int *d_hist = nullptr;
+        uint32_t *d_sum = nullptr, *d_sq = nullptr, *d_bits = nullptr;  float *d_vnf = nullptr;
+        uint2 *d_queue = nullptr;  uint32_t *d_cand = nullptr, *d_sorted = nullptr;  int4 *d_rects = nullptr;
+        uint32_t *d_adj = nullptr;  int *d_grp = nullptr;
+        int *d_counters = nullptr;                          // 16 shared + 16 per image
+        uint8_t *d_result = nullptr, *h_result = nullptr;   // per image: ResultHeader + NV_BATCH_GROUP_CAP rects
+        const uint8_t **d_tab = nullptr, **h_tab = nullptr; // per call: N source frames, N gray images
+        std::vector<const uint8_t *> tab_last;             // what d_tab holds
+        unsigned long long gen = 1;                         // bumped whenever a buffer above moves
+    } b;
+    struct BatchKey {
+        int kind = 0, n = 0, w = 0, h = 0, stride = 0, cols = 0, rows = 0; const int *rtab = nullptr; bool aligned = false;
+        unsigned long long casc = 0; double sf = 0; int mn = 0, min_w = 0, min_h = 0, max_w = 0, max_h = 0;
+        unsigned long long epoch = 0, bgen = 0; const PlanSlot *slot = nullptr; unsigned long long slot_gen = 0;
+        bool operator==(const BatchKey &o) const {
+            return kind == o.kind && n == o.n && w == o.w && h == o.h && stride == o.stride && cols == o.cols && rows == o.rows &&
+                   rtab == o.rtab && aligned == o.aligned && casc == o.casc && sf == o.sf && mn == o.mn && min_w == o.min_w &&
+                   min_h == o.min_h && max_w == o.max_w && max_h == o.max_h && epoch == o.epoch && bgen == o.bgen && slot == o.slot &&
+                   slot_gen == o.slot_gen;
+        }
+    };
+    cudaGraphExec_t bexec = nullptr;  BatchKey bkey, bkey_seen;  int b_nl = 0;
+    // last batch call: what collect needs (route, images, the overflow re-run's inputs), and what the counters tap reports
+    bool batch_last = false, batch_routed = false, batch_replayed = false;  int batch_n = 0, batch_kind = 0;
+    std::vector<const uint8_t *> batch_src;  int batch_w = 0, batch_h = 0, batch_stride = 0;  bool batch_on_device = false;
+    nv_face_params batch_fp = {};  nv_detect_params batch_dp = {};  nv_cascade *batch_casc = nullptr;
+    long long batch_sum[3] = {0, 0, 0}, batch_launches = 0;
+    std::vector<nv_rect> batch_out;  std::vector<int> batch_counts;      // collected rectangles (image after image) and counts
+
     // tracker state (gstnubotracker.cpp:88-106 priv + the file-static img_prev :108, made per-ctx)
     // d_trk_hist: the motion history as one byte per pixel, an index into trk_val (the live timestamps; 0 = no history)
     uint8_t *d_trk_prev = nullptr, *d_trk_hist = nullptr, *d_trk_scratch = nullptr;
@@ -472,6 +512,19 @@ cudaError_t launch_cascade_tail_block(const PlanDev *plan, const DevCascade *met
 int nv_detect_device(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, int W, int H, int gstride, const uint8_t *d_lut,
                      const nv_detect_params *p);
 int nv_collect(nv_ctx *ctx, nv_rect *out, int cap, int *n);
+// kernels of the batched route (one launch each for the whole batch)
+cudaError_t launch_face_prep_batch(const uint8_t *const *srcs, int n, bool aligned, int sw, int sh, int sstride, uint8_t *gray,
+                                   int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st);
+cudaError_t launch_pyramid_batch(const PlanDev *plan, int total_rowblk, int total_colblk, int n, const uint8_t *const *grays, int gstride,
+                                 const uint8_t *lut, int lut_stride, const int *ptab, uint32_t *sum, uint32_t *sq, size_t integ_stride,
+                                 cudaStream_t st);
+cudaError_t launch_stage0_rows_p_batch(const Stage0Params &sp, int n, cudaStream_t st);
+cudaError_t launch_cascade_tail_tab_batch(const PlanDev *plan, const DevCascade *meta, const DevCascade &hmeta, const TailStump *tstumps,
+                                          const double *tbase, const uint32_t *sum, size_t integ_stride, const uint2 *queue, int queue_cap,
+                                          int *counters, uint32_t *cand, int cand_stride, cudaStream_t st);
+cudaError_t launch_group_batch(const PlanDev *plan, int n, int *counters, const uint32_t *cand, int cand_stride, int cap, uint32_t *cand_sorted,
+                               int4 *cand_rects, uint32_t *adj, size_t adj_stride, int *grp, int min_neighbors, double eps, int img_w,
+                               int img_h, uint8_t *result, uint8_t *host_result, size_t result_stride, cudaStream_t st);
 int nv_h2d(nv_ctx *ctx, const uint8_t *src, size_t bytes);
 int nv_get_rtab(nv_ctx *ctx, int sw, int sh, int dw, int dh, const int **d_tab, const nv_ctx::RtabEntry **entry = nullptr);
 

@@ -337,16 +337,28 @@ __device__ __forceinline__ uint32_t skip_rule_word(uint32_t f, bool &e)
     return em;
 }
 
+// BATCH: image blockIdx.y; integrals, vnf and alive bits at its strides, its alive count in its own counter block
+// (P.counters + 16 * (1 + image)); queue entries are (image << 14) | dense window index, the queue and its count shared.
+template <bool BATCH>
 __global__ void __launch_bounds__(256) k_stage0_rows_p(const __grid_constant__ Stage0Params P)
 {
     const int lane = threadIdx.x & 31;
     const int row = blockIdx.x * 8 + uniformize_s0(threadIdx.x >> 5);
     if (row >= P.total_rows) return;
+    const uint32_t *sum = P.sum, *sq = P.sq;
+    float *vnfs = P.vnf;
+    uint32_t *bits_alive = P.bits_alive;
+    int *cnt = P.counters;
+    if (BATCH) {
+        sum += blockIdx.y * P.integ_stride; sq += blockIdx.y * P.integ_stride;
+        vnfs += blockIdx.y * (size_t)P.win_stride; bits_alive += blockIdx.y * (size_t)P.bits_stride;
+        cnt += 16 * (1 + blockIdx.y);
+    }
     int l = 0;
     while (l + 1 < P.nlevels && P.lv_a[l + 1].x <= row) l++;
     const int4 la = P.lv_a[l], lb = P.lv_b[l], vr = P.var[l];
     const int iy = row - la.x, nxw = la.y, nx = la.z;
-    const uint32_t *srow = P.sum + lb.x + (size_t)iy * la.w, *qrow = P.sq + lb.x + (size_t)iy * la.w;
+    const uint32_t *srow = sum + lb.x + (size_t)iy * la.w, *qrow = sq + lb.x + (size_t)iy * la.w;
     const double area = (double)((P.win_w - 2) * (P.win_h - 2));
     const double thr0 = (double)P.thr0;
     bool e = true;                                   // is the next window visited?  (x = 0 always is)
@@ -388,22 +400,24 @@ __global__ void __launch_bounds__(256) k_stage0_rows_p(const __grid_constant__ S
         bool alive = visited && ok && !fail;
         uint32_t am = __ballot_sync(0xffffffffu, alive);
         nalive += __popc(am);
-        if (lane == 0) P.bits_alive[lb.z + iy * nxw + cx] = am;
-        if (alive) P.vnf[lb.y + iy * nx + ix] = vnf;
+        if (lane == 0) bits_alive[lb.z + iy * nxw + cx] = am;
+        if (alive) vnfs[lb.y + iy * nx + ix] = vnf;
         if (P.queue && am) {                             // small plan: k_alive_to_queue's job, without its launch
             int base = 0;
             if (lane == 0) base = atomicAdd(&P.counters[P.queue_cidx], __popc(am));
             base = __shfl_sync(0xffffffffu, base, 0);
             if (alive) {
                 const int pos = base + __popc(am & ((1u << lane) - 1u));
-                if (pos < P.queue_cap) P.queue[pos] = make_uint2(((uint32_t)l << 26) | ((uint32_t)iy << 13) | (uint32_t)ix, __float_as_uint(vnf));
+                const uint32_t id = BATCH ? ((uint32_t)blockIdx.y << 14) | (uint32_t)(lb.y + iy * nx + ix)
+                                          : ((uint32_t)l << 26) | ((uint32_t)iy << 13) | (uint32_t)ix;
+                if (pos < P.queue_cap) P.queue[pos] = make_uint2(id, __float_as_uint(vnf));
                 else P.counters[2] = 1;
             }
         }
         if (P.depth && valid && !alive)
             P.depth[lb.y + iy * nx + ix] = (int16_t)(!visited ? NV_DEPTH_SKIPPED : (!ok ? NV_DEPTH_VARREJ : 0));
     }
-    if (lane == 0 && nalive) atomicAdd(&P.counters[0], nalive);
+    if (lane == 0 && nalive) atomicAdd(&cnt[0], nalive);
 }
 
 bool fill_stage0_params(const nv_cascade *c, const PlanDev &P, Stage0Params *sp)
@@ -1370,12 +1384,15 @@ k_cascade_tail_fast(const PlanDev *__restrict__ plan, const DevCascade *__restri
 // (half the rounds, the two evaluations overlap), and the stage bounds / thresholds / base sums sit in shared memory
 // too.  Fewer, fatter blocks: as many per SM as the table allows, persistent over the window queue.  Same certificates,
 // same arithmetic, same results as k_cascade_tail_fast; used when the table fits (launch_cascade_tail_tab).
-template <int NWARP>
+// BATCH: the queue holds the windows of a batch of images, (image << 14) | dense window index (k_stage0_rows_p<true>); the
+// image's integrals lie at image * integ_stride, its candidates go to its own segment cand + image * cand_stride with the
+// count in its own counter block (counters + 16 * (1 + image)).  Queue count and ticket stay in counters[3] / [5].
+template <int NWARP, bool BATCH>
 __global__ void __launch_bounds__(32 * NWARP)
 k_cascade_tail_tab(const PlanDev *__restrict__ plan, const DevCascade *__restrict__ meta, const TailStump *__restrict__ ts,
                    const double *__restrict__ tbase, const uint32_t *__restrict__ sum, const uint2 *__restrict__ tail,
                    int *__restrict__ counters, uint32_t *__restrict__ cand, int cand_cap, int16_t *__restrict__ depth,
-                   int stage_begin, int stage_end, uint2 *__restrict__ deep, int deep_cap)
+                   int stage_begin, int stage_end, uint2 *__restrict__ deep, int deep_cap, size_t integ_stride = 0, int cand_stride = 0)
 {
     extern __shared__ __align__(16) uint32_t s_tab[];            // A[nt] uint4 | B[nt] uint4 | C[nt] double | NWARP patches
     __shared__ int s_first[NV_MAX_STAGES + 1];
@@ -1417,11 +1434,28 @@ k_cascade_tail_tab(const PlanDev *__restrict__ plan, const DevCascade *__restric
         e = __shfl_sync(0xffffffffu, e, 0);
         if (e >= n) break;
         const uint2 q = tail[e];
-        const int l = q.x >> 26, iy = (q.x >> 13) & 8191, ix = q.x & 8191;
+        int l, iy, ix;
+        uint32_t id = q.x;
+        const uint32_t *isum = sum;
+        int *icnt = counters;
+        uint32_t *icand = cand;
+        int icap = cand_cap;
+        if (BATCH) {
+            const int img = q.x >> 14, w = q.x & 16383;
+            l = 0;
+            while (l + 1 < plan->nlevels && plan->lv[l + 1].wofs <= w) l++;
+            const int r = w - plan->lv[l].wofs;
+            iy = r / plan->lv[l].nx; ix = r - iy * plan->lv[l].nx;
+            id = ((uint32_t)l << 26) | ((uint32_t)iy << 13) | (uint32_t)ix;
+            isum = sum + img * integ_stride; icnt = counters + 16 * (1 + img);
+            icand = cand + img * (size_t)cand_stride; icap = cand_stride;
+        } else {
+            l = q.x >> 26; iy = (q.x >> 13) & 8191; ix = q.x & 8191;
+        }
         const float vnf = __uint_as_float(q.y);
         const LevelDesc &L = plan->lv[l];
         const int pitch = L.ipitch;
-        const uint32_t *wb = sum + L.iofs + (size_t)iy * L.ystep * pitch + ix;
+        const uint32_t *wb = isum + L.iofs + (size_t)iy * L.ystep * pitch + ix;
         __syncwarp();                                            // the previous window's reads of the patch are done
         copy_patch(win, wb, pitch, L.ystep, L.iplane, LP, npatch, lane);         // private copy of the window's integral patch
         __syncwarp();
@@ -1457,9 +1491,9 @@ k_cascade_tail_tab(const PlanDev *__restrict__ plan, const DevCascade *__restric
         if (lane == 0) {
             if (depth && (last || code != NV_DEPTH_PASS)) depth[L.wofs + iy * L.nx + ix] = (int16_t)code;
             if (code == NV_DEPTH_PASS && last) {
-                const int pos = atomicAdd(&counters[1], 1);
-                if (pos < cand_cap) cand[pos] = q.x;
-                else counters[2] = 1;
+                const int pos = atomicAdd(&icnt[1], 1);
+                if (pos < icap) icand[pos] = id;
+                else icnt[2] = 1;
             } else if (code == NV_DEPTH_PASS) {
                 const int pos = atomicAdd(&counters[6], 1);
                 if (pos < deep_cap) deep[pos] = q;
@@ -1914,10 +1948,11 @@ size_t tail_tab_smem(const DevCascade &m, int stage_begin, int stage_end)
     return nt * 40 + (size_t)NV_TAILTAB_WARPS * (m.win_w + 1) * (m.win_h + 1) * 4;
 }
 
-cudaError_t launch_cascade_tail_tab(const PlanDev *plan, const DevCascade *meta, const DevCascade &hmeta, const TailStump *tstumps,
-                                    const double *tbase, const uint32_t *sum, const uint2 *tail, int *counters, uint32_t *cand,
-                                    int cand_cap, int16_t *depth, int stage_begin, int stage_end, uint2 *deep, int deep_cap,
-                                    cudaStream_t st)
+template <bool BATCH>
+static cudaError_t launch_tail_tab_t(const PlanDev *plan, const DevCascade *meta, const DevCascade &hmeta, const TailStump *tstumps,
+                                     const double *tbase, const uint32_t *sum, const uint2 *tail, int *counters, uint32_t *cand,
+                                     int cand_cap, int16_t *depth, int stage_begin, int stage_end, uint2 *deep, int deep_cap,
+                                     cudaStream_t st, size_t integ_stride, int cand_stride)
 {
     const size_t smem = tail_tab_smem(hmeta, stage_begin, stage_end);
     if (smem > NV_TAILTAB_MAX_SMEM) return cudaErrorInvalidConfiguration;
@@ -1928,7 +1963,7 @@ cudaError_t launch_cascade_tail_tab(const PlanDev *plan, const DevCascade *meta,
     {
         std::lock_guard<std::mutex> lk(mu);
         if (!((attr_set >> (dev & 63)) & 1ull)) {
-            cudaError_t e = cudaFuncSetAttribute(k_cascade_tail_tab<NV_TAILTAB_WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NV_TAILTAB_MAX_SMEM);
+            cudaError_t e = cudaFuncSetAttribute(k_cascade_tail_tab<NV_TAILTAB_WARPS, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NV_TAILTAB_MAX_SMEM);
             if (e != cudaSuccess) return e;
             attr_set |= 1ull << (dev & 63);
         }
@@ -1937,9 +1972,27 @@ cudaError_t launch_cascade_tail_tab(const PlanDev *plan, const DevCascade *meta,
     per_sm = per_sm < 1 ? 1 : per_sm > 8 ? 8 : per_sm;
     // (fewer blocks when the queue is short — every block copies the table — was measured: no gain down to one block per 32
     // windows of the plan, slower below)
-    k_cascade_tail_tab<NV_TAILTAB_WARPS><<<148 * per_sm, 32 * NV_TAILTAB_WARPS, smem, st>>>(
-        plan, meta, tstumps, tbase, sum, tail, counters, cand, cand_cap, depth, stage_begin, stage_end, deep, deep_cap);
+    k_cascade_tail_tab<NV_TAILTAB_WARPS, BATCH><<<148 * per_sm, 32 * NV_TAILTAB_WARPS, smem, st>>>(
+        plan, meta, tstumps, tbase, sum, tail, counters, cand, cand_cap, depth, stage_begin, stage_end, deep, deep_cap, integ_stride,
+        cand_stride);
     return cudaGetLastError();
+}
+
+cudaError_t launch_cascade_tail_tab(const PlanDev *plan, const DevCascade *meta, const DevCascade &hmeta, const TailStump *tstumps,
+                                    const double *tbase, const uint32_t *sum, const uint2 *tail, int *counters, uint32_t *cand,
+                                    int cand_cap, int16_t *depth, int stage_begin, int stage_end, uint2 *deep, int deep_cap,
+                                    cudaStream_t st)
+{
+    return launch_tail_tab_t<false>(plan, meta, hmeta, tstumps, tbase, sum, tail, counters, cand, cand_cap, depth, stage_begin, stage_end,
+                                    deep, deep_cap, st, 0, 0);
+}
+
+cudaError_t launch_cascade_tail_tab_batch(const PlanDev *plan, const DevCascade *meta, const DevCascade &hmeta, const TailStump *tstumps,
+                                          const double *tbase, const uint32_t *sum, size_t integ_stride, const uint2 *queue, int queue_cap,
+                                          int *counters, uint32_t *cand, int cand_stride, cudaStream_t st)
+{
+    return launch_tail_tab_t<true>(plan, meta, hmeta, tstumps, tbase, sum, queue, counters, cand, cand_stride, nullptr, 1, hmeta.nstages,
+                                   nullptr, queue_cap, st, integ_stride, cand_stride);
 }
 
 cudaError_t launch_stage0_rows_gen(const PlanDev *plan, int total_rows, const DevCascade *meta, const GenModel &g,
@@ -1993,6 +2046,12 @@ cudaError_t launch_queue_stages_gen_staged(const PlanDev *plan, const DevCascade
 
 cudaError_t launch_stage0_rows_p(const Stage0Params &sp, cudaStream_t st)
 {
-    k_stage0_rows_p<<<(sp.total_rows + 7) / 8, 256, 0, st>>>(sp);
+    k_stage0_rows_p<false><<<(sp.total_rows + 7) / 8, 256, 0, st>>>(sp);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_stage0_rows_p_batch(const Stage0Params &sp, int n, cudaStream_t st)
+{
+    k_stage0_rows_p<true><<<dim3((sp.total_rows + 7) / 8, n), 256, 0, st>>>(sp);
     return cudaGetLastError();
 }

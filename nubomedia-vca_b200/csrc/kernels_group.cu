@@ -406,13 +406,27 @@ k_group(int *__restrict__ counters, int cand_cap, const int4 *__restrict__ rects
 // parameter here.  256 threads: with the few dozen candidates of such a call 24 of a 1024-thread block's warps only run loop
 // control and barriers.  (Keeping keys, rectangles, matrix and class tables of up to 256 candidates in shared memory was
 // measured too: no change, 19 us under ncu either way — the launch is a chain of short dependent phases of one block.)
+//
+// BATCH: one block per image of a batch, image blockIdx.y (gridDim.x stays 1, so the bodies' grid-stride loops cover the
+// image's own candidates).  The image's counters are counters + 16 * (1 + image), its candidates the segment at
+// image * cand_stride, its scratch and result block at image times their sizes; block 0 also clears the batch's shared
+// counter block (counters[0 .. 15]: queue count and ticket).
 #define NV_GROUP_FUSED_THREADS 256
-template <bool SCORES>
+template <bool SCORES, bool BATCH>
 __global__ void __launch_bounds__(NV_GROUP_FUSED_THREADS)
 k_group_fused(const PlanDev *__restrict__ plan, int *counters, const uint32_t *__restrict__ cand, int cand_cap, uint32_t *sorted,
               int4 *rects, uint32_t *adj, int *grp, int min_neighbors, double eps, int img_w, int img_h, uint8_t *result,
-              int result_cap, uint8_t *host_result, const ScoreArgs sa)
+              int result_cap, uint8_t *host_result, const ScoreArgs sa, int cand_stride = 0, size_t adj_stride = 0,
+              size_t result_stride = 0)
 {
+    if (BATCH) {
+        const int img = blockIdx.y;
+        if (img == 0 && threadIdx.x < 16) counters[threadIdx.x] = 0;
+        counters += 16 * (1 + img);
+        cand += img * (size_t)cand_stride;
+        sorted += img * (size_t)cand_cap; rects += img * (size_t)cand_cap; grp += img * 8 * (size_t)cand_cap; adj += img * adj_stride;
+        result += img * result_stride; host_result += img * result_stride;
+    }
     const int n = min(counters[1], cand_cap);
     cand_sort_body<SCORES>(plan, n, cand, sorted, rects, min_neighbors > 0 ? grp : nullptr, sa);
     __syncthreads();
@@ -431,7 +445,7 @@ static cudaError_t launch_group_t(const PlanDev *plan, int *counters, const uint
                                   uint8_t *host_result, const ScoreArgs &sa)
 {
     if (fused) {
-        k_group_fused<SCORES><<<1, NV_GROUP_FUSED_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(
+        k_group_fused<SCORES, false><<<1, NV_GROUP_FUSED_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(
             plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h, result, result_cap,
             host_result, sa);
         (*nlaunch)++;
@@ -460,4 +474,14 @@ cudaError_t launch_group(const PlanDev *plan, int *counters, const uint32_t *can
                                     result, result_cap, nblocks, st, nlaunch, fused, host_result, *scores);
     return launch_group_t<false>(plan, counters, cand, cand_cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h,
                                  result, result_cap, nblocks, st, nlaunch, fused, host_result, ScoreArgs{});
+}
+
+cudaError_t launch_group_batch(const PlanDev *plan, int n, int *counters, const uint32_t *cand, int cand_stride, int cap, uint32_t *cand_sorted,
+                               int4 *cand_rects, uint32_t *adj, size_t adj_stride, int *grp, int min_neighbors, double eps, int img_w,
+                               int img_h, uint8_t *result, uint8_t *host_result, size_t result_stride, cudaStream_t st)
+{
+    k_group_fused<false, true><<<dim3(1, n), NV_GROUP_FUSED_THREADS, GROUP_SMEM_LABELS * sizeof(int), st>>>(
+        plan, counters, cand, cap, cand_sorted, cand_rects, adj, grp, min_neighbors, eps, img_w, img_h, result, cap, host_result,
+        ScoreArgs{}, cand_stride, adj_stride, result_stride);
+    return cudaGetLastError();
 }

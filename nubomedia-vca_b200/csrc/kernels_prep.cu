@@ -85,6 +85,8 @@ __device__ __forceinline__ uint8_t lut_entry(int t, int hv, int total, int *cum,
 // End of a face-prep kernel: flush the block's histogram; with `lut` set, the block that finishes LAST (a ticket in
 // hist[256]) turns the complete histogram into the LUT and clears histogram and ticket for the next frame — what a k_lut
 // does as a launch of its own (one block, ~4 us of a small call's chain) when the histogram comes from elsewhere.
+// BATCH: one image per gridDim.y row; the ticket counts that image's blocks only.
+template <bool BATCH = false>
 __device__ __forceinline__ void prep_finish(int tid, int *sh_hist, int *__restrict__ hist, uint8_t *__restrict__ lut, int total)
 {
     __shared__ int s_i0, s_last;
@@ -93,7 +95,7 @@ __device__ __forceinline__ void prep_finish(int tid, int *sh_hist, int *__restri
     if (!lut) return;
     __threadfence();
     __syncthreads();
-    if (tid == 0) s_last = atomicAdd(&hist[256], 1) == (int)(gridDim.x * gridDim.y) - 1;
+    if (tid == 0) s_last = atomicAdd(&hist[256], 1) == (int)(BATCH ? gridDim.x : gridDim.x * gridDim.y) - 1;
     __syncthreads();
     if (!s_last) return;
     __threadfence();
@@ -108,11 +110,19 @@ __device__ __forceinline__ void prep_finish(int tid, int *sh_hist, int *__restri
 // Blocks walk the 32x8-pixel output tiles with a grid stride (the launchers size the grid to a few blocks per SM): the
 // shared histogram is flushed once per block, so the global histogram sees a few hundred atomics per bin and frame
 // instead of one per bin and tile (8100 tiles on a 1080p frame).
+// BATCH: image blockIdx.y reads its frame from srcs[blockIdx.y] and owns gray, histogram (+ ticket) and LUT at
+// blockIdx.y times the strides.
+template <bool BATCH>
 __global__ void __launch_bounds__(256)
 k_face_prep(const uint8_t *__restrict__ src, int sw, int sh, int sstride, int cn, uint8_t *__restrict__ gray, int dw,
-            int dh, const int *__restrict__ rtab, int *__restrict__ hist, uint8_t *__restrict__ lut)
+            int dh, const int *__restrict__ rtab, int *__restrict__ hist, uint8_t *__restrict__ lut,
+            const uint8_t *const *__restrict__ srcs = nullptr, size_t gray_stride = 0)
 {
     __shared__ int sh_hist[256];
+    if (BATCH) {
+        src = srcs[blockIdx.y];
+        gray += blockIdx.y * gray_stride; hist += blockIdx.y * NV_HIST_STRIDE; lut += blockIdx.y * 256;
+    }
     int tid = threadIdx.y * 32 + threadIdx.x;
     sh_hist[tid] = 0;
     __syncthreads();
@@ -143,7 +153,7 @@ k_face_prep(const uint8_t *__restrict__ src, int sw, int sh, int sstride, int cn
         gray[(size_t)y * dw + x] = (uint8_t)g;
         atomicAdd(&sh_hist[g], 1);
     }
-    prep_finish(tid, sh_hist, hist, lut, dw * dh);
+    prep_finish<BATCH>(tid, sh_hist, hist, lut, dw * dh);
 }
 
 // Vectorised forms of the two streaming modes (same size, exact 2x): a lane owns FOUR consecutive output pixels, reads
@@ -153,12 +163,17 @@ k_face_prep(const uint8_t *__restrict__ src, int sw, int sh, int sstride, int cn
 // byte-per-lane kernel above runs.
 __device__ __forceinline__ int byte_of(uint32_t w, int i) { return (int)((w >> (8 * i)) & 255u); }
 
-template <int MODE>
+template <int MODE, bool BATCH>
 __global__ void __launch_bounds__(256)
 k_face_prep_bgr4(const uint8_t *__restrict__ src, int sstride, uint8_t *__restrict__ gray, int dw, int dh,
-                 int *__restrict__ hist, uint8_t *__restrict__ lut)
+                 int *__restrict__ hist, uint8_t *__restrict__ lut, const uint8_t *const *__restrict__ srcs = nullptr,
+                 size_t gray_stride = 0)
 {
     __shared__ int sh_hist[256];
+    if (BATCH) {
+        src = srcs[blockIdx.y];
+        gray += blockIdx.y * gray_stride; hist += blockIdx.y * NV_HIST_STRIDE; lut += blockIdx.y * 256;
+    }
     int tid = threadIdx.y * 32 + threadIdx.x;
     sh_hist[tid] = 0;
     __syncthreads();
@@ -197,7 +212,7 @@ k_face_prep_bgr4(const uint8_t *__restrict__ src, int sstride, uint8_t *__restri
 #pragma unroll
         for (int k = 0; k < 4; k++) atomicAdd(&sh_hist[g[k]], 1);
     }
-    prep_finish(tid, sh_hist, hist, lut, dw * dh);
+    prep_finish<BATCH>(tid, sh_hist, hist, lut, dw * dh);
 }
 
 // ---- 4:2:0 ingest (SURVEY §8f rank 4): the same block fed by I420 / NV12 / NV21 planes.  Every source pixel the
@@ -440,12 +455,28 @@ cudaError_t launch_face_prep(const uint8_t *src, int sw, int sh, int sstride, in
     const int mode = (sw == dw && sh == dh) ? RT_COPY : (sw == 2 * dw && sh == 2 * dh) ? RT_BOX2 : RT_LINEAR;   // = rtab[0]
     if (mode != RT_LINEAR && cn == 3 && (dw & 3) == 0 && aligned4(src, sstride) && aligned4(gray, 0)) {
         int tiles = ((dw / 4 + 31) / 32) * ((dh + 7) / 8);
-        if (mode == RT_COPY) k_face_prep_bgr4<RT_COPY><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sstride, gray, dw, dh, hist, lut);
-        else k_face_prep_bgr4<RT_BOX2><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sstride, gray, dw, dh, hist, lut);
+        if (mode == RT_COPY) k_face_prep_bgr4<RT_COPY, false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sstride, gray, dw, dh, hist, lut);
+        else k_face_prep_bgr4<RT_BOX2, false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sstride, gray, dw, dh, hist, lut);
         return cudaGetLastError();
     }
     int tiles = ((dw + 31) / 32) * ((dh + 7) / 8);
-    k_face_prep<<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sw, sh, sstride, cn, gray, dw, dh, rtab, hist, lut);
+    k_face_prep<false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(src, sw, sh, sstride, cn, gray, dw, dh, rtab, hist, lut);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_face_prep_batch(const uint8_t *const *srcs, int n, bool aligned, int sw, int sh, int sstride, uint8_t *gray,
+                                   int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st)
+{
+    const int mode = (sw == dw && sh == dh) ? RT_COPY : (sw == 2 * dw && sh == 2 * dh) ? RT_BOX2 : RT_LINEAR;   // = rtab[0]
+    const size_t gs = (size_t)dw * dh;
+    if (mode != RT_LINEAR && (dw & 3) == 0 && aligned) {
+        const dim3 grid(prep_grid(((dw / 4 + 31) / 32) * ((dh + 7) / 8)), n);
+        if (mode == RT_COPY) k_face_prep_bgr4<RT_COPY, true><<<grid, dim3(32, 8), 0, st>>>(nullptr, sstride, gray, dw, dh, hist, lut, srcs, gs);
+        else k_face_prep_bgr4<RT_BOX2, true><<<grid, dim3(32, 8), 0, st>>>(nullptr, sstride, gray, dw, dh, hist, lut, srcs, gs);
+        return cudaGetLastError();
+    }
+    const dim3 grid(prep_grid(((dw + 31) / 32) * ((dh + 7) / 8)), n);
+    k_face_prep<true><<<grid, dim3(32, 8), 0, st>>>(nullptr, sw, sh, sstride, 3, gray, dw, dh, rtab, hist, lut, srcs, gs);
     return cudaGetLastError();
 }
 template <int FMT>

@@ -24,13 +24,19 @@ __device__ __forceinline__ int find_level(const PlanDev *__restrict__ plan, int 
 // 8-byte stores on the de-interleaved ystep-2 layout: columns c, c + 2 are neighbours in the even plane, c + 1, c + 3
 // in the odd one).  Round 1's kernel did one pixel per lane: 3.4 x the instructions, and a 1920-pixel row was a chain
 // of 60 dependent load -> scan -> carry rounds where this one has 15.
-__global__ void __launch_bounds__(256, 8)                        // 32 registers, no spills: eight blocks per SM (40.3 -> 38.9 us alone)
+// BATCH: image blockIdx.y reads grays[blockIdx.y] through the LUT at blockIdx.y * lut_stride and writes the integrals at
+// blockIdx.y * integ_stride elements.
+template <bool BATCH>
+// 32 registers, no spills: eight blocks per SM (40.3 -> 38.9 us alone); the batched form needs 40 (six blocks per SM) not to spill
+__global__ void __launch_bounds__(256, BATCH ? 6 : 8)
 k_pyr_rowscan(const PlanDev *__restrict__ plan, const uint8_t *__restrict__ gray, int gstride,
               const uint8_t *__restrict__ lut, const int2 *__restrict__ ptab, uint32_t *__restrict__ sum,
-              uint32_t *__restrict__ sq, uint8_t *__restrict__ pyr_debug)
+              uint32_t *__restrict__ sq, uint8_t *__restrict__ pyr_debug, const uint8_t *const *__restrict__ grays = nullptr,
+              int lut_stride = 0, unsigned integ_stride = 0)
 {
     __shared__ uint8_t s_lut[256];
     int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (BATCH) lut += blockIdx.y * lut_stride;
     s_lut[tid] = lut[tid];
     __syncthreads();
 
@@ -39,7 +45,8 @@ k_pyr_rowscan(const PlanDev *__restrict__ plan, const uint8_t *__restrict__ gray
     const int lw = L.lw, lh = L.lh, ys = L.ystep, pitch = L.ipitch, plane = L.iplane;
     int y = (blockIdx.x - L.rowblk0) * 8 + warp;
     if (y >= lh) return;
-    uint32_t *srow = sum + L.iofs, *qrow = sq + L.iofs;
+    const size_t iofs = L.iofs + (BATCH ? (size_t)blockIdx.y * integ_stride : 0);
+    uint32_t *srow = sum + iofs, *qrow = sq + iofs;
     if (y == 0)                                         // first integral row is all zeros (pitch is a multiple of 4)
         for (int c = lane * 4; c < pitch; c += 128) {
             *reinterpret_cast<uint4 *>(srow + c) = make_uint4(0, 0, 0, 0);
@@ -50,6 +57,7 @@ k_pyr_rowscan(const PlanDev *__restrict__ plan, const uint8_t *__restrict__ gray
 
     const int4 *xt = reinterpret_cast<const int4 *>(ptab + L.xtab);     // two (index, fraction) entries per int4
     int2 ty = (ptab + L.ytab)[y];
+    if (BATCH) gray = grays[blockIdx.y];
     const uint8_t *g0 = gray + (size_t)ty.x * gstride, *g1 = g0 + gstride;
     const uint32_t r1 = (uint32_t)ty.y, r0 = 256u - r1;
     uint32_t carry_s = 0, carry_q = 0;
@@ -116,14 +124,17 @@ __device__ __forceinline__ uint4 add4(uint4 a, uint4 b) { return make_uint4(a.x 
 #ifndef NV_COLBANDS
 #define NV_COLBANDS 16
 #endif
-__global__ void __launch_bounds__(32 * NV_COLBANDS)
-k_colscan(const PlanDev *__restrict__ plan, int total_colblk, uint32_t *__restrict__ sum, uint32_t *__restrict__ sq)
+template <bool BATCH>                                             // BATCH: image blockIdx.y, integrals at blockIdx.y * integ_stride
+__global__ void __launch_bounds__(32 * NV_COLBANDS, BATCH ? 2 : 0)   // the batched form spills at the 40 registers ptxas picks unbounded
+k_colscan(const PlanDev *__restrict__ plan, int total_colblk, uint32_t *__restrict__ sum, uint32_t *__restrict__ sq,
+          unsigned integ_stride = 0)
 {
     __shared__ uint4 tot[NV_COLBANDS][33];
     int lane = threadIdx.x & 31, band = threadIdx.x >> 5;
     int b = blockIdx.x;
     uint32_t *arr = sum;
     if (b >= total_colblk) { b -= total_colblk; arr = sq; }
+    if (BATCH) arr += (size_t)blockIdx.y * integ_stride;
     int l = find_level(plan, b, &LevelDesc::colblk0);
     const LevelDesc &L = plan->lv[l];
     const int pitch = L.ipitch, rows = L.lh + 1;
@@ -223,12 +234,22 @@ cudaError_t launch_tilted(const PlanDev *plan, int total_dblk, const uint32_t *s
 cudaError_t launch_pyr_rowscan(const PlanDev *plan, int total_rowblk, const uint8_t *gray, int gstride, const uint8_t *lut,
                                const int *ptab, uint32_t *sum, uint32_t *sq, uint8_t *pyr_debug, cudaStream_t st)
 {
-    k_pyr_rowscan<<<total_rowblk, 256, 0, st>>>(plan, gray, gstride, lut, (const int2 *)ptab, sum, sq, pyr_debug);
+    k_pyr_rowscan<false><<<total_rowblk, 256, 0, st>>>(plan, gray, gstride, lut, (const int2 *)ptab, sum, sq, pyr_debug);
     return cudaGetLastError();
 }
 
 cudaError_t launch_colscan(const PlanDev *plan, int total_colblk, uint32_t *sum, uint32_t *sq, cudaStream_t st)
 {
-    k_colscan<<<2 * total_colblk, 32 * NV_COLBANDS, 0, st>>>(plan, total_colblk, sum, sq);
+    k_colscan<false><<<2 * total_colblk, 32 * NV_COLBANDS, 0, st>>>(plan, total_colblk, sum, sq);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_pyramid_batch(const PlanDev *plan, int total_rowblk, int total_colblk, int n, const uint8_t *const *grays, int gstride,
+                                 const uint8_t *lut, int lut_stride, const int *ptab, uint32_t *sum, uint32_t *sq, size_t integ_stride,
+                                 cudaStream_t st)
+{
+    k_pyr_rowscan<true><<<dim3(total_rowblk, n), 256, 0, st>>>(plan, nullptr, gstride, lut, (const int2 *)ptab, sum, sq, nullptr, grays,
+                                                               lut_stride, (unsigned)integ_stride);
+    k_colscan<true><<<dim3(2 * total_colblk, n), 32 * NV_COLBANDS, 0, st>>>(plan, total_colblk, sum, sq, (unsigned)integ_stride);
     return cudaGetLastError();
 }

@@ -149,7 +149,12 @@ _SIGS = {
     "nv_debug_get_depth_map": (_i, [_vp, _i, _vp]),
     "nv_debug_get_candidates": (_i, [_vp, _vp, _i, _ip]),
     "nv_debug_get_counters": (_i, [_vp, C.POINTER(C.c_longlong)]),
+    "nv_detect_multiscale_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(DetectParams), _vp, _i, _ip]),
+    "nv_face_submit_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(FaceParams)]),
+    "nv_face_collect_batch": (_i, [_vp, _vp, _i, _ip, _ip]),
+    "nv_face_detect_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(FaceParams), _vp, _i, _ip, _ip]),
 }
+BATCH_MAX = 256           # NV_BATCH_MAX
 EXPORTS = sorted(_SIGS)
 for _name, (_res, _args) in _SIGS.items():
     _f = getattr(_lib, _name)          # AttributeError here = a declared symbol is not exported
@@ -185,6 +190,41 @@ def _u8(a):
 
 def _rects(buf, n):
     return np.frombuffer(buf, dtype=np.int32, count=4 * n).reshape(n, 4).copy()
+
+
+def _batch_frames(images, cn):
+    """(pointer table, n, w, h, row stride, on_device, keep-alive) of a batch: a uint8 numpy array or CUDA torch tensor
+    [N, H, W] (cn == 1) / [N, H, W, 3] (cn == 3) whose pixels are packed within a row; rows and images may be further
+    apart than packed.  A torch tensor's stream is synchronised here, so the library reads finished frames."""
+    ndim = 3 if cn == 1 else 4
+    if type(images).__module__.startswith("torch"):
+        import torch
+        if images.dtype != torch.uint8:
+            raise TypeError(f"batch must be a uint8 tensor, got {images.dtype}")
+        if images.dim() != ndim or (cn == 3 and images.shape[3] != 3):
+            raise ValueError(f"batch tensor must be [N, H, W{', 3' if cn == 3 else ''}], got {tuple(images.shape)}")
+        if not images.is_cuda:
+            images = images.numpy()
+        else:
+            if images.stride(2) != cn or (cn == 3 and images.stride(3) != 1):
+                raise ValueError("the pixels of a row must be packed (stride(2) == channels)")
+            n, h, w = images.shape[:3]
+            torch.cuda.current_stream(images.device).synchronize()
+            base = images.data_ptr()
+            ptrs = (C.c_void_p * max(n, 1))(*[base + i * images.stride(0) for i in range(n)])
+            return ptrs, n, w, h, images.stride(1), 1, images
+    if not isinstance(images, np.ndarray) or images.dtype != np.uint8:
+        raise TypeError("batch must be a uint8 numpy array or a CUDA torch tensor")
+    shape, strides = images.shape, images.strides
+    if len(shape) != ndim or (cn == 3 and shape[3] != 3):
+        raise ValueError(f"batch array must be [N, H, W{', 3' if cn == 3 else ''}], got {shape}")
+    if strides[2] != cn or (cn == 3 and strides[3] != 1) or min(strides) < 0:
+        images = np.ascontiguousarray(images)
+        strides = images.strides
+    n, h, w = shape[:3]
+    base, s0 = images.ctypes.data, strides[0]
+    ptrs = (C.c_void_p * max(n, 1))(*range(base, base + n * s0, s0)) if s0 else (C.c_void_p * max(n, 1))(*([base] * n))
+    return ptrs, n, w, h, strides[1], 0, images
 
 
 NUM_STAGES = 8
@@ -491,6 +531,50 @@ class Context:
         p = self._face_params(width_to_process, scale_factor, min_neighbors, min_size)
         _check(_lib.nv_face_submit_device(self.handle, casc.handle, _vp(dev_ptr), w, h, stride, C.byref(p)),
                "nv_face_submit_device")
+
+    # ---- batches: N same-size images per call (see nubovca.h).  images: a uint8 numpy array or CUDA torch tensor
+    #      [N, H, W] (gray) / [N, H, W, 3] (BGR); a torch tensor's current stream is synchronised before the submit.
+    #      Returns a list of N int32 arrays [k, 4], image by image.
+    def _batch_out(self, counts):
+        flat = np.frombuffer(self._bout, dtype=np.int32, count=4 * sum(counts)).reshape(-1, 4)
+        out, o = [], 0
+        for k in counts:
+            out.append(flat[o:o + k].copy())
+            o += k
+        return out
+
+    def _batch_buffers(self, n):
+        self._bcounts = (C.c_int * max(n, 1))()
+        if not hasattr(self, "_bout"):
+            self._bout = (Rect * (1 << 20))()
+
+    def detect_multiscale_batch(self, casc: Cascade, images, scale_factor=1.1, min_neighbors=3, min_size=(0, 0), max_size=(0, 0)):
+        ptrs, n, w, h, stride, dev, keep = _batch_frames(images, 1)
+        p = DetectParams(scale_factor, min_neighbors, 0, min_size[0], min_size[1], max_size[0], max_size[1])
+        self._batch_buffers(n)
+        _check(_lib.nv_detect_multiscale_batch(self.handle, casc.handle, ptrs, n, w, h, stride, dev, C.byref(p), self._bout,
+                                               len(self._bout), self._bcounts), "nv_detect_multiscale_batch")
+        return self._batch_out(self._bcounts[:n])
+
+    def face_submit_batch(self, casc: Cascade, frames, width_to_process=160, scale_factor=1.25, min_neighbors=3, min_size=None):
+        ptrs, n, w, h, stride, dev, keep = _batch_frames(frames, 3)
+        p = self._face_params(width_to_process, scale_factor, min_neighbors, min_size)
+        self._batch_buffers(n)
+        _check(_lib.nv_face_submit_batch(self.handle, casc.handle, ptrs, n, w, h, stride, dev, C.byref(p)), "nv_face_submit_batch")
+        self._batch_keep, self._batch_n = keep, n          # page-locked / device frames are read until collect
+
+    def face_collect_batch(self):
+        total = C.c_int(0)
+        try:
+            _check(_lib.nv_face_collect_batch(self.handle, self._bout, len(self._bout), self._bcounts, C.byref(total)),
+                   "nv_face_collect_batch")
+        finally:
+            self._batch_keep = None
+        return self._batch_out(self._bcounts[:self._batch_n])
+
+    def face_detect_batch(self, casc: Cascade, frames, width_to_process=160, scale_factor=1.25, min_neighbors=3, min_size=None):
+        self.face_submit_batch(casc, frames, width_to_process, scale_factor, min_neighbors, min_size)
+        return self.face_collect_batch()
 
     # ---- 4:2:0 ingest: planes = (y, u, v) for I420 (YV12: pass the planes in I420 meaning), (y, uv) for NV12 / NV21;
     #      each a 2-D uint8 array with unit column stride (row strides are honoured)
