@@ -508,8 +508,6 @@ static int ensure_plan(nv_ctx *ctx, const nv_cascade *casc, int W, int H, const 
         if (scales.size() > 4096) break;
     }
     int nstripes = 1;
-    for (int c = 0; c < 2; c++)
-        if (!nv_wide_tile_config(c, &P.wide_w[c], &P.wide_h[c])) P.wide_w[c] = P.wide_h[c] = 0;
     long long iofs = 0, wofs = 0, bofs = 0, tofs = 0, pofs = 0;
     int nl = 0;
     for (size_t k = 0; k < scales.size(); k++) {
@@ -546,10 +544,9 @@ static int ensure_plan(nv_ctx *ctx, const nv_cascade *casc, int W, int H, const 
         if (ystep == 2) { L.ctile0 = P.ctiles2; P.ctiles2 += cnt; P.nlv2 = nl; }
         else { L.ctile0 = P.ctiles1; P.ctiles1 += cnt; }
         L.wtile0 = 0; L.wntx = 0;
-        const int wc = ystep == 2 ? 0 : 1;
-        if (P.wide_w[wc] > 0) {
-            L.wntx = (L.nx + P.wide_w[wc] - 1) / P.wide_w[wc];
-            L.wtile0 = P.wtiles[wc]; P.wtiles[wc] += L.wntx * ((L.ny + P.wide_h[wc] - 1) / P.wide_h[wc]);
+        if (ystep == 1) {
+            L.wntx = (L.nx + NV_WTX - 1) / NV_WTX;
+            L.wtile0 = P.wtiles[1]; P.wtiles[1] += L.wntx * ((L.ny + NV_WTY - 1) / NV_WTY);
         }
         if (iofs > 0x7fffffffLL || wofs > 0x7fffffffLL) { nv_set_error("frame too large"); return NV_ERR_CAPACITY; }
     }
@@ -662,8 +659,7 @@ static int ensure_tile_params(nv_ctx *ctx, const nv_cascade *casc)
             return g;
         };
         const Geo g0 = geometry(NV_CTX, NV_CTY);
-        const bool wide = P.wide_w[c] > 0;
-        const Geo g = wide ? geometry(P.wide_w[c], P.wide_h[c]) : g0;
+        const Geo g = ys == 1 ? geometry(NV_WTX, NV_WTY) : g0;
         if (g.cp > 256 || g.rt > 256) return NV_OK;             // TMA box limit: keep the generic queue path
         tp.cp = g.cp; tp.rt = g.rt; tp.kskew = g.kskew; tp.ps = g.ps;
         tp.level_begin = c == 0 ? 0 : P.nlv2;
@@ -764,27 +760,18 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
         NV_CUDA(launch_colscan(ctx->ps->d_plan, P.total_colblk, ctx->d_sum, ctx->d_sq, st));
         if (tilt) { NV_CUDA(launch_tilted(ctx->ps->d_plan, P.total_dblk, ctx->d_sum, ctx->d_tilt, st)); nl += 2; }
         prof_mark(ctx, 4);
-        static const int small_limit = [] { const char *e = getenv("NUBOVCA_SMALL_PLAN"); return e ? atoi(e) : NV_SMALL_PLAN_WINDOWS; }();
-        static const bool s0_tiles = [] { const char *e = getenv("NUBOVCA_S0_TILES"); return !e || atoi(e) != 0; }();
-        // k_cascade_tail_tab (classifier table in shared memory): 1 large plans, 2 small plans up to the block-per-window split,
-        // 4 small plans through all stages (no k_cascade_tail_block launch).  Measured (profiles/r2_summary.md section 8):
-        // small plans gain (a 96x64 ROI detect 100.6 -> 88.5 us per call, eyes-in-faces 374 -> 359 us), config 3 does not
-        // (tail 45 -> 49 / 45 / 41 us with 8 / 16 / 32 warps per block, bench.py -1 .. -4 %: fewer resident warps for its
-        // 15 000 shallow windows, and 84 KB blocks queue behind the bulk kernels of the other streams) — default 4.
-        static const int tail_tab = [] { const char *e = getenv("NUBOVCA_TAIL_TAB"); return e ? atoi(e) : 4; }();
-        static const bool two_streams = [] { const char *e = getenv("NUBOVCA_TWO_STREAMS"); return !e || atoi(e) != 0; }();
         // small plan of a cascade with the certificates: every window alive after stage 0 goes to the warp-per-window kernel;
         // k_stage0_rows_p appends them to its queue itself
-        const bool small_fast = ctx->ps->use_tiles && ctx->cur_tail && P.total_windows <= small_limit && casc->meta.nstages > 1;
+        const bool small_fast = ctx->ps->use_tiles && ctx->cur_tail && P.total_windows <= NV_SMALL_PLAN_WINDOWS && casc->meta.nstages > 1;
         const int qcap = (int)std::min<size_t>(ctx->queue_cap, 0x7fffffff);
         bool queued = false;
         if (ctx->use_gen) {
             NV_CUDA(launch_stage0_rows_gen(ctx->ps->d_plan, P.total_rows, meta, ctx->cur_gen, ctx->d_sum, ctx->d_sq, tilt, ctx->d_vnf,
                                            ctx->d_bits_ok, ctx->d_counters, depth, st));
-        } else if (ctx->ps->use_tiles && ctx->ps->use_s0t && s0_tiles && P.total_windows > small_limit) {
+        } else if (ctx->ps->use_tiles && ctx->ps->use_s0t && P.total_windows > NV_SMALL_PLAN_WINDOWS) {
             // large plan, FAST cascade: stage 0 densely on the bulk kernel's tiles, then the skip rule along the rows
             uint32_t *bits_fail = ctx->d_bits_ok + ctx->ps->bits_words, *bits_okv = ctx->d_bits_ok + 2 * (size_t)ctx->ps->bits_words;
-            const bool fork = two_streams && P.ctiles2 > 0 && P.ctiles1 > 0;      // the ystep-1 levels' launch goes to the side stream
+            const bool fork = P.ctiles2 > 0 && P.ctiles1 > 0;      // the ystep-1 levels' launch goes to the side stream
             if (fork) { NV_CUDA(cudaEventRecord(ctx->ev_fork[0], st)); NV_CUDA(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork[0], 0)); }
             for (int c = 0; c < 2; c++) {
                 Stage0TileParams &s0 = ctx->ps->s0t[c];
@@ -818,11 +805,13 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
                 nl++;
             }
             prof_mark(ctx, 6);
-            // stages narrower than NV_TAIL_BLOCK_MIN_STUMPS with a warp per window, the deep ones with a block per window
+            // stages narrower than NV_TAIL_BLOCK_MIN_STUMPS with a warp per window, the deep ones with a block per window —
+            // unless the whole classifier table fits shared memory: then k_cascade_tail_tab takes every stage (measured,
+            // profiles/r2_summary.md section 8: a 96x64 ROI detect 100.6 -> 88.5 us per call, eyes-in-faces 374 -> 359 us)
             int split = 1;
             while (split < casc->meta.nstages && casc->meta.stage_first[split + 1] - casc->meta.stage_first[split] < NV_TAIL_BLOCK_MIN_STUMPS) split++;
-            if ((tail_tab & 4) && tail_tab_smem(casc->meta, 1, casc->meta.nstages) <= NV_TAILTAB_MAX_SMEM) split = casc->meta.nstages;
-            if ((tail_tab & 6) && tail_tab_smem(casc->meta, 1, split) <= NV_TAILTAB_MAX_SMEM)
+            if (tail_tab_smem(casc->meta, 1, casc->meta.nstages) <= NV_TAILTAB_MAX_SMEM) split = casc->meta.nstages;
+            if (tail_tab_smem(casc->meta, 1, split) <= NV_TAILTAB_MAX_SMEM)
                 NV_CUDA(launch_cascade_tail_tab(ctx->ps->d_plan, meta, casc->meta, ctx->cur_tail, ctx->cur_tail_base, ctx->d_sum, ctx->d_queue,
                                                 ctx->d_counters, ctx->d_cand, ctx->cand_cap, depth, 1, split, ctx->d_deepq, NV_DEEPQ_CAP, st));
             else
@@ -836,42 +825,37 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
                 nl++;
             }
         } else if (ctx->ps->use_tiles) {
-            const bool fork = two_streams && P.ctiles2 > 0 && P.ctiles1 > 0;
+            const bool fork = P.ctiles2 > 0 && P.ctiles1 > 0;
             if (fork) { NV_CUDA(cudaEventRecord(ctx->ev_fork[1], st)); NV_CUDA(cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork[1], 0)); }
-            // Launch order decides what the two kernels share.  The ystep-2 levels first (default): their 742 blocks fill every
-            // SM's shared memory and the wide blocks of the ystep-1 levels follow as they drain — 2970 frames/s with eight
-            // frames in flight, bulk stages 0.34 ms when a frame is alone.  NUBOVCA_FORK_ORDER=1, the ystep-1 levels first:
-            // their 368 wide blocks leave room for a block of the other kernel on every SM, so a lone frame's bulk stages
-            // take 0.27 ms, but eight frames in flight lose 4 % (2845 frames/s).
-            static const bool wide_first = [] { const char *e = getenv("NUBOVCA_FORK_ORDER"); return e && atoi(e) != 0; }();
-            for (int k = 0; k < 2; k++) {
-                const int c = wide_first ? 1 - k : k;
+            // Launch order decides what the two kernels share.  The ystep-2 levels first: their 742 blocks fill every SM's
+            // shared memory and the wide blocks of the ystep-1 levels follow as they drain — 2970 frames/s with eight frames
+            // in flight, bulk stages 0.34 ms when a frame is alone.  The ystep-1 levels first was measured: their 368 wide
+            // blocks leave room for a block of the other kernel on every SM, so a lone frame's bulk stages take 0.27 ms, but
+            // eight frames in flight lose 4 % (2845 frames/s).
+            for (int c = 0; c < 2; c++) {
                 TileParams &tp = ctx->ps->tp[c];
-                const cudaStream_t cst = k == 1 && fork ? ctx->stream2 : st;
-                int ntiles = c == 0 ? P.ctiles2 : P.ctiles1;
-                if (ntiles == 0) continue;
+                const cudaStream_t cst = c == 1 && fork ? ctx->stream2 : st;
+                if ((c == 0 ? P.ctiles2 : P.ctiles1) == 0) continue;
                 tp.plan = ctx->ps->d_plan; tp.bits_alive = ctx->d_bits_ok; tp.vnf = ctx->d_vnf; tp.depth = depth;
                 tp.tail = ctx->d_queue; tp.cand = ctx->d_cand; tp.counters = ctx->d_counters; tp.maps = ctx->ps->d_maps;
                 tp.tail_cap = qcap; tp.cand_cap = ctx->cand_cap;
-                if (P.wide_w[c] > 0) NV_CUDA(launch_cascade_wide(tp, c == 0 ? 2 : 1, P.wide_w[c], P.wide_h[c], P.wtiles[c], cst));
-                else NV_CUDA(launch_cascade_classes(tp, c == 0 ? 2 : 1, ntiles, cst));
+                if (c == 0) NV_CUDA(launch_cascade_classes(tp, P.ctiles2, cst));
+                else NV_CUDA(launch_cascade_wide(tp, P.wtiles[1], cst));
                 nl++;
             }
             if (fork) { NV_CUDA(cudaEventRecord(ctx->ev_join[1], ctx->stream2)); NV_CUDA(cudaStreamWaitEvent(st, ctx->ev_join[1], 0)); }
             prof_mark(ctx, 6);
             if (ctx->ps->bulk_end < casc->meta.nstages && ctx->cur_tail) {
                 // the survivors of the bulk stages (~15 000 per config-3 frame, most of them gone within a few stages): a warp
-                // per window.  (Handing the deep ones to the block-per-window kernel after NV_TAIL_WARP_STAGES stages was
-                // measured: 55 us against 45 us isolated, 2538 against 2577 frames/s — with that many windows the warp kernel
-                // is bound by throughput, not by its deepest window; the split pays on small plans only.)
-                if ((tail_tab & 1) && tail_tab_smem(casc->meta, ctx->ps->bulk_end, casc->meta.nstages) <= NV_TAILTAB_MAX_SMEM)
-                    NV_CUDA(launch_cascade_tail_tab(ctx->ps->d_plan, meta, casc->meta, ctx->cur_tail, ctx->cur_tail_base, ctx->d_sum, ctx->d_queue,
-                                                    ctx->d_counters, ctx->d_cand, ctx->cand_cap, depth, ctx->ps->bulk_end, casc->meta.nstages,
-                                                    nullptr, qcap, st));
-                else
-                    NV_CUDA(launch_cascade_tail_fast(ctx->ps->d_plan, meta, ctx->cur_tail, ctx->cur_tail_base, ctx->d_sum, ctx->d_queue,
-                                                     ctx->d_counters, ctx->d_cand, ctx->cand_cap, depth, ctx->ps->bulk_end, casc->meta.nstages,
-                                                     nullptr, qcap, st, 8 * (casc->meta.win_w + 1) * (casc->meta.win_h + 1) * 4));
+                // per window.  (Handing the deep ones to the block-per-window kernel after four stages was measured: 55 us
+                // against 45 us isolated, 2538 against 2577 frames/s — with that many windows the warp kernel is bound by
+                // throughput, not by its deepest window; the split pays on small plans only.  Nor does k_cascade_tail_tab pay
+                // here, profiles/r2_summary.md section 8: tail 45 -> 49 / 45 / 41 us with 8 / 16 / 32 warps per block, bench.py
+                // -1 .. -4 % — fewer resident warps for these shallow windows, and 84 KB blocks queue behind the bulk kernels of
+                // the other streams.)
+                NV_CUDA(launch_cascade_tail_fast(ctx->ps->d_plan, meta, ctx->cur_tail, ctx->cur_tail_base, ctx->d_sum, ctx->d_queue,
+                                                 ctx->d_counters, ctx->d_cand, ctx->cand_cap, depth, ctx->ps->bulk_end, casc->meta.nstages,
+                                                 nullptr, qcap, st, 8 * (casc->meta.win_w + 1) * (casc->meta.win_h + 1) * 4));
                 nl++;
             } else if (ctx->ps->bulk_end < casc->meta.nstages) {
                 NV_CUDA(launch_cascade_tail(ctx->ps->d_plan, meta, stumps, ctx->d_sum, ctx->d_queue, ctx->d_counters, ctx->d_cand,
@@ -883,7 +867,7 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
             NV_CUDA(launch_alive_to_queue(ctx->ps->d_plan, P.total_rows, ctx->d_vnf, ctx->d_bits_ok, ctx->d_queue, ctx->d_counters,
                                           qcap, st));
             prof_mark(ctx, 6);
-            if (ctx->use_gen && P.total_windows > small_limit && ctx->d_queue2 && ctx->queue2_cap >= ctx->queue_cap && casc->meta.nstages > 1) {
+            if (ctx->use_gen && P.total_windows > NV_SMALL_PLAN_WINDOWS && ctx->d_queue2 && ctx->queue2_cap >= ctx->queue_cap && casc->meta.nstages > 1) {
                 int extra = 0;                                   // large plan: stage-wise compaction between thread-per-window passes
                 NV_CUDA(launch_queue_stages_gen_staged(ctx->ps->d_plan, meta, ctx->cur_gen, ctx->d_sum, tilt, ctx->d_queue, ctx->d_queue2, qcap,
                                                        ctx->d_counters, ctx->d_cand, ctx->cand_cap, depth, casc->meta.nstages,
@@ -899,29 +883,15 @@ static int detect_enqueue(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, 
         }
     }
     prof_mark(ctx, 7);
-    static const bool host_writes = [] { const char *e = getenv("NUBOVCA_HOST_WRITES"); return !e || atoi(e) != 0; }();
-    // small plans: sort + similarity matrix + grouping in one launch of one block (k_group_fused)
-    static const bool group_fused = [] { const char *e = getenv("NUBOVCA_GROUP_FUSED"); return !e || atoi(e) != 0; }();
-    static const int small_limit_g = [] { const char *e = getenv("NUBOVCA_SMALL_PLAN"); return e ? atoi(e) : NV_SMALL_PLAN_WINDOWS; }();
     const ScoreArgs sa = {ctx->cur_meta, ctx->cur_stumps, ctx->use_gen ? ctx->cur_gen : GenModel{}, ctx->use_gen ? 1 : 0, ctx->d_sum, ctx->d_sq,
                           ctx->use_gen && ctx->cur_tilted ? ctx->d_tilt : nullptr, ctx->d_cand_w, ctx->d_cls_wmax};
+    // small plans: sort + similarity matrix + grouping in one launch of one block (k_group_fused).  The grouping kernel writes
+    // header and rectangles into the page-locked result block itself (mapped memory, posted writes over PCIe, visible once
+    // the stream has been waited for): no device-to-host copy behind it.
     NV_CUDA(launch_group(ctx->ps->d_plan, ctx->d_counters, ctx->d_cand, ctx->cand_cap, ctx->d_cand_sorted, ctx->d_cand_rects,
                          ctx->d_adj, ctx->d_grp, p->min_neighbors, 0.2, W, H, ctx->d_result, ctx->result_cap, 148 * 2, st, &nl,
-                         group_fused && P.total_windows <= small_limit_g, host_writes ? ctx->h_result : nullptr,
-                         ctx->scores ? &sa : nullptr));
+                         P.total_windows <= NV_SMALL_PLAN_WINDOWS, ctx->h_result, ctx->scores ? &sa : nullptr));
     prof_mark(ctx, 8);
-    // the grouping kernel writes header and rectangles into the page-locked result block itself (mapped memory, posted
-    // writes over PCIe, visible once the stream has been waited for): no device-to-host copy behind it.
-    // NUBOVCA_HOST_WRITES=0: the copy (what every call did before).
-    if (!host_writes) {
-        NV_CUDA(cudaMemcpyAsync(ctx->h_result, ctx->d_result, sizeof(ResultHeader) + NV_RESULT_INLINE * sizeof(nv_rect),
-                                cudaMemcpyDeviceToHost, st));
-        if (ctx->scores) {
-            const size_t wofs = sizeof(ResultHeader) + (size_t)ctx->result_cap * sizeof(nv_rect), nofs = wofs + (size_t)ctx->result_cap * sizeof(double);
-            NV_CUDA(cudaMemcpyAsync(ctx->h_result + wofs, ctx->d_result + wofs, NV_RESULT_INLINE * sizeof(double), cudaMemcpyDeviceToHost, st));
-            NV_CUDA(cudaMemcpyAsync(ctx->h_result + nofs, ctx->d_result + nofs, NV_RESULT_INLINE * sizeof(int), cudaMemcpyDeviceToHost, st));
-        }
-    }
     *nlaunch += nl;
     counters_guard.done = true;
     return NV_OK;
@@ -1968,10 +1938,7 @@ static int tracker_impl(nv_ctx *ctx, const FaceSrc &src, int width, int height, 
     std::vector<nv_rect> v;
     if (!first) {
         const int4 *d_out = reinterpret_cast<const int4 *>(ctx->d_trk_scratch + ctx->trk_lo.out);
-        // count and the first 1024 rectangles: written into h_trk by the kernel's last block (mapped memory) unless
-        // NUBOVCA_HOST_WRITES=0 asks for the copy
-        static const bool host_writes = [] { const char *e = getenv("NUBOVCA_HOST_WRITES"); return !e || atoi(e) != 0; }();
-        if (!host_writes) NV_CUDA(cudaMemcpyAsync(ctx->h_trk, d_out, (1 + 1024) * sizeof(int4), cudaMemcpyDeviceToHost, ctx->stream));
+        // count and the first 1024 rectangles: written into h_trk by the kernel's last block (mapped memory)
         NV_CUDA(cudaStreamSynchronize(ctx->stream));
         const int4 *h = reinterpret_cast<const int4 *>(ctx->h_trk);
         total = h[0].x;

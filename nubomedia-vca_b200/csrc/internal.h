@@ -18,7 +18,6 @@
 #define NV_DEEPQ_CAP NV_SMALL_PLAN_WINDOWS   // a small plan has no more windows than that
 #define NV_TAILTAB_MAX_SMEM (200 * 1024)      // k_cascade_tail_tab: classifier table + window patches per block
 #define NV_TAIL_BLOCK_MIN_STUMPS 64            // stages at least this wide go to the block-per-window kernel
-#define NV_TAIL_WARP_STAGES 4                  // large plans: tail stages run with a warp per window before the block-per-window kernel takes over
 #define NV_COLBLK 128            // physical integral columns per block of the column scan
 #define NV_MAX_LEVELS 64          // level index is packed in 6 bits of a window id
 #define NV_MAX_STAGES 64
@@ -147,7 +146,7 @@ struct LevelDesc {
     int row0;              // first window row in k_stage0_rows' grid
     int dblk0;             // first block (256 diagonals) of this level in the tilted-integral kernels' grid
     int ctile0, cntx;      // k_cascade_classes: first 64x32-window tile within the ystep class, tile columns = ceil(nx/64)
-    int wtile0, wntx;      // k_cascade_wide: first tile of the level within its ystep class, tile columns = ceil(nx / wide_w[class])
+    int wtile0, wntx;      // k_cascade_wide: first tile of the level within its ystep class, tile columns = ceil(nx / NV_WTX)
 };
 
 struct PlanDev {
@@ -157,7 +156,7 @@ struct PlanDev {
     int total_rowblk, total_colblk, total_chunks, total_rows, total_windows;
     int nlv2;              // levels [0, nlv2) have ystep 2, [nlv2, nlevels) ystep 1 (scales ascend)
     int ctiles2, ctiles1;  // 64x32-window tile counts of the two ystep classes
-    int wtiles[2], wide_w[2], wide_h[2];   // k_cascade_wide: tile count and tile shape (windows) of the ystep-2 [0] / ystep-1 [1] levels; wide_w 0: class runs k_cascade_classes
+    int wtiles[2];         // k_cascade_wide: tile counts of the ystep-2 [0] / ystep-1 [1] levels (the ystep-2 levels run k_cascade_classes: 0)
     int total_dblk;        // blocks of the tilted-integral kernels
     LevelDesc lv[NV_MAX_LEVELS];
 };
@@ -182,15 +181,11 @@ struct ResizeKey {
 // stages' weak classifiers live in the constant bank, so they cost no load/store-unit bandwidth) ----
 #define NV_BULK_MAX_STUMPS 384
 #define NV_BULK_MAX_STAGES 16
-#ifndef NV_WIDE_DEFAULT                      // (w << 16) | h of k_cascade_wide's tiles; 0: the class runs k_cascade_classes (64x32)
-#define NV_WIDE_DEFAULT ((128 << 16) | 64)   // ystep-1 levels
-#endif
-#ifndef NV_WIDE2_DEFAULT
-#define NV_WIDE2_DEFAULT 0                   // ystep-2 levels stay on k_cascade_classes: two column planes per tile make a 64x64 tile 89 KB of
-                                             // shared memory (2800 against 2880 frames/s), and at 64x32 the interleaved ranks are 1 % ahead
-#endif
-#define NV_CTX 64                  // tile width and height in windows
+#define NV_CTX 64                  // k_stage0_tiles, k_cascade_classes: tile width and height in windows
 #define NV_CTY 32
+#define NV_WTX 128                 // k_cascade_wide (ystep-1 levels): tile width and height in windows.  The ystep-2 levels stay on
+#define NV_WTY 64                  // k_cascade_classes: two column planes per tile make a 64x64 tile 89 KB of shared memory (2800
+                                   // against 2880 frames/s), and at 64x32 the interleaved ranks are 1 % ahead
 
 // One bulk-stage weak classifier, 64 bytes, warp-uniform.  Offsets are BYTE offsets of the rect corners a, b, c, d
 // from the window's origin in the shared-memory tile.
@@ -479,9 +474,8 @@ cudaError_t launch_queue_stages_gen_staged(const PlanDev *plan, const DevCascade
                                            const uint32_t *tilt, uint2 *queue_a, uint2 *queue_b, int qcap, int *counters,
                                            uint32_t *cand, int cand_cap, int16_t *depth, int nstages, int order_free,
                                            cudaStream_t st, int *nlaunch);
-cudaError_t launch_cascade_classes(const TileParams &tp, int ystep, int ntiles, cudaStream_t st);
-bool nv_wide_tile_config(int cls, int *tw, int *th);  // tile shape of k_cascade_wide on ystep-2 (cls 0) / ystep-1 (cls 1) levels; false: k_cascade_classes
-cudaError_t launch_cascade_wide(const TileParams &tp, int ystep, int tw, int th, int ntiles, cudaStream_t st);
+cudaError_t launch_cascade_classes(const TileParams &tp, int ntiles, cudaStream_t st);   // ystep-2 levels
+cudaError_t launch_cascade_wide(const TileParams &tp, int ntiles, cudaStream_t st);      // ystep-1 levels
 cudaError_t launch_stage0_rows_p(const Stage0Params &sp, cudaStream_t st);
 bool fill_stage0_params(const nv_cascade *c, const PlanDev &P, Stage0Params *sp);
 cudaError_t launch_cascade_tail(const PlanDev *plan, const DevCascade *meta, const DevStump *stumps, const uint32_t *sum,

@@ -10,6 +10,8 @@
 // taller than 32); k_stage0_rows is the generic form of k_stage0_rows_p (more than 8 stage-0 classifiers).
 #include "cascade_eval.cuh"
 
+#include <set>
+
 __device__ __forceinline__ int find_level_c(const PlanDev *__restrict__ plan, int idx, int LevelDesc::*first)
 {
     int n = plan->nlevels, l = 0;
@@ -536,9 +538,6 @@ __device__ __forceinline__ int uniformize(int v, int bits)
 #ifndef NV_CLS_UNROLL
 #define NV_CLS_UNROLL 2            // weak classifiers in flight per lane in the bulk kernel's inner loops
 #endif
-#ifndef NV_CLS_PACK_GAIN
-#define NV_CLS_PACK_GAIN 2         // a stage of a tile takes the packed schedule when it saves at least this many warp steps
-#endif
 constexpr int CLS_UNROLL = NV_CLS_UNROLL;
 
 __device__ __forceinline__ uint32_t lds_u32(uint32_t addr)
@@ -639,9 +638,6 @@ __global__ void __launch_bounds__(256) k_cascade_classes(const __grid_constant__
     __shared__ __align__(8) unsigned long long mbar;
     __shared__ uint32_t s_mask[3][2][32];                        // rotating alive masks: [buffer][member / 32][class]
     __shared__ uint32_t s_words[NV_CTY][2];
-#ifdef NV_CLS_PACK
-    __shared__ unsigned short s_list[NV_CTX * NV_CTY];           // packed schedule of a stage: (class << 6) | member, rank-major
-#endif
     const PlanDev *__restrict__ plan = P.plan;
     const int tid = threadIdx.x, lane = tid & 31;
     const int warp = uniformize(tid >> 5, 3);
@@ -694,80 +690,6 @@ __global__ void __launch_bounds__(256) k_cascade_classes(const __grid_constant__
         if (warp == 0) { s_mask[zer][0][lane] = 0u; s_mask[zer][1][lane] = 0u; }
         unsigned long long rem = ((unsigned long long)mhi << 32) | mlo, pass_bits = 0ull;
         for (int i = 0; i < warp; i++) rem &= rem - 1ull;        // warp w takes the set bits of rank w, w + 8, ...
-#ifdef NV_CLS_PACK
-        // ---- packed schedule (experiment of round 2, OFF by default: measured slower twice, profiles/r2_summary.md) ----------
-        // The rank schedule below costs maxc warp steps per weak classifier (one member of every class per step) whatever
-        // the number of windows alive.  When the classes are unbalanced — the sparse later stages: 40 windows, the fullest
-        // class holds 5 — the members are laid out RANK-MAJOR in a list (all first members, then all second members, ...)
-        // and the warps take 32 consecutive entries per step.  Entries of one rank belong to different classes, so a step
-        // only conflicts where it holds several ranks.
-        //   variant 1, steps of 32 consecutive entries (ceil(N / 32) steps): 9-12 % fewer warp instructions, but steps
-        //     straddle ranks, the shared-memory pipe (already at 67-74 %) took 20 % more wavefronts, 40 % of them replays:
-        //     bulk stages 0.392 ms against 0.346 ms, 2411 against 2540 frames/s;
-        //   variant 2 (below), whole ranks packed into a step while they fit, so that the wavefront count stays what the
-        //     rank schedule pays: 0.43 ms, 2270 against 2628 frames/s — the dry run, the list, the second barrier per stage
-        //     and one shared-memory atomic per surviving window cost more than the idle lanes they remove.
-        {
-            const int cnt = __popc(mlo) + __popc(mhi);
-            // dry run: how many steps if whole ranks are packed into a step while they fit (a step never straddles a rank,
-            // so a class appears at most once per rank in it and the wavefront count stays what the rank schedule pays)
-            int nsteps, fill = 0, steps = 0;
-            for (int r = 0; r < maxc; r++) {
-                const int h = __popc(__ballot_sync(0xffffffffu, cnt > r));
-                if (fill + h > 32) { steps++; fill = 0; }
-                fill += h;
-            }
-            nsteps = steps + (fill > 0);
-            if (maxc - nsteps >= NV_CLS_PACK_GAIN) {
-                int base = 0;
-                for (int r = 0; r < maxc; r++) {                 // every warp counts, warp (r mod 8) writes rank r
-                    const uint32_t b = __ballot_sync(0xffffffffu, cnt > r);
-                    const int h = __popc(b), room = 32 - (base & 31);
-                    const bool mine = (r & 7) == warp;
-                    if ((base & 31) && h > room) {               // close the step: the rest of it stays empty
-                        if (mine && lane < room) s_list[base + lane] = 0xffff;
-                        base += room;
-                    }
-                    if (mine) {
-                        if (cnt > r) s_list[base + __popc(b & ((1u << lane) - 1u))] = (unsigned short)((lane << 6) | (__ffsll((long long)rem) - 1));
-#pragma unroll
-                        for (int q = 0; q < 8; q++) rem &= rem - 1ull;
-                    }
-                    base += h;
-                }
-                const int nalive = base;                          // list length, holes included
-                __syncthreads();
-                for (int t = warp; t < nsteps; t += 16) {        // two list entries per lane and round: steps t and t + 8
-                    int cls[2], bit[2], ly[2], lx[2]; bool active[2], pass[2]; uint32_t wa[2]; float vnf[2];
-#pragma unroll
-                    for (int i = 0; i < 2; i++) {
-                        const int p = (t + 8 * i) * 32 + lane;
-                        int e = p < nalive ? (int)s_list[p] : 0xffff;
-                        active[i] = e != 0xffff;
-                        if (!active[i]) e = lane << 6;
-                        cls[i] = e >> 6; bit[i] = e & 63;
-                        ly[i] = bit[i] >> 1; lx[i] = ((cls[i] - K * ly[i]) & 31) + ((bit[i] & 1) << 5);
-                        wa[i] = tile_sa + (uint32_t)(ly[i] * rowb + lx[i] * 4);
-                        vnf[i] = active[i] ? __ldg(vnf_tile + ly[i] * L.nx + lx[i]) : 0.f;
-                    }
-                    if (t + 8 < nsteps) class_stage<FAST, 2>(P, si, wa, vnf, pass);
-                    else {
-                        const uint32_t wa1[1] = {wa[0]}; const float vnf1[1] = {vnf[0]}; bool pass1[1];
-                        class_stage<FAST, 1>(P, si, wa1, vnf1, pass1);
-                        pass[0] = pass1[0]; pass[1] = false;
-                    }
-#pragma unroll
-                    for (int i = 0; i < 2; i++) {
-                        if (active[i] && pass[i]) atomicOr(&s_mask[nxt][bit[i] >> 5][cls[i]], 1u << (bit[i] & 31));
-                        if (P.depth && active[i] && !pass[i]) P.depth[L.wofs + (iy0 + ly[i]) * L.nx + ix0 + lx[i]] = (int16_t)(-st);
-                    }
-                }
-                __syncthreads();
-                cur = nxt;
-                continue;
-            }
-        }
-#endif
         int j = warp;
         for (; j + 8 < maxc; j += 16) {                          // two windows per lane and round
             int bit[2]; bool active[2], pass[2]; uint32_t wa[2]; float vnf[2]; int ly[2], lx[2];
@@ -1788,23 +1710,26 @@ cudaError_t launch_alive_to_queue(const PlanDev *plan, int total_rows, const flo
     return cudaGetLastError();
 }
 
+// The dynamic shared-memory limit is an attribute of a device's copy of a kernel: raised once per (kernel, device).
+static cudaError_t raise_smem_limit(const void *kernel, int bytes)
+{
+    static std::mutex mu;
+    static std::set<std::pair<const void *, int>> done;
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    std::lock_guard<std::mutex> lk(mu);
+    if (done.count({kernel, dev})) return cudaSuccess;
+    if ((e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes)) == cudaSuccess) done.insert({kernel, dev});
+    return e;
+}
+
 cudaError_t launch_stage0_tiles(const Stage0TileParams &sp, int ystep, int ntiles, cudaStream_t st)
 {
-    const size_t smem = (size_t)ystep * sp.ps * sizeof(uint32_t);
-    static std::mutex mu;
-    static unsigned long long attr_set = 0ull;                   // per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        if (!((attr_set >> (dev & 63)) & 1ull)) {
-            cudaFuncSetAttribute(k_stage0_tiles<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-            cudaFuncSetAttribute(k_stage0_tiles<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-            attr_set |= 1ull << (dev & 63);
-        }
-    }
-    if (ystep == 2) k_stage0_tiles<2><<<ntiles, 256, smem, st>>>(sp);
-    else k_stage0_tiles<1><<<ntiles, 256, smem, st>>>(sp);
+    const auto kernel = ystep == 2 ? k_stage0_tiles<2> : k_stage0_tiles<1>;
+    cudaError_t e = raise_smem_limit((const void *)kernel, 160 * 1024);
+    if (e != cudaSuccess) return e;
+    kernel<<<ntiles, 256, (size_t)ystep * sp.ps * sizeof(uint32_t), st>>>(sp);
     return cudaGetLastError();
 }
 
@@ -1822,86 +1747,24 @@ cudaError_t launch_stage0_chain(const PlanDev &plan, const uint32_t *bits_fail, 
     return cudaGetLastError();
 }
 
-cudaError_t launch_cascade_classes(const TileParams &tp, int ystep, int ntiles, cudaStream_t st)
+// the bulk stages of the ystep-2 levels: NV_CTX x NV_CTY-window tiles, two column planes each
+cudaError_t launch_cascade_classes(const TileParams &tp, int ntiles, cudaStream_t st)
 {
-    size_t smem = (size_t)ystep * tp.ps * sizeof(uint32_t);
-    if (const char *pad = getenv(ystep == 2 ? "NUBOVCA_YS2_SMEM" : "NUBOVCA_YS1_SMEM"))    // experiments: cap resident blocks
-        smem = std::max(smem, (size_t)atoi(pad));
-    static std::mutex mu;
-    static unsigned long long attr_set = 0ull;                   // per device: the attribute belongs to the device's function
-    int dev = 0;
-    cudaGetDevice(&dev);
-    std::lock_guard<std::mutex> lk(mu);
-    if (!((attr_set >> (dev & 63)) & 1ull)) {
-        cudaFuncSetAttribute(k_cascade_classes<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        cudaFuncSetAttribute(k_cascade_classes<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        cudaFuncSetAttribute(k_cascade_classes<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        cudaFuncSetAttribute(k_cascade_classes<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        attr_set |= 1ull << (dev & 63);
-    }
-    if (ystep == 2) {
-        if (tp.fast) k_cascade_classes<2, true><<<ntiles, 256, smem, st>>>(tp);
-        else k_cascade_classes<2, false><<<ntiles, 256, smem, st>>>(tp);
-    } else {
-        if (tp.fast) k_cascade_classes<1, true><<<ntiles, 256, smem, st>>>(tp);
-        else k_cascade_classes<1, false><<<ntiles, 256, smem, st>>>(tp);
-    }
+    const auto kernel = tp.fast ? k_cascade_classes<2, true> : k_cascade_classes<2, false>;
+    cudaError_t e = raise_smem_limit((const void *)kernel, 160 * 1024);
+    if (e != cudaSuccess) return e;
+    kernel<<<ntiles, 256, 2 * (size_t)tp.ps * sizeof(uint32_t), st>>>(tp);
     return cudaGetLastError();
 }
 
-// NUBOVCA_WIDE=WxH / NUBOVCA_WIDE2=WxH pick the tile shape of the ystep-1 / ystep-2 levels in k_cascade_wide (64x32, 64x64 or
-// 128x64; ystep 2: 64x32 or 64x64); "0" sends the class to k_cascade_classes (64x32 tiles, interleaved ranks)
-bool nv_wide_tile_config(int cls, int *tw, int *th)
+// the bulk stages of the ystep-1 levels: NV_WTX x NV_WTY-window tiles, eight warps
+cudaError_t launch_cascade_wide(const TileParams &tp, int ntiles, cudaStream_t st)
 {
-    static const int cfg[2] = {[] {
-        const char *e = getenv("NUBOVCA_WIDE2");
-        if (!e) return NV_WIDE2_DEFAULT;
-        int w = 0, h = 0;
-        if (sscanf(e, "%dx%d", &w, &h) == 2 && w == 64 && (h == 64 || h == 32)) return (w << 16) | h;
-        return 0;
-    }(), [] {
-        const char *e = getenv("NUBOVCA_WIDE");
-        if (!e) return NV_WIDE_DEFAULT;
-        int w = 0, h = 0;
-        if (sscanf(e, "%dx%d", &w, &h) == 2 && ((w == 64 && h == 64) || (w == 128 && h == 64) || (w == 64 && h == 32))) return (w << 16) | h;
-        return 0;
-    }()};
-    *tw = cfg[cls] >> 16; *th = cfg[cls] & 0xffff;
-    return cfg[cls] != 0;
-}
-
-template <int YS, int TW, int TH, int NWARP>
-static cudaError_t launch_wide_t(const TileParams &tp, int ntiles, size_t smem, cudaStream_t st)
-{
-    static std::mutex mu;
-    static unsigned long long attr_set = 0ull;                   // per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        if (!((attr_set >> (dev & 63)) & 1ull)) {
-            cudaFuncSetAttribute(k_cascade_wide<YS, true, TW, TH, NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-            cudaFuncSetAttribute(k_cascade_wide<YS, false, TW, TH, NWARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-            attr_set |= 1ull << (dev & 63);
-        }
-    }
-    if (tp.fast) k_cascade_wide<YS, true, TW, TH, NWARP><<<ntiles, 32 * NWARP, smem, st>>>(tp);
-    else k_cascade_wide<YS, false, TW, TH, NWARP><<<ntiles, 32 * NWARP, smem, st>>>(tp);
+    const auto kernel = tp.fast ? k_cascade_wide<1, true, NV_WTX, NV_WTY, 8> : k_cascade_wide<1, false, NV_WTX, NV_WTY, 8>;
+    cudaError_t e = raise_smem_limit((const void *)kernel, 160 * 1024);
+    if (e != cudaSuccess) return e;
+    kernel<<<ntiles, 32 * 8, (size_t)tp.ps * sizeof(uint32_t), st>>>(tp);
     return cudaGetLastError();
-}
-
-cudaError_t launch_cascade_wide(const TileParams &tp, int ystep, int tw, int th, int ntiles, cudaStream_t st)
-{
-    const size_t smem = (size_t)ystep * tp.ps * sizeof(uint32_t);
-    static const int nwarp[2] = {[] { const char *e = getenv("NUBOVCA_WIDE2_WARPS"); return e && atoi(e) == 8 ? 8 : 16; }(),
-                                 [] { const char *e = getenv("NUBOVCA_WIDE_WARPS"); return e && atoi(e) == 16 ? 16 : 8; }()};
-    const int nw = nwarp[ystep == 2 ? 0 : 1];
-    if (ystep == 1 && tw == 64 && th == 64) return nw == 16 ? launch_wide_t<1, 64, 64, 16>(tp, ntiles, smem, st) : launch_wide_t<1, 64, 64, 8>(tp, ntiles, smem, st);
-    if (ystep == 1 && tw == 128 && th == 64) return nw == 16 ? launch_wide_t<1, 128, 64, 16>(tp, ntiles, smem, st) : launch_wide_t<1, 128, 64, 8>(tp, ntiles, smem, st);
-    if (ystep == 1 && tw == 64 && th == 32) return launch_wide_t<1, 64, 32, 8>(tp, ntiles, smem, st);
-    if (ystep == 2 && tw == 64 && th == 64) return nw == 16 ? launch_wide_t<2, 64, 64, 16>(tp, ntiles, smem, st) : launch_wide_t<2, 64, 64, 8>(tp, ntiles, smem, st);
-    if (ystep == 2 && tw == 64 && th == 32) return launch_wide_t<2, 64, 32, 8>(tp, ntiles, smem, st);
-    return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_cascade_tail(const PlanDev *plan, const DevCascade *meta, const DevStump *stumps, const uint32_t *sum,
@@ -1956,18 +1819,8 @@ static cudaError_t launch_tail_tab_t(const PlanDev *plan, const DevCascade *meta
 {
     const size_t smem = tail_tab_smem(hmeta, stage_begin, stage_end);
     if (smem > NV_TAILTAB_MAX_SMEM) return cudaErrorInvalidConfiguration;
-    static std::mutex mu;
-    static unsigned long long attr_set = 0ull;                   // per device: the attribute belongs to the device's function
-    int dev = 0;
-    cudaGetDevice(&dev);
-    {
-        std::lock_guard<std::mutex> lk(mu);
-        if (!((attr_set >> (dev & 63)) & 1ull)) {
-            cudaError_t e = cudaFuncSetAttribute(k_cascade_tail_tab<NV_TAILTAB_WARPS, BATCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NV_TAILTAB_MAX_SMEM);
-            if (e != cudaSuccess) return e;
-            attr_set |= 1ull << (dev & 63);
-        }
-    }
+    cudaError_t e = raise_smem_limit((const void *)k_cascade_tail_tab<NV_TAILTAB_WARPS, BATCH>, (int)NV_TAILTAB_MAX_SMEM);
+    if (e != cudaSuccess) return e;
     int per_sm = (int)((227 * 1024) / (smem + 2048));            // static tables + the per-block reserve
     per_sm = per_sm < 1 ? 1 : per_sm > 8 ? 8 : per_sm;
     // (fewer blocks when the queue is short — every block copies the table — was measured: no gain down to one block per 32

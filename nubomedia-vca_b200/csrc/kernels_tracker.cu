@@ -72,7 +72,7 @@ struct TrkParams {
     int4 *rects;                    // [TRK_MAX_COMPONENTS]
     int4 *out;                      // [1 + TRK_MAX_COMPONENTS]: (count, 0, 0, 0), rects in raster order of the first seed
     int4 *hout;                     // the context's page-locked copy of out[0 .. 1024] (mapped host memory): written by the last block,
-                                    // so that no device-to-host copy follows the launch; nullptr: the host copies
+                                    // so that no device-to-host copy follows the launch
     float val[256];                 // timestamp of history index k after this frame's expiry (0: none / expired)
 };
 
@@ -500,8 +500,7 @@ cudaError_t launch_tracker(nv_ctx *ctx, int fmt, const SrcPlanes &src, int w, in
     P.parent = reinterpret_cast<int *>(base + lo.parent); P.edge_flag = reinterpret_cast<int *>(base + lo.edge_flag);
     P.counters = reinterpret_cast<int *>(base + lo.counters); P.keys = reinterpret_cast<int *>(base + lo.keys);
     P.rects = reinterpret_cast<int4 *>(base + lo.rects); P.out = reinterpret_cast<int4 *>(base + lo.out);
-    static const bool host_writes = [] { const char *e = getenv("NUBOVCA_HOST_WRITES"); return !e || atoi(e) != 0; }();
-    P.hout = host_writes ? reinterpret_cast<int4 *>(ctx->h_trk) : nullptr;
+    P.hout = reinterpret_cast<int4 *>(ctx->h_trk);
     for (int i = 0; i < 256; i++) P.val[i] = val256[i];
     const int nt = lo.ntx * lo.nty;
     cudaStream_t st = ctx->stream;
