@@ -320,7 +320,7 @@ extern "C" void nv_ctx_destroy(nv_ctx *c)
         for (int i = 0; i < NV_PLAN_SLOTS; i++) {
             PlanSlot &sl = c->slots[i];
             cudaFree(sl.d_plan); cudaFree(sl.d_ptab); cudaFree(sl.d_maps);
-            if (sl.dexec) cudaGraphExecDestroy(sl.dexec);
+            sl.graph.drop();
         }
         delete[] c->slots;
     }
@@ -330,8 +330,8 @@ extern "C" void nv_ctx_destroy(nv_ctx *c)
     cudaFree(c->d_cand_w); cudaFree(c->d_cls_wmax);
     cudaFreeHost(c->h_result);
     cudaFree(c->d_trk_prev); cudaFree(c->d_trk_hist); cudaFree(c->d_trk_scratch); cudaFreeHost(c->h_trk);
-    if (c->gexec) cudaGraphExecDestroy(c->gexec);
-    if (c->bexec) cudaGraphExecDestroy(c->bexec);
+    c->face_graph.drop();
+    c->batch_graph.drop();
     batch_free(c->b);
     if (c->ev_done) cudaEventDestroy(c->ev_done);
     for (int i = 0; i < 2; i++) { if (c->ev_fork[i]) cudaEventDestroy(c->ev_fork[i]); if (c->ev_join[i]) cudaEventDestroy(c->ev_join[i]); }
@@ -598,8 +598,7 @@ static int ensure_plan(nv_ctx *ctx, const nv_cascade *casc, int W, int H, const 
     ctx->ps->tp_casc = 0;                  // tensor maps and tile geometry follow the plan
     ctx->ps->buf_gen = ctx->buf_gen;
     ctx->ps->gen++;
-    if (ctx->ps->dexec) { cudaGraphExecDestroy(ctx->ps->dexec); ctx->ps->dexec = nullptr; }
-    ctx->ps->dkey = DetGraphKey(); ctx->ps->dkey_seen = DetGraphKey();
+    ctx->ps->graph.reset();
     return NV_OK;
 }
 
@@ -628,7 +627,7 @@ static int ensure_tile_params(nv_ctx *ctx, const nv_cascade *casc)
     ctx->ps->tp_casc = casc->uid;
     ctx->ps->use_tiles = false;  ctx->ps->use_s0t = false;
     ctx->ps->gen++;                                              // graphs hold the parameter banks by value
-    if (ctx->ps->dexec) { cudaGraphExecDestroy(ctx->ps->dexec); ctx->ps->dexec = nullptr; }
+    ctx->ps->graph.drop();
     ctx->ps->use_s0p = !casc->h.general && P.nlevels > 0 && fill_stage0_params(casc, P, &ctx->ps->s0p);
     encode_tiled_fn enc = get_encode_tiled();
     if (casc->h.general || !enc || m.win_w > 32 || m.win_h > 32 || P.nlevels == 0) return NV_OK;
@@ -908,6 +907,50 @@ static void detect_bookkeeping(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_g
     ctx->batch_last = false;
 }
 
+enum GraphRun { RUN_PLAIN, RUN_CAPTURED, RUN_REPLAYED };
+
+// One call path's launches (enqueue(&nl) issues them on ctx->stream and counts them): the first call with a key runs them
+// plainly and remembers the key, the second captures them into a graph and launches it, every later one replays the graph.
+// Should capture fail, the context stays on plain launches for good (no_graph).  *how reports which of the three ran; the
+// capture records the stage events it marked (GraphCache::prof_mask) for callers whose replays must restore prof_set.
+template <class Key, class Enqueue>
+static int graph_run(nv_ctx *ctx, GraphCache<Key> &gc, const Key &key, bool graphable, Enqueue &&enqueue, int *nl, GraphRun *how)
+{
+    *nl = 0;
+    *how = RUN_PLAIN;
+    if (graphable && gc.exec && key == gc.key) {
+        NV_CUDA(cudaGraphLaunch(gc.exec, ctx->stream));
+        *nl = gc.nl;
+        *how = RUN_REPLAYED;
+        return NV_OK;
+    }
+    if (!graphable || !(key == gc.seen)) {
+        gc.seen = key;
+        return enqueue(nl);
+    }
+    gc.drop();
+    cudaGraph_t g = nullptr;
+    NV_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
+    int rc = enqueue(nl);
+    cudaError_t ce = cudaStreamEndCapture(ctx->stream, &g);
+    if (rc != NV_OK || ce != cudaSuccess || !g) {
+        if (g) cudaGraphDestroy(g);
+        cudaGetLastError();
+        ctx->no_graph = true;                      // capture is not possible here: stay on plain launches
+        *nl = 0;
+        return enqueue(nl);
+    }
+    ce = cudaGraphInstantiate(&gc.exec, g, 0);
+    cudaGraphDestroy(g);
+    if (ce != cudaSuccess) { gc.exec = nullptr; nv_set_error("cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return NV_ERR_CUDA; }
+    gc.key = key; gc.nl = *nl;
+    gc.prof_mask = 0;
+    for (int i = 0; i <= NV_NUM_STAGES; i++) if (ctx->prof_set[i]) gc.prof_mask |= 1u << i;
+    NV_CUDA(cudaGraphLaunch(gc.exec, ctx->stream));
+    *how = RUN_CAPTURED;
+    return NV_OK;
+}
+
 int nv_detect_device(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, int W, int H, int gstride,
                      const uint8_t *d_lut, const nv_detect_params *p)
 {
@@ -916,38 +959,14 @@ int nv_detect_device(nv_ctx *ctx, nv_cascade *casc, const uint8_t *d_gray, int W
     // A plan that sees the same (image, cascade, parameters) again replays its launches as one CUDA graph: the nested
     // ROI stages of the eye / mouth / nose / ear elements call this several times per frame on tiny images, where the
     // launches cost more than the kernels.  Debug / profiling runs keep individual launches (taps and events).
-    PlanSlot *sl = ctx->ps;
     DetGraphKey key;
     key.gray = d_gray; key.gstride = gstride; key.lut = d_lut; key.casc = casc->uid; key.sf = p->scale_factor; key.mn = p->min_neighbors;
     key.epoch = ctx->epoch; key.scores = ctx->scores;
-    bool graphable = !ctx->debug && !ctx->profile && !ctx->no_graph;
-    int nl = 0;
-    if (graphable && sl->dexec && key == sl->dkey) {
-        NV_CUDA(cudaGraphLaunch(sl->dexec, ctx->stream));
-        nl = sl->d_nl;
-    } else if (graphable && key == sl->dkey_seen) {
-        if (sl->dexec) { cudaGraphExecDestroy(sl->dexec); sl->dexec = nullptr; }
-        cudaGraph_t g = nullptr;
-        NV_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-        rc = detect_enqueue(ctx, casc, d_gray, W, H, gstride, d_lut, p, &nl);
-        cudaError_t ce = cudaStreamEndCapture(ctx->stream, &g);
-        if (rc != NV_OK || ce != cudaSuccess || !g) {
-            if (g) cudaGraphDestroy(g);
-            cudaGetLastError();
-            ctx->no_graph = true;                      // capture is not possible here: stay on plain launches
-            nl = 0;
-            if ((rc = detect_enqueue(ctx, casc, d_gray, W, H, gstride, d_lut, p, &nl)) != NV_OK) return rc;
-        } else {
-            ce = cudaGraphInstantiate(&sl->dexec, g, 0);
-            cudaGraphDestroy(g);
-            if (ce != cudaSuccess) { sl->dexec = nullptr; nv_set_error("cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return NV_ERR_CUDA; }
-            sl->dkey = key; sl->d_nl = nl;
-            NV_CUDA(cudaGraphLaunch(sl->dexec, ctx->stream));
-        }
-    } else {
-        sl->dkey_seen = key;
-        if ((rc = detect_enqueue(ctx, casc, d_gray, W, H, gstride, d_lut, p, &nl)) != NV_OK) return rc;
-    }
+    int nl;
+    GraphRun how;
+    rc = graph_run(ctx, ctx->ps->graph, key, !ctx->debug && !ctx->profile && !ctx->no_graph,
+                   [&](int *n) { return detect_enqueue(ctx, casc, d_gray, W, H, gstride, d_lut, p, n); }, &nl, &how);
+    if (rc != NV_OK) return rc;
     ctx->launches += nl;
     detect_bookkeeping(ctx, casc, d_gray, W, H, gstride, d_lut, p);
     return NV_OK;
@@ -1003,21 +1022,42 @@ int nv_collect(nv_ctx *ctx, nv_rect *out, int cap, int *n)
     return NV_OK;
 }
 
-// host -> device copy of an input image on the ctx's stream: page-locked caller memory is read directly by the
-// DMA engine, pageable memory goes through the ctx's pinned staging buffer
-int nv_h2d(nv_ctx *ctx, const uint8_t *src, size_t bytes)
+cudaMemoryType nv_memory_type(const void *p)
 {
     cudaPointerAttributes at;
-    bool known = cudaPointerGetAttributes(&at, src) == cudaSuccess;
-    if (known && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged)) {
-        // a frame that already lives in device memory (nv_element_transform_frame_device): one copy inside HBM
-        NV_CUDA(cudaMemcpyAsync(ctx->d_frame, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) at.type = cudaMemoryTypeUnregistered;
+    if (at.type == cudaMemoryTypeUnregistered) cudaGetLastError();
+    return at.type;
+}
+
+// A frame of `height` rows of `stride` bytes at src (of memory `type`) -> dst, on the ctx's stream: the whole frame
+// (period == 0), or only the row pairs a + k * period, a + k * period + 1 (k < n) that an integer down-scale reads, at their
+// own offsets as one strided copy — half the bytes of a 640x480 frame processed at 160x120.  Device memory (a frame
+// decoded on the GPU) is copied whole inside HBM, page-locked memory is read in place by the DMA engine, pageable memory
+// goes through the pinned staging buffer `stage`.
+static int upload_rows(nv_ctx *ctx, uint8_t *dst, uint8_t *stage, const uint8_t *src, cudaMemoryType type, size_t stride, int height,
+                       int a, int period, int n)
+{
+    if (type == cudaMemoryTypeDevice || type == cudaMemoryTypeManaged) {
+        NV_CUDA(cudaMemcpyAsync(dst, src, stride * height, cudaMemcpyDeviceToDevice, ctx->stream));
         return NV_OK;
     }
-    bool pinned = known && at.type == cudaMemoryTypeHost;
-    if (!pinned) { cudaGetLastError(); memcpy(ctx->h_frame, src, bytes); }
-    NV_CUDA(cudaMemcpyAsync(ctx->d_frame, pinned ? src : ctx->h_frame, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    const bool pinned = type == cudaMemoryTypeHost;
+    if (period <= 0) {
+        if (!pinned) memcpy(stage, src, stride * height);
+        NV_CUDA(cudaMemcpyAsync(dst, pinned ? src : stage, stride * height, cudaMemcpyHostToDevice, ctx->stream));
+        return NV_OK;
+    }
+    const size_t off = (size_t)a * stride, pitch = (size_t)period * stride, run = 2 * stride;
+    if (!pinned)
+        for (int k = 0; k < n; k++) memcpy(stage + off + k * pitch, src + off + k * pitch, run);
+    NV_CUDA(cudaMemcpy2DAsync(dst + off, pitch, (pinned ? src : stage) + off, pitch, run, n, cudaMemcpyHostToDevice, ctx->stream));
     return NV_OK;
+}
+
+int nv_h2d(nv_ctx *ctx, const uint8_t *src, size_t bytes)
+{
+    return upload_rows(ctx, ctx->d_frame, ctx->h_frame, src, nv_memory_type(src), bytes, 1, 0, 0, 0);
 }
 
 static int check_frame(nv_ctx *ctx, const void *img, int w, int h, int stride, int cn)
@@ -1080,24 +1120,6 @@ int nv_get_rtab(nv_ctx *ctx, int sw, int sh, int dw, int dh, const int **d_tab, 
     return NV_OK;
 }
 
-// Host frame -> ctx->d_frame, only the row pairs an integer down-scale reads (RtabEntry::row_period): `n` pairs of rows
-// a + k * period, a + k * period + 1, at their own offsets, as one strided copy — half the bytes of a 640x480 frame that
-// is processed at 160x120.  Page-locked caller memory is read in place, anything else goes through the staging buffer.
-static int nv_h2d_row_pairs(nv_ctx *ctx, const uint8_t *src, int stride, int height, int a, int period, int n)
-{
-    cudaPointerAttributes at;
-    bool known = cudaPointerGetAttributes(&at, src) == cudaSuccess;
-    if (known && (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged)) return nv_h2d(ctx, src, (size_t)stride * height);
-    const bool pinned = known && at.type == cudaMemoryTypeHost;
-    const size_t off = (size_t)a * stride, pitch = (size_t)period * stride, run = 2 * (size_t)stride;
-    if (!pinned) {
-        cudaGetLastError();
-        for (int k = 0; k < n; k++) memcpy(ctx->h_frame + off + k * pitch, src + off + k * pitch, run);
-    }
-    NV_CUDA(cudaMemcpy2DAsync(ctx->d_frame + off, pitch, (pinned ? src : ctx->h_frame) + off, pitch, run, n, cudaMemcpyHostToDevice, ctx->stream));
-    return NV_OK;
-}
-
 // Source frame of the face block: interleaved BGR (p[0], s[0]) or the planes of a 4:2:0 frame.
 struct FaceSrc { int fmt; const uint8_t *p[3]; int s[3]; bool on_device; };
 
@@ -1128,11 +1150,8 @@ static int yuv_h2d(nv_ctx *ctx, const FaceSrc &f, int height, SrcPlanes *d)
         for (int i = 0; i < np; i++) { off[i] = o; o += (bytes[i] + 255) & ~(size_t)255; }
         if (o > ctx->frame_cap) { nv_set_error("4:2:0 frame larger than the context"); return NV_ERR_CAPACITY; }
         for (int i = 0; i < np; i++) {
-            cudaPointerAttributes at;
-            bool pinned = cudaPointerGetAttributes(&at, f.p[i]) == cudaSuccess && at.type == cudaMemoryTypeHost;
-            if (!pinned) { cudaGetLastError(); memcpy(ctx->h_frame + off[i], f.p[i], bytes[i]); }
-            NV_CUDA(cudaMemcpyAsync(ctx->d_frame + off[i], pinned ? f.p[i] : ctx->h_frame + off[i], bytes[i],
-                                    cudaMemcpyHostToDevice, ctx->stream));
+            int rc = upload_rows(ctx, ctx->d_frame + off[i], ctx->h_frame + off[i], f.p[i], nv_memory_type(f.p[i]), bytes[i], 1, 0, 0, 0);
+            if (rc != NV_OK) return rc;
         }
     }
     d->p0 = ctx->d_frame; d->p1 = ctx->d_frame + off[1]; d->p2 = np == 3 ? ctx->d_frame + off[2] : nullptr;
@@ -1215,10 +1234,9 @@ static int face_submit_impl(nv_ctx *ctx, const nv_cascade *c, const FaceSrc &src
     const uint8_t *d_src = bgr;
     SrcPlanes planes = {src.p[0], src.p[1], src.p[2], src.s[0], src.s[1], src.s[2]};
     if (!on_device) {
-        // page-locked caller memory is copied straight from the caller; anything else goes through the pinned staging buffer
-        if (yuv) { if ((rc = yuv_h2d(ctx, src, height, &planes)) != NV_OK) return rc; }
-        else if (row_period > 0) { if ((rc = nv_h2d_row_pairs(ctx, bgr, stride, height, row_a, row_period, rows)) != NV_OK) return rc; }
-        else if ((rc = nv_h2d(ctx, bgr, (size_t)stride * height)) != NV_OK) return rc;
+        if (yuv) rc = yuv_h2d(ctx, src, height, &planes);
+        else rc = upload_rows(ctx, ctx->d_frame, ctx->h_frame, bgr, nv_memory_type(bgr), stride, height, row_a, row_period, rows);
+        if (rc != NV_OK) return rc;
         d_src = ctx->d_frame;
     }
     auto enqueue = [&](int *nl) -> int {
@@ -1233,42 +1251,17 @@ static int face_submit_impl(nv_ctx *ctx, const nv_cascade *c, const FaceSrc &src
         return detect_enqueue(ctx, casc, ctx->d_gray, cols, rows, cols, ctx->d_lut, &dp, nl);
     };
     // A context that sees the same call shape again replays it as ONE CUDA graph launch (the per-stream steady
-    // state of an element); debug / profiling runs keep individual launches so that their events and taps work.
+    // state of an element); debug runs keep individual launches so that their taps work.  With profiling on, the stage
+    // events are event-record nodes of the graph.
     nv_ctx::GraphKey key = {d_src, width, height, stride, cols, rows, d_rtab, casc->uid, dp.scale_factor, dp.min_neighbors,
                             dp.min_w, dp.min_h, ctx->epoch, ctx->ps, ctx->ps->gen,
                             src.fmt, yuv ? planes.p1 : nullptr, yuv ? planes.p2 : nullptr, yuv ? planes.s1 : 0, yuv ? planes.s2 : 0,
                             ctx->scores};
-    bool graphable = !ctx->debug && !ctx->no_graph;
-    int nl = 0;
-    if (graphable && ctx->gexec && key == ctx->gkey) {
-        NV_CUDA(cudaGraphLaunch(ctx->gexec, ctx->stream));
-        nl = ctx->g_nl;
-        for (int i = 0; i <= NV_NUM_STAGES; i++) ctx->prof_set[i] = ctx->profile && ((ctx->g_prof_mask >> i) & 1u);
-    } else if (graphable && key == ctx->gkey_seen) {
-        if (ctx->gexec) { cudaGraphExecDestroy(ctx->gexec); ctx->gexec = nullptr; }
-        cudaGraph_t g = nullptr;
-        NV_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-        rc = enqueue(&nl);
-        cudaError_t ce = cudaStreamEndCapture(ctx->stream, &g);
-        if (rc != NV_OK || ce != cudaSuccess || !g) {
-            if (g) cudaGraphDestroy(g);
-            cudaGetLastError();
-            ctx->no_graph = true;                      // capture is not possible here: stay on plain launches
-            nl = 0;
-            if ((rc = enqueue(&nl)) != NV_OK) return rc;
-        } else {
-            ce = cudaGraphInstantiate(&ctx->gexec, g, 0);
-            cudaGraphDestroy(g);
-            if (ce != cudaSuccess) { ctx->gexec = nullptr; nv_set_error("cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return NV_ERR_CUDA; }
-            ctx->gkey = key; ctx->g_nl = nl;
-            ctx->g_prof_mask = 0;
-            for (int i = 0; i <= NV_NUM_STAGES; i++) if (ctx->prof_set[i]) ctx->g_prof_mask |= 1u << i;
-            NV_CUDA(cudaGraphLaunch(ctx->gexec, ctx->stream));
-        }
-    } else {
-        ctx->gkey_seen = key;
-        if ((rc = enqueue(&nl)) != NV_OK) return rc;
-    }
+    int nl;
+    GraphRun how;
+    if ((rc = graph_run(ctx, ctx->face_graph, key, !ctx->debug && !ctx->no_graph, enqueue, &nl, &how)) != NV_OK) return rc;
+    if (how == RUN_REPLAYED)                        // the graph records the stage events its capture marked
+        for (int i = 0; i <= NV_NUM_STAGES; i++) ctx->prof_set[i] = ctx->profile && ((ctx->face_graph.prof_mask >> i) & 1u);
     ctx->launches += nl;
     detect_bookkeeping(ctx, casc, ctx->d_gray, cols, rows, cols, ctx->d_lut, &dp);
     return NV_OK;
@@ -1426,29 +1419,6 @@ static int batch_buffers(nv_ctx *ctx, int n, size_t frame_bytes, size_t gray_byt
     return NV_OK;
 }
 
-// host frame -> device: whole frame (period == 0) or the row pairs a + k * period, + 1 that an integer down-scale reads.
-// Page-locked memory (type cudaMemoryTypeHost) is read in place, pageable memory goes through `stage`, device memory is
-// copied inside HBM.
-static int batch_upload(nv_ctx *ctx, uint8_t *dst, uint8_t *stage, const uint8_t *src, cudaMemoryType type, int stride, int height, int a,
-                        int period, int n)
-{
-    if (type == cudaMemoryTypeDevice || type == cudaMemoryTypeManaged) {
-        NV_CUDA(cudaMemcpyAsync(dst, src, (size_t)stride * height, cudaMemcpyDeviceToDevice, ctx->stream));
-        return NV_OK;
-    }
-    const bool pinned = type == cudaMemoryTypeHost;
-    if (period <= 0) {
-        if (!pinned) memcpy(stage, src, (size_t)stride * height);
-        NV_CUDA(cudaMemcpyAsync(dst, pinned ? src : stage, (size_t)stride * height, cudaMemcpyHostToDevice, ctx->stream));
-        return NV_OK;
-    }
-    const size_t off = (size_t)a * stride, pitch = (size_t)period * stride, run = 2 * (size_t)stride;
-    if (!pinned)
-        for (int k = 0; k < n; k++) memcpy(stage + off + k * pitch, src + off + k * pitch, run);
-    NV_CUDA(cudaMemcpy2DAsync(dst + off, pitch, (pinned ? src : stage) + off, pitch, run, n, cudaMemcpyHostToDevice, ctx->stream));
-    return NV_OK;
-}
-
 enum { BATCH_GRAY = 1, BATCH_FACE = 2 };
 
 // the stream-ordered chain of the batched route: six launches whatever n is (five for gray images)
@@ -1566,10 +1536,8 @@ static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *
     bool pageable = false;
     std::vector<cudaMemoryType> types(on_device ? 0 : n);
     for (size_t i = 0; i < types.size(); i++) {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, frames[i]) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
-        types[i] = at.type;
-        pageable = pageable || at.type == cudaMemoryTypeUnregistered;
+        types[i] = nv_memory_type(frames[i]);
+        pageable = pageable || types[i] == cudaMemoryTypeUnregistered;
     }
     if ((rc = batch_buffers(ctx, n, on_device ? 0 : fbytes, kind == BATCH_FACE ? (size_t)cols * rows : 0, pageable)) != NV_OK) return rc;
     nv_ctx::Batch &b = ctx->b;
@@ -1578,8 +1546,8 @@ static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *
         const uint8_t *d = frames[i];
         if (!on_device) {
             uint8_t *dst = b.d_frame + i * fbytes;
-            if ((rc = batch_upload(ctx, dst, b.h_stage ? b.h_stage + i * fbytes : nullptr, frames[i], types[i], stride, h,
-                                   kind == BATCH_FACE ? row_a : 0, kind == BATCH_FACE ? row_period : 0, rows)) != NV_OK) return rc;
+            if ((rc = upload_rows(ctx, dst, b.h_stage ? b.h_stage + i * fbytes : nullptr, frames[i], types[i], stride, h, row_a, row_period,
+                                  rows)) != NV_OK) return rc;
             d = dst;
         }
         aligned = aligned && ((uintptr_t)d & 3u) == 0;
@@ -1597,36 +1565,13 @@ static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *
     key.aligned = aligned; key.casc = casc->uid; key.sf = dp.scale_factor; key.mn = dp.min_neighbors; key.min_w = dp.min_w;
     key.min_h = dp.min_h; key.max_w = dp.max_w; key.max_h = dp.max_h; key.epoch = ctx->epoch; key.bgen = b.gen; key.slot = ctx->ps;
     key.slot_gen = ctx->ps->gen;
-    const bool graphable = !ctx->debug && !ctx->no_graph;
-    int nl = 0;
-    ctx->batch_replayed = false;
-    if (graphable && ctx->bexec && key == ctx->bkey) {
-        NV_CUDA(cudaGraphLaunch(ctx->bexec, ctx->stream));
-        nl = ctx->b_nl;
-        ctx->batch_replayed = true;
-    } else if (graphable && key == ctx->bkey_seen) {
-        if (ctx->bexec) { cudaGraphExecDestroy(ctx->bexec); ctx->bexec = nullptr; }
-        cudaGraph_t g = nullptr;
-        NV_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-        rc = batch_enqueue(ctx, casc, kind, n, w, h, stride, cols, rows, d_rtab, aligned, dp.min_neighbors, &nl);
-        cudaError_t ce = cudaStreamEndCapture(ctx->stream, &g);
-        if (rc != NV_OK || ce != cudaSuccess || !g) {
-            if (g) cudaGraphDestroy(g);
-            cudaGetLastError();
-            ctx->no_graph = true;                      // capture is not possible here: stay on plain launches
-            nl = 0;
-            if ((rc = batch_enqueue(ctx, casc, kind, n, w, h, stride, cols, rows, d_rtab, aligned, dp.min_neighbors, &nl)) != NV_OK) return rc;
-        } else {
-            ce = cudaGraphInstantiate(&ctx->bexec, g, 0);
-            cudaGraphDestroy(g);
-            if (ce != cudaSuccess) { ctx->bexec = nullptr; nv_set_error("cudaGraphInstantiate: %s", cudaGetErrorString(ce)); return NV_ERR_CUDA; }
-            ctx->bkey = key; ctx->b_nl = nl;
-            NV_CUDA(cudaGraphLaunch(ctx->bexec, ctx->stream));
-        }
-    } else {
-        ctx->bkey_seen = key;
-        if ((rc = batch_enqueue(ctx, casc, kind, n, w, h, stride, cols, rows, d_rtab, aligned, dp.min_neighbors, &nl)) != NV_OK) return rc;
-    }
+    int nl;
+    GraphRun how;
+    rc = graph_run(ctx, ctx->batch_graph, key, !ctx->debug && !ctx->no_graph,
+                   [&](int *c) { return batch_enqueue(ctx, casc, kind, n, w, h, stride, cols, rows, d_rtab, aligned, dp.min_neighbors, c); },
+                   &nl, &how);
+    ctx->batch_replayed = how == RUN_REPLAYED;
+    if (rc != NV_OK) return rc;
     ctx->launches += nl;
     ctx->batch_launches = nl;
     for (int i = 0; i < n; i++) ctx->batch_src[i] = b.h_tab[i];   // device copies: what an overflow re-run in collect reads
@@ -1718,7 +1663,7 @@ extern "C" int nv_detect_multiscale_batch(nv_ctx *ctx, const nv_cascade *c, cons
 // ------------------------------------------------------------------------------------------------
 // standalone image ops (host in, host out) for the nested elements
 // ------------------------------------------------------------------------------------------------
-static int upload(nv_ctx *ctx, const uint8_t *src, size_t bytes)
+int nv_upload(nv_ctx *ctx, const uint8_t *src, size_t bytes)
 {
     if (bytes > ctx->frame_cap) { nv_set_error("image larger than the context"); return NV_ERR_CAPACITY; }
     NV_CUDA(cudaSetDevice(ctx->gpu));
@@ -1756,7 +1701,7 @@ extern "C" int nv_bgr2gray(nv_ctx *ctx, const uint8_t *src, int width, int heigh
     int rc = check_frame(ctx, src, width, height, stride_bytes, channels);
     if (rc != NV_OK) return rc;
     if (!dst_gray || dst_stride < width) { nv_set_error("bad destination"); return NV_ERR_ARG; }
-    if ((rc = upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
+    if ((rc = nv_upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
     NV_CUDA(launch_bgr2gray(ctx->d_frame, width, height, stride_bytes, channels, ctx->d_gray, width, ctx->stream));
     ctx->launches++;
     return download(ctx, ctx->d_gray, width, height, dst_gray, dst_stride);
@@ -1768,7 +1713,7 @@ extern "C" int nv_equalize_hist(nv_ctx *ctx, const uint8_t *src, int width, int 
     int rc = check_frame(ctx, src, width, height, stride_bytes, 1);
     if (rc != NV_OK) return rc;
     if (!dst || dst_stride < width) { nv_set_error("bad destination"); return NV_ERR_ARG; }
-    if ((rc = upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
+    if ((rc = nv_upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
     NV_CUDA(launch_hist(ctx->d_frame, width, height, stride_bytes, ctx->d_hist, ctx->stream, ctx->d_lut));
     NV_CUDA(launch_apply_lut(ctx->d_frame, width, height, stride_bytes, ctx->d_lut, ctx->d_gray, width, ctx->stream));
     ctx->launches += 2;
@@ -1782,7 +1727,7 @@ extern "C" int nv_resize_linear(nv_ctx *ctx, const uint8_t *src, int width, int 
     int rc = check_frame(ctx, src, width, height, stride_bytes, channels);
     if (rc != NV_OK) return rc;
     if (!dst || dst_width <= 0 || dst_height <= 0 || dst_stride < dst_width * channels) { nv_set_error("bad destination"); return NV_ERR_ARG; }
-    if ((rc = upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
+    if ((rc = nv_upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
     const int *d_rtab;
     if ((rc = nv_get_rtab(ctx, width, height, dst_width, dst_height, &d_rtab)) != NV_OK) return rc;
     if ((rc = ensure(&ctx->d_aux, &ctx->aux_cap, (size_t)dst_width * dst_height * channels)) != NV_OK) return rc;
@@ -1798,7 +1743,7 @@ extern "C" int nv_flip_horizontal(nv_ctx *ctx, const uint8_t *src, int width, in
     int rc = check_frame(ctx, src, width, height, stride_bytes, 1);
     if (rc != NV_OK) return rc;
     if (!dst || dst_stride < width) { nv_set_error("bad destination"); return NV_ERR_ARG; }
-    if ((rc = upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
+    if ((rc = nv_upload(ctx, src, (size_t)stride_bytes * height)) != NV_OK) return rc;
     NV_CUDA(launch_flip(ctx->d_frame, width, height, stride_bytes, ctx->d_gray, width, ctx->stream));
     ctx->launches++;
     return download(ctx, ctx->d_gray, width, height, dst, dst_stride);

@@ -195,13 +195,6 @@ bool clamp_roi(nv_rect &r, int W, int H)
     return true;
 }
 
-int upload_frame(nv_ctx *ctx, const uint8_t *frame, int stride, int h)
-{
-    if ((size_t)stride * h > ctx->frame_cap) { nv_set_error("frame larger than the element's context"); return NV_ERR_CAPACITY; }
-    if (ctx->pending) NV_CUDA(cudaStreamSynchronize(ctx->stream));
-    return nv_h2d(ctx, frame, (size_t)stride * h);
-}
-
 // first step of the nested elements (EYE:949, MOUTH:836, NOSE:834, EAR:786): the full-resolution gray image, from the BGR
 // frame or — for a 4:2:0 buffer — from cvtColor(COLOR_YUV2BGR_*) of its planes, per pixel
 int frame_to_gray(nv_element *e, nv_ctx *ctx, const uint8_t *frame, int stride, int W, int H, uint8_t *gray)
@@ -212,7 +205,7 @@ int frame_to_gray(nv_element *e, nv_ctx *ctx, const uint8_t *frame, int stride, 
         if ((r = nv_yuv_upload(ctx, e->yuv, &pl)) != NV_OK) return r;
         NV_CUDA(launch_yuv2gray(e->yuv->format, pl, W, H, gray, W, ctx->stream));
     } else {
-        if ((r = upload_frame(ctx, frame, stride, H)) != NV_OK) return r;
+        if ((r = nv_upload(ctx, frame, (size_t)stride * H)) != NV_OK) return r;
         NV_CUDA(launch_bgr2gray(ctx->d_frame, W, H, stride, 3, gray, W, ctx->stream));
     }
     ctx->launches++;
@@ -1284,9 +1277,8 @@ extern "C" int nv_element_transform_frame_device(nv_element *e, uint8_t *d_frame
                                                  uint64_t pts_ns, double now_ms)
 {
     if (!e || !d_frame) { nv_set_error("bad argument"); return NV_ERR_ARG; }
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, d_frame) != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)) {
-        cudaGetLastError();
+    const cudaMemoryType type = nv_memory_type(d_frame);
+    if (type != cudaMemoryTypeDevice && type != cudaMemoryTypeManaged) {
         nv_set_error("nv_element_transform_frame_device: the frame is not in device memory");
         return NV_ERR_ARG;
     }
@@ -1350,9 +1342,8 @@ extern "C" int nv_draw_shapes_device(nv_ctx *ctx, uint8_t *d_frame, int width, i
 {
     if (!ctx || !d_frame || width <= 0 || height <= 0 || (channels != 3 && channels != 4) || stride_bytes < width * channels || n < 0 ||
         (n > 0 && !shapes)) { nv_set_error("bad argument"); return NV_ERR_ARG; }
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, d_frame) != cudaSuccess || (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged)) {
-        cudaGetLastError();
+    const cudaMemoryType type = nv_memory_type(d_frame);
+    if (type != cudaMemoryTypeDevice && type != cudaMemoryTypeManaged) {
         nv_set_error("nv_draw_shapes_device: the frame is not in device memory");
         return NV_ERR_ARG;
     }

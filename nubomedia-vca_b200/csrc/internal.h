@@ -275,6 +275,14 @@ struct ResultHeader {
     int overflow;       // 1 if a capacity was hit
 };
 
+// The CUDA graph of one call path (graph_run in context.cu): `seen` is the key of the last call that ran plain launches,
+// `key` the key `exec` was captured for, `nl` its launch count and `prof_mask` the stage events (prof_set) it records.
+template <class Key> struct GraphCache {
+    cudaGraphExec_t exec = nullptr;  Key key, seen;  int nl = 0;  unsigned prof_mask = 0;
+    void drop() { if (exec) cudaGraphExecDestroy(exec); exec = nullptr; }     // the next call with `seen` captures again
+    void reset() { drop(); key = Key(); seen = Key(); }
+};
+
 // Everything that depends on one (image size, cascade window, parameters) key.  A context keeps the last
 // NV_PLAN_SLOTS of them: the nested elements run a differently sized ROI through the same context several times per
 // frame, and re-deriving + re-uploading a plan costs more than the detection itself on such small images.
@@ -297,7 +305,7 @@ struct PlanSlot {
     unsigned long long last_use = 0, buf_gen = 0;            // LRU clock; generation of the shared buffers the tensor maps point into
     unsigned long long gen = 0;                              // bumped whenever the slot's plan or parameter banks are rebuilt
     // CUDA graph of detect_enqueue on a device-resident image (the nested ROI stages replay it frame after frame)
-    cudaGraphExec_t dexec = nullptr;  DetGraphKey dkey, dkey_seen;  int d_nl = 0;
+    GraphCache<DetGraphKey> graph;
 };
 #define NV_PLAN_SLOTS 12
 
@@ -369,7 +377,7 @@ struct nv_ctx {
     uint2 *d_queue2 = nullptr;  size_t queue2_cap = 0;                       // second window queue: general cascades on large plans
     uint2 *d_deepq = nullptr;                                                // NV_DEEPQ_CAP windows that reach the block-per-window stages (small plans)
     uint32_t *d_tilt = nullptr;  size_t tilt_cap = 0;
-    cudaGraphExec_t gexec = nullptr;  GraphKey gkey, gkey_seen;  int g_nl = 0;  bool no_graph = false;  unsigned g_prof_mask = 0;
+    GraphCache<GraphKey> face_graph;  bool no_graph = false;
     unsigned long long epoch = 1;     // bumped whenever a buffer the pipeline binds is re-allocated or re-planned
 
     // last-call bookkeeping (kept so that collect() can re-run a call whose candidate buffers overflowed)
@@ -406,7 +414,7 @@ struct nv_ctx {
                    slot_gen == o.slot_gen;
         }
     };
-    cudaGraphExec_t bexec = nullptr;  BatchKey bkey, bkey_seen;  int b_nl = 0;
+    GraphCache<BatchKey> batch_graph;
     // last batch call: what collect needs (route, images, the overflow re-run's inputs), and what the counters tap reports
     bool batch_last = false, batch_routed = false, batch_replayed = false;  int batch_n = 0, batch_kind = 0;
     std::vector<const uint8_t *> batch_src;  int batch_w = 0, batch_h = 0, batch_stride = 0;  bool batch_on_device = false;
@@ -519,7 +527,10 @@ cudaError_t launch_cascade_tail_tab_batch(const PlanDev *plan, const DevCascade 
 cudaError_t launch_group_batch(const PlanDev *plan, int n, int *counters, const uint32_t *cand, int cand_stride, int cap, uint32_t *cand_sorted,
                                int4 *cand_rects, uint32_t *adj, size_t adj_stride, int *grp, int min_neighbors, double eps, int img_w,
                                int img_h, uint8_t *result, uint8_t *host_result, size_t result_stride, cudaStream_t st);
+// pageable host memory, and a pointer the runtime cannot place, read as cudaMemoryTypeUnregistered (error state cleared)
+cudaMemoryType nv_memory_type(const void *p);
 int nv_h2d(nv_ctx *ctx, const uint8_t *src, size_t bytes);
+int nv_upload(nv_ctx *ctx, const uint8_t *src, size_t bytes);      // nv_h2d after the capacity check and the pending call
 int nv_get_rtab(nv_ctx *ctx, int sw, int sh, int dw, int dh, const int **d_tab, const nv_ctx::RtabEntry **entry = nullptr);
 
 // kernels_group.cu

@@ -403,7 +403,7 @@ def test_prep_modes_and_alignment(ctx, face, case):
 @pytest.mark.parametrize("pinned", [False, True])
 def test_integer_downscale_uploads_row_pairs(face, case, pinned):
     """An integer down-scale by 3 or more (the element's default 640 -> 160) reads two of every `scale` source rows; only
-    those row pairs are uploaded (context.cu: nv_h2d_row_pairs; page-locked frames in place, others through the staging
+    those row pairs are uploaded (context.cu: upload_rows; page-locked frames in place, others through the staging
     buffer).  The rows that stay on the host are POISONED on the device side here by a first, full-size call with a frame of 0xFF, so a
     kernel that read one of them would not reproduce the oracle's gray image.  646x486 is the irregular case (646 / 160 = 4
     but 486 rows do not divide: the whole frame travels).  Non-debug context: graph replay on the third call."""
