@@ -177,7 +177,8 @@ NV_API int nv_host_unregister(void *p);
  *      nv_debug_get_counters reports [0..2] summed over its images, [3] the kernel launches of the whole call and [4] 1 when
  *      the batched chain was replayed from a CUDA graph captured by an earlier call (0 otherwise); the other
  *      parity taps, nv_get_scores and nv_ctx_get_stage_times return NV_ERR_STATE (they describe single calls); a pending
- *      batch is collected with nv_face_collect_batch only. ---------------------------------------------------------------- */
+ *      batch is collected with nv_face_collect_batch only.  Batches of 4:2:0 frames: nv_face_submit_batch_yuv /
+ *      nv_face_detect_batch_yuv below. ------------------------------------------------------------------------------------ */
 #define NV_BATCH_MAX 256
 NV_API int nv_detect_multiscale_batch(nv_ctx *ctx, const nv_cascade *c, const uint8_t *const *frames, int n, int width, int height,
                                       int stride_bytes, int on_device, const nv_detect_params *p, nv_rect *out, int cap, int *counts);
@@ -209,6 +210,19 @@ typedef struct {
 NV_API int nv_face_detect_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *f, const nv_face_params *p,
                               nv_rect *out, int cap, int *n);
 NV_API int nv_face_submit_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *f, const nv_face_params *p);   /* + nv_face_collect */
+/* Batches of 4:2:0 frames: the face batch calls above (same route, results, counts, capacity, limits and refusals; a pending
+ * batch is collected with nv_face_collect_batch) on n decoder frames.  Every frame passes the checks of nv_face_detect_yuv,
+ * and all share format, width, height, plane strides (stride[2] of I420 only) and on_device, else NV_ERR_ARG naming the
+ * first frame that differs.  Each frame's planes may lie anywhere: one block or scattered, pageable, page-locked (read in
+ * place until collect) or, with on_device, device memory (read in place, no copy).  Image i's rectangles are exactly
+ * those of nv_face_detect_yuv on frame i.  On the batched route, host frames travel plane by plane: of the luma plane only
+ * the row pairs the resize reads, the chroma planes whole.  A 640x480 NV12 frame processed at 160x120 moves 307 200 bytes
+ * (120 luma row pairs, 153 600 bytes, and the 153 600-byte chroma plane), against 460 800 for the BGR frame's row pairs in
+ * nv_face_detect_batch. */
+NV_API int nv_face_submit_batch_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n,
+                                    const nv_face_params *p);
+NV_API int nv_face_detect_batch_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n,
+                                    const nv_face_params *p, nv_rect *out, int cap, int *counts, int *total);
 /* cvtColor(COLOR_YUV2BGR_*) alone, host in / host out (parity tap of the ingest arithmetic) */
 NV_API int nv_yuv2bgr(nv_ctx *ctx, const nv_yuv_frame *f, uint8_t *dst_bgr, int dst_stride);
 

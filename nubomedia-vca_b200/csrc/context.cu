@@ -1120,9 +1120,6 @@ int nv_get_rtab(nv_ctx *ctx, int sw, int sh, int dw, int dh, const int **d_tab, 
     return NV_OK;
 }
 
-// Source frame of the face block: interleaved BGR (p[0], s[0]) or the planes of a 4:2:0 frame.
-struct FaceSrc { int fmt; const uint8_t *p[3]; int s[3]; bool on_device; };
-
 // Host planes of a 4:2:0 frame -> ctx->d_frame.  Planes that lie in one ascending block of host memory (a GstVideoFrame
 // mapped from a single GstMemory, a cv::Mat of h*3/2 rows) travel as ONE copy and keep their relative offsets; scattered
 // planes are copied one by one to 256-byte aligned offsets.  Fills the device plane pointers.
@@ -1409,8 +1406,8 @@ static int batch_buffers(nv_ctx *ctx, int n, size_t frame_bytes, size_t gray_byt
             NV_CUDA(cudaMalloc(&b.d_result, N * BATCH_RESULT_BYTES));
             NV_CUDA(cudaMallocHost(&b.h_result, N * BATCH_RESULT_BYTES));
             memset(b.h_result, 0, N * BATCH_RESULT_BYTES);
-            NV_CUDA(cudaMalloc(&b.d_tab, 2 * N * sizeof(uint8_t *)));
-            NV_CUDA(cudaMallocHost(&b.h_tab, 2 * N * sizeof(uint8_t *)));
+            NV_CUDA(cudaMalloc(&b.d_tab, 4 * N * sizeof(uint8_t *)));
+            NV_CUDA(cudaMallocHost(&b.h_tab, 4 * N * sizeof(uint8_t *)));
             return NV_OK;
         }();
         if (rc != NV_OK) { batch_free(b); return rc; }
@@ -1419,11 +1416,13 @@ static int batch_buffers(nv_ctx *ctx, int n, size_t frame_bytes, size_t gray_byt
     return NV_OK;
 }
 
-enum { BATCH_GRAY = 1, BATCH_FACE = 2 };
+// gray images, face detection on BGR frames, face detection on 4:2:0 frames
+enum { BATCH_GRAY = 1, BATCH_FACE = 2, BATCH_YUV = 3 };
 
-// the stream-ordered chain of the batched route: six launches whatever n is (five for gray images)
-static int batch_enqueue(nv_ctx *ctx, nv_cascade *casc, int kind, int n, int w, int h, int stride, int cols, int rows, const int *rtab,
-                         bool aligned, int min_neighbors, int *nlaunch)
+// the stream-ordered chain of the batched route: six launches whatever n is (five for gray images).  f: format and plane
+// strides of every image; the device table holds the image planes (one per image, three for 4:2:0), then the gray images.
+static int batch_enqueue(nv_ctx *ctx, nv_cascade *casc, int kind, int n, int w, int h, const FaceSrc &f, int cols, int rows,
+                         const int *rtab, bool aligned, int min_neighbors, int *nlaunch)
 {
     nv_ctx::Batch &b = ctx->b;
     const PlanDev &P = ctx->ps->plan;
@@ -1431,11 +1430,16 @@ static int batch_enqueue(nv_ctx *ctx, nv_cascade *casc, int kind, int n, int w, 
     const int qcap = (int)(n * b.wins);
     const uint8_t *const *grays = b.d_tab;
     const uint8_t *lut = ctx->d_lut + 256;                   // gray images: the identity LUT
-    int lut_stride = 0, gstride = stride, nl = 0;
+    int lut_stride = 0, gstride = f.s[0], nl = 0;
     if (kind == BATCH_FACE) {
-        NV_CUDA(launch_face_prep_batch(b.d_tab, n, aligned, w, h, stride, b.d_gray, cols, rows, rtab, b.d_hist, b.d_lut, st));
-        grays = b.d_tab + n; lut = b.d_lut; lut_stride = 256; gstride = cols; nl++;
+        NV_CUDA(launch_face_prep_batch(b.d_tab, n, aligned, w, h, f.s[0], b.d_gray, cols, rows, rtab, b.d_hist, b.d_lut, st));
+        grays = b.d_tab + n;
+    } else if (kind == BATCH_YUV) {
+        NV_CUDA(launch_face_prep_yuv_batch(f.fmt, b.d_tab, n, aligned, f.s[0], f.s[1], f.s[2], w, h, b.d_gray, cols, rows, rtab, b.d_hist,
+                                           b.d_lut, st));
+        grays = b.d_tab + 3 * n;
     }
+    if (kind != BATCH_GRAY) { lut = b.d_lut; lut_stride = 256; gstride = cols; nl++; }
     NV_CUDA(launch_pyramid_batch(ctx->ps->d_plan, P.total_rowblk, P.total_colblk, n, grays, gstride, lut, lut_stride, ctx->ps->d_ptab,
                                  b.d_sum, b.d_sq, b.integ, st));
     Stage0Params &sp = ctx->ps->s0p;
@@ -1453,19 +1457,18 @@ static int batch_enqueue(nv_ctx *ctx, nv_cascade *casc, int kind, int n, int w, 
 }
 
 // one image of a batch through the single-image pipeline, collected into ctx->batch_out (appended; count in ctx->batch_counts[i])
-static int batch_single(nv_ctx *ctx, int i, const uint8_t *src, bool on_device)
+static int batch_single(nv_ctx *ctx, int i, const FaceSrc &src)
 {
     int rc;
-    if (ctx->batch_kind == BATCH_FACE) {
-        FaceSrc fs = {NV_FMT_BGR, {src, nullptr, nullptr}, {ctx->batch_stride, 0, 0}, on_device};
-        rc = face_submit_impl(ctx, ctx->batch_casc, fs, ctx->batch_w, ctx->batch_h, &ctx->batch_fp);
+    if (ctx->batch_kind != BATCH_GRAY) {
+        rc = face_submit_impl(ctx, ctx->batch_casc, src, ctx->batch_w, ctx->batch_h, &ctx->batch_fp);
     } else {
-        const uint8_t *d = src;
-        if (!on_device) {
-            if ((rc = nv_h2d(ctx, src, (size_t)ctx->batch_stride * ctx->batch_h)) != NV_OK) return rc;
+        const uint8_t *d = src.p[0];
+        if (!src.on_device) {
+            if ((rc = nv_h2d(ctx, d, (size_t)src.s[0] * ctx->batch_h)) != NV_OK) return rc;
             d = ctx->d_frame;
         }
-        rc = nv_detect_device(ctx, ctx->batch_casc, d, ctx->batch_w, ctx->batch_h, ctx->batch_stride, ctx->d_lut + 256, &ctx->batch_dp);
+        rc = nv_detect_device(ctx, ctx->batch_casc, d, ctx->batch_w, ctx->batch_h, src.s[0], ctx->d_lut + 256, &ctx->batch_dp);
     }
     if (rc != NV_OK) return rc;
     const size_t base = ctx->batch_out.size();
@@ -1495,16 +1498,51 @@ static int batch_check(nv_ctx *ctx, const nv_cascade *c, const uint8_t *const *f
     return NV_OK;
 }
 
-static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *const *frames, int n, int w, int h, int stride,
-                        bool on_device, const nv_face_params *fp, const nv_detect_params *gp)
+// BGR or gray frames as batch sources: one plane each
+static std::vector<FaceSrc> batch_sources(const uint8_t *const *frames, int n, int stride, int on_device)
 {
+    std::vector<FaceSrc> v(n);
+    for (int i = 0; i < n; i++) v[i] = FaceSrc{NV_FMT_BGR, {frames[i], nullptr, nullptr}, {stride, 0, 0}, on_device != 0};
+    return v;
+}
+
+// 4:2:0 frames: every frame passes check_yuv, and all share format, size, plane strides and on_device
+static int batch_check_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n, const nv_face_params *p,
+                           std::vector<FaceSrc> *srcs)
+{
+    if (!ctx || !c || !frames || !p) { nv_set_error("null argument"); return NV_ERR_ARG; }
+    if (n < 1 || n > NV_BATCH_MAX) { nv_set_error("batch of %d images: 1 .. %d are supported", n, NV_BATCH_MAX); return NV_ERR_ARG; }
+    srcs->resize(n);
+    const nv_yuv_frame &f0 = frames[0];
+    for (int i = 0; i < n; i++) {
+        const nv_yuv_frame &f = frames[i];
+        if (f.format != f0.format || f.width != f0.width || f.height != f0.height || f.stride[0] != f0.stride[0] ||
+            f.stride[1] != f0.stride[1] || (f.format == NV_FMT_I420 && f.stride[2] != f0.stride[2]) || (f.on_device != 0) != (f0.on_device != 0)) {
+            nv_set_error("image %d differs from image 0 in format, size, plane strides or on_device", i);
+            return NV_ERR_ARG;
+        }
+        const int rc = check_yuv(ctx, &f, &(*srcs)[i]);
+        if (rc != NV_OK) {
+            const std::string why = nv_last_error();
+            nv_set_error("image %d: %s", i, why.c_str());
+            return rc;
+        }
+    }
+    if (ctx->scores) { nv_set_error("batch calls do not compute scores: switch them off with nv_ctx_set_scores(ctx, 0)"); return NV_ERR_STATE; }
+    return NV_OK;
+}
+
+static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const std::vector<FaceSrc> &srcs, int w, int h,
+                        const nv_face_params *fp, const nv_detect_params *gp)
+{
+    const int n = (int)srcs.size();
     NV_CUDA(cudaSetDevice(ctx->gpu));
     if (ctx->pending) NV_CUDA(cudaStreamSynchronize(ctx->stream));
     ctx->pending = false;
     int rc, cols = w, rows = h, row_a = 0, row_period = 0;
     const int *d_rtab = nullptr;
     nv_detect_params dp;
-    if (kind == BATCH_FACE) {
+    if (kind != BATCH_GRAY) {
         if (fp->width_to_process <= 0) { nv_set_error("width_to_process must be > 0 (kmsfacedetect.cpp:304 divides by it)"); return NV_ERR_ARG; }
         face_geometry(w, h, fp, &cols, &rows, &dp);
         const nv_ctx::RtabEntry *rt = nullptr;
@@ -1515,9 +1553,8 @@ static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *
         dp = *gp;
         ctx->batch_dp = *gp;
     }
-    ctx->batch_casc = casc; ctx->batch_kind = kind; ctx->batch_n = n; ctx->batch_w = w; ctx->batch_h = h; ctx->batch_stride = stride;
-    ctx->batch_on_device = on_device;
-    ctx->batch_src.assign(frames, frames + n);
+    ctx->batch_casc = casc; ctx->batch_kind = kind; ctx->batch_n = n; ctx->batch_w = w; ctx->batch_h = h;
+    ctx->batch_src = srcs;
     ctx->batch_out.clear(); ctx->batch_counts.assign(n, 0);
     ctx->batch_sum[0] = ctx->batch_sum[1] = ctx->batch_sum[2] = 0;
     const long long launches0 = ctx->launches;
@@ -1526,56 +1563,72 @@ static int batch_submit(nv_ctx *ctx, nv_cascade *casc, int kind, const uint8_t *
     if (!ctx->batch_routed) {
         // sequential fallback: the single-image pipeline once per image, collected here
         for (int i = 0; i < n; i++)
-            if ((rc = batch_single(ctx, i, frames[i], on_device)) != NV_OK) { ctx->batch_last = true; return rc; }
+            if ((rc = batch_single(ctx, i, srcs[i])) != NV_OK) { ctx->batch_last = true; return rc; }
         ctx->batch_launches = ctx->launches - launches0;
         ctx->batch_last = true;
         ctx->pending = true;
         return NV_OK;
     }
-    const size_t fbytes = (size_t)stride * h;
+    // an uploaded image holds its planes one after another, each rounded up to 256 bytes (NV12 / NV21: plane 2 is empty)
+    const FaceSrc &f0 = srcs[0];
+    const bool on_device = f0.on_device;
+    const int np = kind == BATCH_YUV ? 3 : 1, plane_h[3] = {h, h / 2, h / 2};
+    size_t off[4] = {0, 0, 0, 0};
+    for (int k = 0; k < np; k++) off[k + 1] = off[k] + (((size_t)f0.s[k] * plane_h[k] + 255) & ~(size_t)255);
+    const size_t fbytes = off[np];
     bool pageable = false;
-    std::vector<cudaMemoryType> types(on_device ? 0 : n);
-    for (size_t i = 0; i < types.size(); i++) {
-        types[i] = nv_memory_type(frames[i]);
-        pageable = pageable || types[i] == cudaMemoryTypeUnregistered;
-    }
-    if ((rc = batch_buffers(ctx, n, on_device ? 0 : fbytes, kind == BATCH_FACE ? (size_t)cols * rows : 0, pageable)) != NV_OK) return rc;
-    nv_ctx::Batch &b = ctx->b;
-    bool aligned = (stride & 3) == 0;
-    for (int i = 0; i < n; i++) {
-        const uint8_t *d = frames[i];
-        if (!on_device) {
-            uint8_t *dst = b.d_frame + i * fbytes;
-            if ((rc = upload_rows(ctx, dst, b.h_stage ? b.h_stage + i * fbytes : nullptr, frames[i], types[i], stride, h, row_a, row_period,
-                                  rows)) != NV_OK) return rc;
-            d = dst;
+    std::vector<cudaMemoryType> types(on_device ? 0 : (size_t)n * np, cudaMemoryTypeDevice);
+    for (int i = 0; i < n && !on_device; i++)
+        for (int k = 0; k < np; k++) {
+            if (!srcs[i].p[k]) continue;
+            types[i * np + k] = nv_memory_type(srcs[i].p[k]);
+            pageable = pageable || types[i * np + k] == cudaMemoryTypeUnregistered;
         }
-        aligned = aligned && ((uintptr_t)d & 3u) == 0;
-        b.h_tab[i] = d;
-        b.h_tab[n + i] = kind == BATCH_FACE ? b.d_gray + (size_t)i * cols * rows : d;
+    if ((rc = batch_buffers(ctx, n, on_device ? 0 : fbytes, kind != BATCH_GRAY ? (size_t)cols * rows : 0, pageable)) != NV_OK) return rc;
+    nv_ctx::Batch &b = ctx->b;
+    bool aligned = ((f0.s[0] | f0.s[1] | f0.s[2]) & 3) == 0;
+    for (int i = 0; i < n; i++) {
+        for (int k = 0; k < np; k++) {
+            const uint8_t *d = srcs[i].p[k];
+            if (d && !on_device) {
+                // the frame or luma plane: only the row pairs the resize reads; a chroma plane whole (at period 4 the vertical
+                // pass reads every chroma row)
+                uint8_t *dst = b.d_frame + i * fbytes + off[k];
+                if ((rc = upload_rows(ctx, dst, b.h_stage ? b.h_stage + i * fbytes + off[k] : nullptr, d, types[i * np + k], f0.s[k],
+                                      plane_h[k], k == 0 ? row_a : 0, k == 0 ? row_period : 0, rows)) != NV_OK) return rc;
+                d = dst;
+            }
+            aligned = aligned && ((uintptr_t)d & 3u) == 0;
+            b.h_tab[np * i + k] = d;
+        }
+        b.h_tab[np * n + i] = kind != BATCH_GRAY ? b.d_gray + (size_t)i * cols * rows : b.h_tab[i];
     }
     // host frames always land at the same places: the table is only copied when it changes (device frames, a new shape)
-    if (!std::equal(b.h_tab, b.h_tab + 2 * n, b.tab_last.begin(), b.tab_last.end())) {
-        NV_CUDA(cudaMemcpyAsync(b.d_tab, b.h_tab, 2 * (size_t)n * sizeof(uint8_t *), cudaMemcpyHostToDevice, ctx->stream));
-        b.tab_last.assign(b.h_tab, b.h_tab + 2 * n);
+    const size_t ntab = (size_t)(np + 1) * n;
+    if (!std::equal(b.h_tab, b.h_tab + ntab, b.tab_last.begin(), b.tab_last.end())) {
+        NV_CUDA(cudaMemcpyAsync(b.d_tab, b.h_tab, ntab * sizeof(uint8_t *), cudaMemcpyHostToDevice, ctx->stream));
+        b.tab_last.assign(b.h_tab, b.h_tab + ntab);
     }
     // the repeated shape replays as one CUDA graph; frame addresses reach it through the table, so they are not part of the key
     nv_ctx::BatchKey key;
-    key.kind = kind; key.n = n; key.w = w; key.h = h; key.stride = stride; key.cols = cols; key.rows = rows; key.rtab = d_rtab;
+    key.kind = kind; key.n = n; key.w = w; key.h = h; key.stride = f0.s[0]; key.cols = cols; key.rows = rows; key.rtab = d_rtab;
+    key.fmt = f0.fmt; key.s1 = f0.s[1]; key.s2 = f0.s[2];
     key.aligned = aligned; key.casc = casc->uid; key.sf = dp.scale_factor; key.mn = dp.min_neighbors; key.min_w = dp.min_w;
     key.min_h = dp.min_h; key.max_w = dp.max_w; key.max_h = dp.max_h; key.epoch = ctx->epoch; key.bgen = b.gen; key.slot = ctx->ps;
     key.slot_gen = ctx->ps->gen;
     int nl;
     GraphRun how;
     rc = graph_run(ctx, ctx->batch_graph, key, !ctx->debug && !ctx->no_graph,
-                   [&](int *c) { return batch_enqueue(ctx, casc, kind, n, w, h, stride, cols, rows, d_rtab, aligned, dp.min_neighbors, c); },
+                   [&](int *c) { return batch_enqueue(ctx, casc, kind, n, w, h, f0, cols, rows, d_rtab, aligned, dp.min_neighbors, c); },
                    &nl, &how);
     ctx->batch_replayed = how == RUN_REPLAYED;
     if (rc != NV_OK) return rc;
     ctx->launches += nl;
     ctx->batch_launches = nl;
-    for (int i = 0; i < n; i++) ctx->batch_src[i] = b.h_tab[i];   // device copies: what an overflow re-run in collect reads
-    ctx->batch_on_device = true;
+    for (int i = 0; i < n; i++) {                 // device copies: what an overflow re-run in collect reads
+        for (int k = 0; k < np; k++) ctx->batch_src[i].p[k] = b.h_tab[np * i + k];
+        ctx->batch_src[i].on_device = true;
+    }
     ctx->batch_last = true;
     ctx->pending = true;
     return NV_OK;
@@ -1609,7 +1662,7 @@ static int batch_collect(nv_ctx *ctx, nv_rect *out, int cap, int *counts, int *t
             }
             // the re-run reads the image's device copy (or the caller's device frame); batch_single appends to batch_out
             ctx->batch_out.clear();
-            if ((rc = batch_single(ctx, i, ctx->batch_src[i], true)) != NV_OK) break;
+            if ((rc = batch_single(ctx, i, ctx->batch_src[i])) != NV_OK) break;
             rects.insert(rects.end(), ctx->batch_out.begin(), ctx->batch_out.end());
             cnt[i] = ctx->batch_counts[i];
         }
@@ -1632,7 +1685,8 @@ extern "C" int nv_face_submit_batch(nv_ctx *ctx, const nv_cascade *c, const uint
 {
     int rc = batch_check(ctx, c, frames, n, width, height, stride_bytes, 3, p);
     if (rc != NV_OK) return rc;
-    return batch_submit(ctx, const_cast<nv_cascade *>(c), BATCH_FACE, frames, n, width, height, stride_bytes, on_device != 0, p, nullptr);
+    return batch_submit(ctx, const_cast<nv_cascade *>(c), BATCH_FACE, batch_sources(frames, n, stride_bytes, on_device), width, height, p,
+                        nullptr);
 }
 
 extern "C" int nv_face_collect_batch(nv_ctx *ctx, nv_rect *out, int cap, int *counts, int *total)
@@ -1655,9 +1709,27 @@ extern "C" int nv_detect_multiscale_batch(nv_ctx *ctx, const nv_cascade *c, cons
     if (!counts) { nv_set_error("null argument"); return NV_ERR_ARG; }
     int rc = batch_check(ctx, c, frames, n, width, height, stride_bytes, 1, p);
     if (rc != NV_OK) return rc;
-    if ((rc = batch_submit(ctx, const_cast<nv_cascade *>(c), BATCH_GRAY, frames, n, width, height, stride_bytes, on_device != 0, nullptr, p)) != NV_OK)
+    if ((rc = batch_submit(ctx, const_cast<nv_cascade *>(c), BATCH_GRAY, batch_sources(frames, n, stride_bytes, on_device), width, height,
+                           nullptr, p)) != NV_OK)
         return rc;
     return batch_collect(ctx, out, cap, counts, nullptr);
+}
+
+extern "C" int nv_face_submit_batch_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n, const nv_face_params *p)
+{
+    std::vector<FaceSrc> srcs;
+    int rc = batch_check_yuv(ctx, c, frames, n, p, &srcs);
+    if (rc != NV_OK) return rc;
+    return batch_submit(ctx, const_cast<nv_cascade *>(c), BATCH_YUV, srcs, frames[0].width, frames[0].height, p, nullptr);
+}
+
+extern "C" int nv_face_detect_batch_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n, const nv_face_params *p,
+                                        nv_rect *out, int cap, int *counts, int *total)
+{
+    if (!counts) { nv_set_error("null argument"); return NV_ERR_ARG; }
+    int rc = nv_face_submit_batch_yuv(ctx, c, frames, n, p);
+    if (rc != NV_OK) return rc;
+    return batch_collect(ctx, out, cap, counts, total);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -312,6 +312,9 @@ struct PlanSlot {
 // byte offsets of the tracker's per-tile scratch inside nv_ctx::d_trk_scratch (kernels_tracker.cu)
 struct TrkLayout { int ntx, nty; size_t bbox, rects, out, bseed, parent, slotlist, bcount, keys, bslot, counters, edge_flag, zero_begin, zero_end; };
 
+// Source frame of the face block: interleaved BGR (p[0], s[0]) or the planes of a 4:2:0 frame.
+struct FaceSrc { int fmt; const uint8_t *p[3]; int s[3]; bool on_device; };
+
 struct nv_ctx {
     int gpu = 0;
     int max_w = 0, max_h = 0;
@@ -388,7 +391,8 @@ struct nv_ctx {
     int last_min_neighbors = 0;
     long long launches = 0;
 
-    // batched route (nv_detect_multiscale_batch / nv_face_submit_batch): per-image buffers, grow-only, sized for bcap images
+    // batched route (nv_detect_multiscale_batch / nv_face_submit_batch / nv_face_submit_batch_yuv): per-image buffers, grow-only,
+    // sized for cap images
     struct Batch {
         int cap = 0;                                        // images the per-image buffers below hold
         size_t frame_bytes = 0, gray_bytes = 0, integ = 0, wins = 0, bits = 0;   // per-image sizes the buffers were made for
@@ -399,16 +403,18 @@ struct nv_ctx {
         uint32_t *d_adj = nullptr;  int *d_grp = nullptr;
         int *d_counters = nullptr;                          // 16 shared + 16 per image
         uint8_t *d_result = nullptr, *h_result = nullptr;   // per image: ResultHeader + NV_BATCH_GROUP_CAP rects
-        const uint8_t **d_tab = nullptr, **h_tab = nullptr; // per call: N source frames, N gray images
+        const uint8_t **d_tab = nullptr, **h_tab = nullptr; // per call: N source frames (3N planes of 4:2:0 frames), N gray images
         std::vector<const uint8_t *> tab_last;             // what d_tab holds
         unsigned long long gen = 1;                         // bumped whenever a buffer above moves
     } b;
     struct BatchKey {
         int kind = 0, n = 0, w = 0, h = 0, stride = 0, cols = 0, rows = 0; const int *rtab = nullptr; bool aligned = false;
+        int fmt = 0, s1 = 0, s2 = 0;                        // 4:2:0 frames: format, chroma strides
         unsigned long long casc = 0; double sf = 0; int mn = 0, min_w = 0, min_h = 0, max_w = 0, max_h = 0;
         unsigned long long epoch = 0, bgen = 0; const PlanSlot *slot = nullptr; unsigned long long slot_gen = 0;
         bool operator==(const BatchKey &o) const {
             return kind == o.kind && n == o.n && w == o.w && h == o.h && stride == o.stride && cols == o.cols && rows == o.rows &&
+                   fmt == o.fmt && s1 == o.s1 && s2 == o.s2 &&
                    rtab == o.rtab && aligned == o.aligned && casc == o.casc && sf == o.sf && mn == o.mn && min_w == o.min_w &&
                    min_h == o.min_h && max_w == o.max_w && max_h == o.max_h && epoch == o.epoch && bgen == o.bgen && slot == o.slot &&
                    slot_gen == o.slot_gen;
@@ -417,7 +423,7 @@ struct nv_ctx {
     GraphCache<BatchKey> batch_graph;
     // last batch call: what collect needs (route, images, the overflow re-run's inputs), and what the counters tap reports
     bool batch_last = false, batch_routed = false, batch_replayed = false;  int batch_n = 0, batch_kind = 0;
-    std::vector<const uint8_t *> batch_src;  int batch_w = 0, batch_h = 0, batch_stride = 0;  bool batch_on_device = false;
+    std::vector<FaceSrc> batch_src;  int batch_w = 0, batch_h = 0;
     nv_face_params batch_fp = {};  nv_detect_params batch_dp = {};  nv_cascade *batch_casc = nullptr;
     long long batch_sum[3] = {0, 0, 0}, batch_launches = 0;
     std::vector<nv_rect> batch_out;  std::vector<int> batch_counts;      // collected rectangles (image after image) and counts
@@ -517,6 +523,9 @@ int nv_collect(nv_ctx *ctx, nv_rect *out, int cap, int *n);
 // kernels of the batched route (one launch each for the whole batch)
 cudaError_t launch_face_prep_batch(const uint8_t *const *srcs, int n, bool aligned, int sw, int sh, int sstride, uint8_t *gray,
                                    int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st);
+// planes: 3 pointers per image (Y, U|UV|VU, V; the third unused for NV12 / NV21); s0..s2: plane strides of every image
+cudaError_t launch_face_prep_yuv_batch(int fmt, const uint8_t *const *planes, int n, bool aligned, int s0, int s1, int s2, int sw,
+                                       int sh, uint8_t *gray, int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st);
 cudaError_t launch_pyramid_batch(const PlanDev *plan, int total_rowblk, int total_colblk, int n, const uint8_t *const *grays, int gstride,
                                  const uint8_t *lut, int lut_stride, const int *ptab, uint32_t *sum, uint32_t *sq, size_t integ_stride,
                                  cudaStream_t st);

@@ -218,12 +218,19 @@ k_face_prep_bgr4(const uint8_t *__restrict__ src, int sstride, uint8_t *__restri
 // ---- 4:2:0 ingest (SURVEY §8f rank 4): the same block fed by I420 / NV12 / NV21 planes.  Every source pixel the
 // resize touches is converted with cvtColor(COLOR_YUV2BGR_*)'s arithmetic (BT.601, 20-bit fixed point, saturated to
 // u8 per pixel; oracle: ora_yuv420_to_bgr), so the result equals the reference block on the converted BGR frame.
-template <int FMT>
+// BATCH: image blockIdx.y takes its three plane pointers from planes[3 * blockIdx.y ..] (the strides in s are shared by
+// all images) and owns gray, histogram (+ ticket) and LUT at blockIdx.y times the strides, as in k_face_prep.
+template <int FMT, bool BATCH>
 __global__ void __launch_bounds__(256)
 k_face_prep_yuv(SrcPlanes s, int sw, int sh, uint8_t *__restrict__ gray, int dw, int dh, const int *__restrict__ rtab,
-                int *__restrict__ hist, uint8_t *__restrict__ lut)
+                int *__restrict__ hist, uint8_t *__restrict__ lut, const uint8_t *const *__restrict__ planes = nullptr,
+                size_t gray_stride = 0)
 {
     __shared__ int sh_hist[256];
+    if (BATCH) {
+        s.p0 = planes[3 * blockIdx.y]; s.p1 = planes[3 * blockIdx.y + 1]; s.p2 = planes[3 * blockIdx.y + 2];
+        gray += blockIdx.y * gray_stride; hist += blockIdx.y * NV_HIST_STRIDE; lut += blockIdx.y * 256;
+    }
     int tid = threadIdx.y * 32 + threadIdx.x;
     sh_hist[tid] = 0;
     __syncthreads();
@@ -258,7 +265,7 @@ k_face_prep_yuv(SrcPlanes s, int sw, int sh, uint8_t *__restrict__ gray, int dw,
         gray[(size_t)y * dw + x] = (uint8_t)g;
         atomicAdd(&sh_hist[g], 1);
     }
-    prep_finish(tid, sh_hist, hist, lut, dw * dh);
+    prep_finish<BATCH>(tid, sh_hist, hist, lut, dw * dh);
 }
 
 // Vectorised 4:2:0 forms: a lane owns four consecutive output pixels.  Copy mode: 4 luma bytes (one word) and their
@@ -278,11 +285,16 @@ __device__ __forceinline__ void yuv_px(int yv, const YuvTerms &t, int c3[3])
     c3[0] = sat_u8((yy + t.b) >> 20); c3[1] = sat_u8((yy + t.g) >> 20); c3[2] = sat_u8((yy + t.r) >> 20);
 }
 
-template <int FMT, int MODE>
+template <int FMT, int MODE, bool BATCH>
 __global__ void __launch_bounds__(256)
-k_face_prep_yuv4(SrcPlanes s, uint8_t *__restrict__ gray, int dw, int dh, int *__restrict__ hist, uint8_t *__restrict__ lut)
+k_face_prep_yuv4(SrcPlanes s, uint8_t *__restrict__ gray, int dw, int dh, int *__restrict__ hist, uint8_t *__restrict__ lut,
+                 const uint8_t *const *__restrict__ planes = nullptr, size_t gray_stride = 0)
 {
     __shared__ int sh_hist[256];
+    if (BATCH) {
+        s.p0 = planes[3 * blockIdx.y]; s.p1 = planes[3 * blockIdx.y + 1]; s.p2 = planes[3 * blockIdx.y + 2];
+        gray += blockIdx.y * gray_stride; hist += blockIdx.y * NV_HIST_STRIDE; lut += blockIdx.y * 256;
+    }
     int tid = threadIdx.y * 32 + threadIdx.x;
     sh_hist[tid] = 0;
     __syncthreads();
@@ -343,7 +355,7 @@ k_face_prep_yuv4(SrcPlanes s, uint8_t *__restrict__ gray, int dw, int dh, int *_
 #pragma unroll
         for (int k = 0; k < 4; k++) atomicAdd(&sh_hist[g[k]], 1);
     }
-    prep_finish(tid, sh_hist, hist, lut, dw * dh);
+    prep_finish<BATCH>(tid, sh_hist, hist, lut, dw * dh);
 }
 
 // BGR2GRAY(cvtColor(COLOR_YUV2BGR_*)) at full resolution: the first step of the nested elements on 4:2:0 frames
@@ -487,13 +499,41 @@ static cudaError_t launch_prep_yuv_fmt(const SrcPlanes &s, int sw, int sh, uint8
     const bool al = aligned4(s.p0, s.s0) && aligned4(s.p1, s.s1) && (FMT != 1 || aligned4(s.p2, s.s2)) && aligned4(gray, 0);
     if (mode != RT_LINEAR && (dw & 3) == 0 && al) {
         int tiles = ((dw / 4 + 31) / 32) * ((dh + 7) / 8);
-        if (mode == RT_COPY) k_face_prep_yuv4<FMT, RT_COPY><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut);
-        else k_face_prep_yuv4<FMT, RT_BOX2><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut);
+        if (mode == RT_COPY) k_face_prep_yuv4<FMT, RT_COPY, false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut);
+        else k_face_prep_yuv4<FMT, RT_BOX2, false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut);
         return cudaGetLastError();
     }
     int tiles = ((dw + 31) / 32) * ((dh + 7) / 8);
-    k_face_prep_yuv<FMT><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, sw, sh, gray, dw, dh, rtab, hist, lut);
+    k_face_prep_yuv<FMT, false><<<prep_grid(tiles), dim3(32, 8), 0, st>>>(s, sw, sh, gray, dw, dh, rtab, hist, lut);
     return cudaGetLastError();
+}
+
+// aligned: every plane pointer of every image and every plane stride is 4-byte aligned (the vectorised kernel's rule)
+template <int FMT>
+static cudaError_t launch_prep_yuv_batch_fmt(const uint8_t *const *planes, int n, bool aligned, const SrcPlanes &s, int sw, int sh,
+                                             uint8_t *gray, int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st)
+{
+    const int mode = (sw == dw && sh == dh) ? RT_COPY : (sw == 2 * dw && sh == 2 * dh) ? RT_BOX2 : RT_LINEAR;   // = rtab[0]
+    const size_t gs = (size_t)dw * dh;
+    if (mode != RT_LINEAR && (dw & 3) == 0 && aligned) {
+        const dim3 grid(prep_grid(((dw / 4 + 31) / 32) * ((dh + 7) / 8)), n);
+        if (mode == RT_COPY) k_face_prep_yuv4<FMT, RT_COPY, true><<<grid, dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut, planes, gs);
+        else k_face_prep_yuv4<FMT, RT_BOX2, true><<<grid, dim3(32, 8), 0, st>>>(s, gray, dw, dh, hist, lut, planes, gs);
+        return cudaGetLastError();
+    }
+    const dim3 grid(prep_grid(((dw + 31) / 32) * ((dh + 7) / 8)), n);
+    k_face_prep_yuv<FMT, true><<<grid, dim3(32, 8), 0, st>>>(s, sw, sh, gray, dw, dh, rtab, hist, lut, planes, gs);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_face_prep_yuv_batch(int fmt, const uint8_t *const *planes, int n, bool aligned, int s0, int s1, int s2, int sw,
+                                       int sh, uint8_t *gray, int dw, int dh, const int *rtab, int *hist, uint8_t *lut, cudaStream_t st)
+{
+    const SrcPlanes s = {nullptr, nullptr, nullptr, s0, s1, s2};
+    if (fmt == NV_FMT_I420) return launch_prep_yuv_batch_fmt<1>(planes, n, aligned, s, sw, sh, gray, dw, dh, rtab, hist, lut, st);
+    if (fmt == NV_FMT_NV12) return launch_prep_yuv_batch_fmt<2>(planes, n, aligned, s, sw, sh, gray, dw, dh, rtab, hist, lut, st);
+    if (fmt == NV_FMT_NV21) return launch_prep_yuv_batch_fmt<3>(planes, n, aligned, s, sw, sh, gray, dw, dh, rtab, hist, lut, st);
+    return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_face_prep_yuv(int fmt, const SrcPlanes &s, int sw, int sh, uint8_t *gray, int dw, int dh, const int *rtab,

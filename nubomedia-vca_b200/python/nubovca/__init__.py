@@ -153,6 +153,8 @@ _SIGS = {
     "nv_face_submit_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(FaceParams)]),
     "nv_face_collect_batch": (_i, [_vp, _vp, _i, _ip, _ip]),
     "nv_face_detect_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(FaceParams), _vp, _i, _ip, _ip]),
+    "nv_face_submit_batch_yuv": (_i, [_vp, _vp, C.POINTER(YuvFrame), _i, C.POINTER(FaceParams)]),
+    "nv_face_detect_batch_yuv": (_i, [_vp, _vp, C.POINTER(YuvFrame), _i, C.POINTER(FaceParams), _vp, _i, _ip, _ip]),
 }
 BATCH_MAX = 256           # NV_BATCH_MAX
 EXPORTS = sorted(_SIGS)
@@ -225,6 +227,58 @@ def _batch_frames(images, cn):
     base, s0 = images.ctypes.data, strides[0]
     ptrs = (C.c_void_p * max(n, 1))(*range(base, base + n * s0, s0)) if s0 else (C.c_void_p * max(n, 1))(*([base] * n))
     return ptrs, n, w, h, strides[1], 0, images
+
+
+def _batch_yuv_frames(frames, fmt):
+    """(nv_yuv_frame array, n, keep-alive) of a 4:2:0 batch: a uint8 numpy array or CUDA torch tensor [N, H*3/2, W], each
+    image one packed 4:2:0 buffer as cv2.cvtColor(.., COLOR_YUV2BGR_<fmt>) reads it.  NV12 / NV21 rows may be further apart
+    than W bytes (a decoder's pitched surface: the chroma rows follow the luma rows at the same pitch); I420 / YV12 need
+    packed rows.  YV12's chroma planes are passed in I420 order.  A torch tensor's stream is synchronised here."""
+    if fmt not in _FMT:
+        raise ValueError(f"format must be one of {sorted(_FMT)}, got {fmt!r}")
+    dev = 0
+    if type(frames).__module__.startswith("torch"):
+        import torch
+        if frames.dtype != torch.uint8:
+            raise TypeError(f"batch must be a uint8 tensor, got {frames.dtype}")
+        if frames.dim() != 3:
+            raise ValueError(f"4:2:0 batch tensor must be [N, H*3/2, W], got {tuple(frames.shape)}")
+        if frames.is_cuda:
+            if frames.stride(2) != 1:
+                raise ValueError("the bytes of a row must be packed (stride(2) == 1)")
+            torch.cuda.current_stream(frames.device).synchronize()
+            base, s0, rs, dev = frames.data_ptr(), frames.stride(0), frames.stride(1), 1
+        else:
+            frames = frames.numpy()
+    if not dev:
+        if not isinstance(frames, np.ndarray) or frames.dtype != np.uint8:
+            raise TypeError("batch must be a uint8 numpy array or a CUDA torch tensor")
+        if frames.ndim != 3:
+            raise ValueError(f"4:2:0 batch array must be [N, H*3/2, W], got {frames.shape}")
+        if frames.strides[2] != 1 or min(frames.strides) < 0:
+            frames = np.ascontiguousarray(frames)
+        base, (s0, rs, _) = frames.ctypes.data, frames.strides
+    n, h3, w = frames.shape
+    if h3 % 3:
+        raise ValueError(f"a 4:2:0 buffer has H*3/2 rows for an even H, got {h3}")
+    h = h3 // 3 * 2
+    planar = _FMT[fmt] == FMT_I420
+    if planar and rs != w:
+        raise ValueError(f"I420 / YV12 buffers need packed rows (row stride {rs} != width {w})")
+    out = (YuvFrame * max(n, 1))()
+    for i in range(n):
+        f, b = out[i], base + i * s0
+        f.format, f.width, f.height, f.on_device = _FMT[fmt], w, h, dev
+        f.plane[0], f.stride[0] = b, rs
+        if planar:
+            u, v = b + w * h, b + w * h + (w // 2) * (h // 2)
+            if fmt == "YV12":
+                u, v = v, u
+            f.plane[1], f.plane[2] = u, v
+            f.stride[1] = f.stride[2] = w // 2
+        else:
+            f.plane[1], f.stride[1] = b + h * rs, rs
+    return out, n, frames
 
 
 NUM_STAGES = 8
@@ -574,6 +628,20 @@ class Context:
 
     def face_detect_batch(self, casc: Cascade, frames, width_to_process=160, scale_factor=1.25, min_neighbors=3, min_size=None):
         self.face_submit_batch(casc, frames, width_to_process, scale_factor, min_neighbors, min_size)
+        return self.face_collect_batch()
+
+    # frames: [N, H*3/2, W] packed 4:2:0 buffers (see _batch_yuv_frames); collected with face_collect_batch
+    def face_submit_batch_yuv(self, casc: Cascade, frames, fmt="NV12", width_to_process=160, scale_factor=1.25, min_neighbors=3,
+                              min_size=None):
+        table, n, keep = _batch_yuv_frames(frames, fmt)
+        p = self._face_params(width_to_process, scale_factor, min_neighbors, min_size)
+        self._batch_buffers(n)
+        _check(_lib.nv_face_submit_batch_yuv(self.handle, casc.handle, table, n, C.byref(p)), "nv_face_submit_batch_yuv")
+        self._batch_keep, self._batch_n = keep, n          # page-locked / device frames are read until collect
+
+    def face_detect_batch_yuv(self, casc: Cascade, frames, fmt="NV12", width_to_process=160, scale_factor=1.25, min_neighbors=3,
+                              min_size=None):
+        self.face_submit_batch_yuv(casc, frames, fmt, width_to_process, scale_factor, min_neighbors, min_size)
         return self.face_collect_batch()
 
     # ---- 4:2:0 ingest: planes = (y, u, v) for I420 (YV12: pass the planes in I420 meaning), (y, uv) for NV12 / NV21;

@@ -6,10 +6,14 @@ Variants, each over N frames per step:
   batch_device   nv_face_detect_batch on a CUDA uint8 tensor [N, 480, 640, 3]
   loop_blocking  N blocking nv_face_detect calls on page-locked frames, one context
   inflight_pinned / inflight_device  N contexts: N face_submit / face_submit_device, then N face_collect, one thread
+With --yuv, the same frames as NV12 (synth.to_yuv420) also run as
+  batch_nv12_pinned    nv_face_detect_batch_yuv on page-locked host frames [N, 720, 640]
+  batch_nv12_device    nv_face_detect_batch_yuv on a CUDA uint8 tensor [N, 720, 640]
+  inflight_nv12_pinned N contexts: N face_submit_yuv on page-locked frames, then N face_collect, one thread
 The variants alternate within every round (the host is shared); frames/s is the median over the rounds.  The card's name
 and power limit are read in the same run and printed with the table.
 
-    python tools/batch_throughput.py [--sizes 1,8,32,128] [--rounds 7] [--seconds 0.3] [--out FILE.json]
+    python tools/batch_throughput.py [--sizes 1,8,32,128] [--rounds 7] [--seconds 0.3] [--yuv] [--out FILE.json]
 """
 import argparse
 import ctypes as C
@@ -62,6 +66,7 @@ def main():
     ap.add_argument("--sizes", default="1,8,32,128")
     ap.add_argument("--rounds", type=int, default=7)
     ap.add_argument("--seconds", type=float, default=0.3)
+    ap.add_argument("--yuv", action="store_true", help="add the NV12 variants")
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
     import torch
@@ -74,6 +79,11 @@ def main():
     for i in range(nmax):
         host[i] = synth.frame(W, H, 1 + i % 4, 2000 + i)
     dev = torch.from_numpy(np.ascontiguousarray(host)).cuda()
+    if a.yuv:
+        yhost, yptr = pinned((nmax, H * 3 // 2, W))
+        for i in range(nmax):
+            yhost[i] = synth.to_yuv420(host[i], "NV12")
+        ydev = torch.from_numpy(np.ascontiguousarray(yhost)).cuda()
     torch.cuda.synchronize()
     bctx = nv.Context(0, W, H)
     sctx = nv.Context(0, W, H)
@@ -110,6 +120,26 @@ def main():
 
         variants = dict(batch_pinned=batch_pinned, batch_device=batch_device, loop_blocking=loop_blocking,
                         inflight_pinned=inflight_pinned, inflight_device=inflight_device)
+        if a.yuv:
+            yb, ydb = yhost[:n], ydev[:n]
+            planes = [synth.yuv420_planes(yb[i], W, H, "NV12") for i in range(n)]
+            yref = bctx.face_detect_batch_yuv(casc, yb, "NV12")
+            assert all((r == sctx.face_detect_yuv(casc, planes[i], "NV12")).all() for i, r in enumerate(yref))
+
+            def batch_nv12_pinned():
+                bctx.face_detect_batch_yuv(casc, yb, "NV12")
+
+            def batch_nv12_device():
+                bctx.face_detect_batch_yuv(casc, ydb, "NV12")
+
+            def inflight_nv12_pinned():
+                for i in range(n):
+                    ctxs[i].face_submit_yuv(casc, planes[i], "NV12")
+                for i in range(n):
+                    ctxs[i].face_collect()
+
+            variants.update(batch_nv12_pinned=batch_nv12_pinned, batch_nv12_device=batch_nv12_device,
+                            inflight_nv12_pinned=inflight_nv12_pinned)
         res = {k: [] for k in variants}
         for _ in range(a.rounds):
             for k, f in variants.items():
@@ -123,6 +153,8 @@ def main():
     for c in ctxs + [bctx, sctx]:
         c.close()
     nv._lib.nv_host_free(hptr)
+    if a.yuv:
+        nv._lib.nv_host_free(yptr)
 
 
 if __name__ == "__main__":
