@@ -244,6 +244,34 @@ NV_API int nv_tracker_reset(nv_ctx *ctx);
  * cvtColor(COLOR_YUV2BGR_*) per pixel, i.e. the result equals nv_tracker_process on the converted frame. */
 NV_API int nv_tracker_process_yuv(nv_ctx *ctx, const nv_yuv_frame *frame, double timestamp_ms, const nv_tracker_params *p,
                                   nv_rect *out, int cap, int *n);
+/* Batched tracker: many video streams on one context, one kernel launch and one synchronise per call.  The context keeps up
+ * to NV_BATCH_MAX stream slots, each with its own tracker state; frame i of a call is the next frame of slot i, with
+ * timestamps_ms[i] and params[i] (streams may differ in threshold, areas and distance).  Slot i's rectangles are exactly
+ * those nv_tracker_process / nv_tracker_process_yuv give on a separate context fed slot i's frames, timestamps and
+ * parameters.
+ *   Frames: BGRA, height rows of stride_bytes (a multiple of 4), or 4:2:0 frames that all share format, size, plane strides
+ *   and on_device (else NV_ERR_ARG naming the first frame that differs); each frame passes the single call's checks.
+ *   Pageable, page-locked (read in place by the copy engine) or, with on_device, device memory (read in place, no copy;
+ *   a CUDA uint8 tensor [N, H, W, 4]: data_ptr() + i * stride(0), at any byte address).
+ *   Output as in nv_face_detect_batch: out holds image 0's rectangles, then image 1's, ...; counts[i] is always image i's
+ *   count after __join_objects, *total (if given) the number written; more than cap in all: the first cap are written and
+ *   the call returns NV_ERR_CAPACITY.  An image with more than 16384 raw motion components gets the single call's truncated
+ *   result and the call returns NV_ERR_CAPACITY naming it, after every image has been written.
+ *   More than 255 distinct timestamps inside a slot's 0.2 ms motion-history window: NV_ERR_CAPACITY naming the slot, checked
+ *   for every slot before anything runs, so no slot changes.  Refused with NV_ERR_ARG: n outside 1 .. NV_BATCH_MAX, a null
+ *   table, timestamps, params or counts (out may be null with cap 0); a frame larger than the context: NV_ERR_CAPACITY, as
+ *   in the single call.
+ *   Slots: a slot's first frame after creation, reset or reconfiguration only primes it (0 rectangles).  The slots grow to the
+ *   largest n seen; a call with a smaller n leaves the higher slots as they are, to continue later.  All slots share one
+ *   frame size: a call at another size starts every slot afresh.  The slots share nothing with nv_tracker_process, and a
+ *   tracker batch leaves a pending nv_face_submit* / nv_face_submit_batch* as it is.  With profiling on,
+ *   nv_ctx_get_tracker_kernel_ms reports the batched kernel of the last call.  Blocking, like nv_tracker_process. */
+NV_API int nv_tracker_process_batch(nv_ctx *ctx, const uint8_t *const *frames, int n, int width, int height, int stride_bytes,
+                                    int on_device, const double *timestamps_ms, const nv_tracker_params *params, nv_rect *out,
+                                    int cap, int *counts, int *total);
+NV_API int nv_tracker_process_batch_yuv(nv_ctx *ctx, const nv_yuv_frame *frames, int n, const double *timestamps_ms,
+                                        const nv_tracker_params *params, nv_rect *out, int cap, int *counts, int *total);
+NV_API int nv_tracker_reset_batch(nv_ctx *ctx, int slot);   /* clears one slot; slot < 0: every slot */
 
 /* ---- image ops used by the nested elements (eye/mouth/nose/ear) on host images:
  *      cvtColor BGR2GRAY (kmseyedetect.cpp:949), equalizeHist (:950,964), cv::resize INTER_LINEAR

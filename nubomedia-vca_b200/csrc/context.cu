@@ -308,6 +308,7 @@ extern "C" int nv_ctx_create(int gpu, int max_width, int max_height, nv_ctx **ou
 }
 
 static void batch_free(nv_ctx::Batch &b);
+static void trk_batch_free(nv_ctx::TrkBatch &t);
 
 extern "C" void nv_ctx_destroy(nv_ctx *c)
 {
@@ -333,6 +334,7 @@ extern "C" void nv_ctx_destroy(nv_ctx *c)
     c->face_graph.drop();
     c->batch_graph.drop();
     batch_free(c->b);
+    trk_batch_free(c->tb);
     if (c->ev_done) cudaEventDestroy(c->ev_done);
     for (int i = 0; i < 2; i++) { if (c->ev_fork[i]) cudaEventDestroy(c->ev_fork[i]); if (c->ev_join[i]) cudaEventDestroy(c->ev_join[i]); }
     if (c->stream2) cudaStreamDestroy(c->stream2);
@@ -1506,12 +1508,10 @@ static std::vector<FaceSrc> batch_sources(const uint8_t *const *frames, int n, i
     return v;
 }
 
-// 4:2:0 frames: every frame passes check_yuv, and all share format, size, plane strides and on_device
-static int batch_check_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n, const nv_face_params *p,
-                           std::vector<FaceSrc> *srcs)
+// 4:2:0 frames of a batch (n checked by the caller): every frame passes check_yuv, and all share format, size, plane strides
+// and on_device
+static int batch_yuv_sources(nv_ctx *ctx, const nv_yuv_frame *frames, int n, std::vector<FaceSrc> *srcs)
 {
-    if (!ctx || !c || !frames || !p) { nv_set_error("null argument"); return NV_ERR_ARG; }
-    if (n < 1 || n > NV_BATCH_MAX) { nv_set_error("batch of %d images: 1 .. %d are supported", n, NV_BATCH_MAX); return NV_ERR_ARG; }
     srcs->resize(n);
     const nv_yuv_frame &f0 = frames[0];
     for (int i = 0; i < n; i++) {
@@ -1528,6 +1528,16 @@ static int batch_check_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame 
             return rc;
         }
     }
+    return NV_OK;
+}
+
+static int batch_check_yuv(nv_ctx *ctx, const nv_cascade *c, const nv_yuv_frame *frames, int n, const nv_face_params *p,
+                           std::vector<FaceSrc> *srcs)
+{
+    if (!ctx || !c || !frames || !p) { nv_set_error("null argument"); return NV_ERR_ARG; }
+    if (n < 1 || n > NV_BATCH_MAX) { nv_set_error("batch of %d images: 1 .. %d are supported", n, NV_BATCH_MAX); return NV_ERR_ARG; }
+    int rc = batch_yuv_sources(ctx, frames, n, srcs);
+    if (rc != NV_OK) return rc;
     if (ctx->scores) { nv_set_error("batch calls do not compute scores: switch them off with nv_ctx_set_scores(ctx, 0)"); return NV_ERR_STATE; }
     return NV_OK;
 }
@@ -1896,6 +1906,25 @@ extern "C" int nv_tracker_reset(nv_ctx *ctx)
     return NV_OK;
 }
 
+// The motion history is stored as an index into the table of live timestamps (kernels_tracker.cu).  updateMotionHistory:
+// a silhouette pixel takes ts, any other pixel whose value is below ts - MHI_DURATION (0.2, :28) drops to 0 — so an entry
+// whose value is below `del` dies in this frame; equal float values share an entry.  live: a stream's table before this frame;
+// val: after it; *cur: the index of ts (0 on a stream's first frame, which only primes it).
+static int trk_timestamps(const float *live, bool first, double timestamp_ms, float val[256], int *cur)
+{
+    const float ts = (float)timestamp_ms, del = (float)(timestamp_ms - 0.2);
+    val[0] = 0.f;
+    for (int k = 1; k < 256; k++) val[k] = (live[k] != 0.f && !(live[k] < del)) ? live[k] : 0.f;
+    *cur = 0;
+    if (!first && ts != 0.f) {                                     // ts == 0: silhouette pixels read as "no history", like every 0
+        for (int k = 1; k < 256 && !*cur; k++) if (val[k] == ts) *cur = k;
+        for (int k = 1; k < 256 && !*cur; k++) if (live[k] == 0.f) *cur = k;           // free BEFORE this frame: no pixel holds it
+        if (!*cur) { nv_set_error("more than 255 distinct timestamps inside the motion-history window"); return NV_ERR_CAPACITY; }
+        val[*cur] = ts;
+    }
+    return NV_OK;
+}
+
 // src.fmt == NV_FMT_BGR: interleaved BGRA in p[0] / s[0]; else the planes of a 4:2:0 frame (checked by the callers)
 static int tracker_impl(nv_ctx *ctx, const FaceSrc &src, int width, int height, double timestamp_ms, const nv_tracker_params *p,
                         nv_rect *out, int cap, int *n)
@@ -1930,21 +1959,9 @@ static int tracker_impl(nv_ctx *ctx, const FaceSrc &src, int width, int height, 
             planes.p0 = ctx->d_frame;
         }
     }
-    int first = ctx->trk_frames == 0, nl = 0;
-    // The motion history is stored as an index into the table of live timestamps (kernels_tracker.cu).  updateMotionHistory:
-    // a silhouette pixel takes ts, any other pixel whose value is below ts - MHI_DURATION (0.2, :28) drops to 0 — so an
-    // entry whose value is below `del` dies in this frame; equal float values share an entry.
-    const float ts = (float)timestamp_ms, del = (float)(timestamp_ms - 0.2);
+    int first = ctx->trk_frames == 0, nl = 0, cur;
     float val[256];
-    val[0] = 0.f;
-    for (int k = 1; k < 256; k++) val[k] = (ctx->trk_val[k] != 0.f && !(ctx->trk_val[k] < del)) ? ctx->trk_val[k] : 0.f;
-    int cur = 0;
-    if (!first && ts != 0.f) {                                     // ts == 0: silhouette pixels read as "no history", like every 0
-        for (int k = 1; k < 256 && !cur; k++) if (val[k] == ts) cur = k;
-        for (int k = 1; k < 256 && !cur; k++) if (ctx->trk_val[k] == 0.f) cur = k;       // free BEFORE this frame: no pixel holds it
-        if (!cur) { nv_set_error("more than 255 distinct timestamps inside the motion-history window"); return NV_ERR_CAPACITY; }
-        val[cur] = ts;
-    }
+    if ((rc = trk_timestamps(ctx->trk_val, first, timestamp_ms, val, &cur)) != NV_OK) return rc;
     if (ctx->profile) prof_mark(ctx, 2);                           // with profiling on: events around the tracker kernel
     NV_CUDA(launch_tracker(ctx, src.fmt, planes, width, height, first, p->threshold, cur, val, &nl));
     if (ctx->profile) prof_mark(ctx, 3);
@@ -1992,6 +2009,223 @@ extern "C" int nv_tracker_process_yuv(nv_ctx *ctx, const nv_yuv_frame *f, double
     int rc = check_yuv(ctx, f, &src);
     if (rc != NV_OK) return rc;
     return tracker_impl(ctx, src, f->width, f->height, timestamp_ms, p, out, cap, n);
+}
+
+// ------------------------------------------------------------------------------------------------
+// batched tracker: N stream slots per call, one launch of k_trk_fused<FMT, true>
+// ------------------------------------------------------------------------------------------------
+static void trk_batch_free(nv_ctx::TrkBatch &t)
+{
+    cudaFree(t.d_prev); cudaFree(t.d_hist); cudaFree(t.d_scratch); cudaFreeHost(t.h_out); cudaFree(t.d_frame); cudaFreeHost(t.h_stage);
+    cudaFree(t.d_tab); cudaFreeHost(t.h_tab);
+    t = nv_ctx::TrkBatch();
+}
+
+// slot state for n slots of w x h frames (grow-only; existing slots keep their state).  Another frame size starts every slot
+// afresh (gstnubotracker.cpp:202-237).
+static int trk_batch_slots(nv_ctx *ctx, int n, int w, int h)
+{
+    nv_ctx::TrkBatch &t = ctx->tb;
+    if (t.w == w && t.h == h && n <= t.cap) return NV_OK;
+    NV_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (t.w != w || t.h != h) {
+        trk_batch_free(t);
+        t.w = w; t.h = h;
+        t.slot_bytes = ((size_t)w * h + 16 + 255) & ~(size_t)255;
+        t.scratch_bytes = tracker_scratch_bytes(w, h, &t.lo);          // a multiple of 256
+    }
+    const int old = t.cap;
+    uint8_t *prev = nullptr, *hist = nullptr, *scratch = nullptr, *hout = nullptr;
+    TrkBatchImage *d_tab = nullptr, *h_tab = nullptr;
+    const int rc = [&]() -> int {
+        NV_CUDA(cudaMalloc(&prev, (size_t)n * t.slot_bytes));
+        NV_CUDA(cudaMalloc(&hist, (size_t)n * t.slot_bytes));
+        NV_CUDA(cudaMalloc(&scratch, (size_t)n * t.scratch_bytes));
+        NV_CUDA(cudaMallocHost(&hout, (size_t)n * (1 + 1024) * sizeof(int4)));
+        NV_CUDA(cudaMalloc(&d_tab, (size_t)n * sizeof(TrkBatchImage)));
+        NV_CUDA(cudaMallocHost(&h_tab, (size_t)n * sizeof(TrkBatchImage)));
+        // the old slots' images and histories move along; new slots start with no history, every slot's counters and edge
+        // flags at zero (the kernel leaves them so)
+        if (old) {
+            NV_CUDA(cudaMemcpyAsync(prev, t.d_prev, (size_t)old * t.slot_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+            NV_CUDA(cudaMemcpyAsync(hist, t.d_hist, (size_t)old * t.slot_bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+        }
+        NV_CUDA(cudaMemsetAsync(hist + (size_t)old * t.slot_bytes, 0, (size_t)(n - old) * t.slot_bytes, ctx->stream));
+        NV_CUDA(cudaMemset2DAsync(scratch + t.lo.zero_begin, t.scratch_bytes, 0, t.lo.zero_end - t.lo.zero_begin, n, ctx->stream));
+        NV_CUDA(cudaStreamSynchronize(ctx->stream));
+        return NV_OK;
+    }();
+    if (rc != NV_OK) {
+        cudaFree(prev); cudaFree(hist); cudaFree(scratch); cudaFreeHost(hout); cudaFree(d_tab); cudaFreeHost(h_tab);
+        return rc;
+    }
+    cudaFree(t.d_prev); cudaFree(t.d_hist); cudaFree(t.d_scratch); cudaFreeHost(t.h_out); cudaFree(t.d_tab); cudaFreeHost(t.h_tab);
+    t.d_prev = prev; t.d_hist = hist; t.d_scratch = scratch; t.h_out = hout; t.d_tab = d_tab; t.h_tab = h_tab;
+    t.cap = n;
+    t.val.resize(n, std::array<float, 256>{});
+    t.frames.resize(n, 0);
+    return NV_OK;
+}
+
+// srcs: n frames of one format, size and plane strides (checked by the callers); slot i takes frame i
+static int tracker_batch_impl(nv_ctx *ctx, const std::vector<FaceSrc> &srcs, int w, int h, const double *timestamps_ms,
+                              const nv_tracker_params *params, nv_rect *out, int cap, int *counts, int *total)
+{
+    const int n = (int)srcs.size();
+    nv_ctx::TrkBatch &t = ctx->tb;
+    NV_CUDA(cudaSetDevice(ctx->gpu));
+    if (ctx->pending) NV_CUDA(cudaStreamSynchronize(ctx->stream));
+    // the timestamp tables of every slot first: a slot that has no free history index refuses the call before anything changes
+    const bool same_size = t.w == w && t.h == h;
+    std::vector<TrkBatchImage> img(n);
+    static const std::array<float, 256> none = {};
+    for (int i = 0; i < n; i++) {
+        const bool kept = same_size && i < t.cap;
+        img[i].first = !kept || t.frames[i] == 0;
+        img[i].thr = params[i].threshold;
+        img[i].pad = 0;
+        if (trk_timestamps(kept ? t.val[i].data() : none.data(), img[i].first, timestamps_ms[i], img[i].val, &img[i].cur) != NV_OK) {
+            const std::string why = nv_last_error();
+            nv_set_error("slot %d: %s", i, why.c_str());
+            return NV_ERR_CAPACITY;
+        }
+    }
+    int rc = trk_batch_slots(ctx, n, w, h);
+    if (rc != NV_OK) return rc;
+    // host frames go whole into per-slot frame buffers, plane by plane, each plane rounded up to 256 bytes
+    const FaceSrc &f0 = srcs[0];
+    const int np = f0.fmt == NV_FMT_BGR ? 1 : 3, plane_h[3] = {h, h / 2, h / 2};
+    size_t off[4] = {0, 0, 0, 0};
+    for (int k = 0; k < np; k++) off[k + 1] = off[k] + (((size_t)f0.s[k] * plane_h[k] + 255) & ~(size_t)255);
+    std::vector<cudaMemoryType> types(f0.on_device ? 0 : (size_t)n * np, cudaMemoryTypeDevice);
+    bool pageable = false;
+    for (int i = 0; i < n && !f0.on_device; i++)
+        for (int k = 0; k < np; k++) {
+            if (!srcs[i].p[k]) continue;
+            types[i * np + k] = nv_memory_type(srcs[i].p[k]);
+            pageable = pageable || types[i * np + k] == cudaMemoryTypeUnregistered;
+        }
+    if (!f0.on_device && (n > t.frame_cap || off[np] > t.frame_bytes || (pageable && !t.h_stage))) {
+        NV_CUDA(cudaStreamSynchronize(ctx->stream));
+        const bool stage = pageable || t.h_stage;
+        cudaFree(t.d_frame); cudaFreeHost(t.h_stage);
+        t.d_frame = nullptr; t.h_stage = nullptr;
+        t.frame_cap = std::max(n, t.frame_cap); t.frame_bytes = std::max(off[np], t.frame_bytes);
+        const size_t bytes = (size_t)t.frame_cap * t.frame_bytes;
+        if (cudaMalloc(&t.d_frame, bytes) != cudaSuccess || (stage && cudaMallocHost(&t.h_stage, bytes) != cudaSuccess)) {
+            cudaGetLastError();
+            cudaFree(t.d_frame); cudaFreeHost(t.h_stage);
+            t.d_frame = nullptr; t.h_stage = nullptr; t.frame_cap = 0; t.frame_bytes = 0;
+            nv_set_error("out of memory for %d tracker frames", n);
+            return NV_ERR_CUDA;
+        }
+    }
+    std::vector<const uint8_t *> planes(3 * (size_t)n, nullptr);
+    for (int i = 0; i < n; i++)
+        for (int k = 0; k < np; k++) {
+            const uint8_t *d = srcs[i].p[k];
+            if (d && !f0.on_device) {
+                const size_t at = (size_t)i * t.frame_bytes + off[k];
+                if ((rc = upload_rows(ctx, t.d_frame + at, t.h_stage ? t.h_stage + at : nullptr, d, types[i * np + k], f0.s[k], plane_h[k],
+                                      0, 0, 0)) != NV_OK) return rc;
+                d = t.d_frame + at;
+            }
+            planes[3 * i + k] = d;
+        }
+    for (int i = 0; i < n; i++) {
+        for (int k = 0; k < 3; k++) img[i].p[k] = planes[3 * i + k];
+        t.h_tab[i] = img[i];
+    }
+    NV_CUDA(cudaMemcpyAsync(t.d_tab, t.h_tab, (size_t)n * sizeof(TrkBatchImage), cudaMemcpyHostToDevice, ctx->stream));
+    const SrcPlanes strides = {nullptr, nullptr, nullptr, f0.s[0], f0.s[1], f0.s[2]};
+    if (ctx->profile) prof_mark(ctx, 2);                           // the events nv_ctx_get_tracker_kernel_ms reads
+    NV_CUDA(launch_tracker_batch(f0.fmt, strides, t.d_tab, planes.data(), n, w, h, t.lo, t.d_prev, t.d_hist, t.slot_bytes, t.d_scratch,
+                                 t.scratch_bytes, t.h_out, ctx->stream));
+    if (ctx->profile) prof_mark(ctx, 3);
+    ctx->launches++;
+    for (int i = 0; i < n; i++) {
+        memcpy(t.val[i].data(), img[i].val, sizeof img[i].val);
+        t.frames[i] = img[i].first ? 1 : t.frames[i] + 1;
+    }
+    NV_CUDA(cudaStreamSynchronize(ctx->stream));
+    // per image: count and the first 1024 rectangles in its mapped block, any beyond from its scratch, then __join_objects
+    std::vector<nv_rect> all;
+    int over = -1;
+    std::vector<int4> more;
+    for (int i = 0; i < n; i++) {
+        counts[i] = 0;
+        if (img[i].first) continue;
+        const int4 *hb = reinterpret_cast<const int4 *>(t.h_out) + (size_t)i * (1 + 1024);
+        const int raw = hb[0].x, m = std::min(raw, TRK_MAX_COMPONENTS);
+        if (raw > TRK_MAX_COMPONENTS && over < 0) over = i;
+        std::vector<nv_rect> v(m);
+        for (int j = 0; j < std::min(m, 1024); j++) v[j] = nv_rect{hb[1 + j].x, hb[1 + j].y, hb[1 + j].z, hb[1 + j].w};
+        if (m > 1024) {
+            more.resize(m - 1024);
+            const int4 *d_out = reinterpret_cast<const int4 *>(t.d_scratch + (size_t)i * t.scratch_bytes + t.lo.out);
+            NV_CUDA(cudaMemcpy(more.data(), d_out + 1 + 1024, (size_t)(m - 1024) * sizeof(int4), cudaMemcpyDeviceToHost));
+            for (int j = 1024; j < m; j++) v[j] = nv_rect{more[j - 1024].x, more[j - 1024].y, more[j - 1024].z, more[j - 1024].w};
+        }
+        trk_join_objects(v, params[i].min_area, params[i].max_area, params[i].distance);
+        counts[i] = (int)v.size();
+        all.insert(all.end(), v.begin(), v.end());
+    }
+    const int sum = (int)all.size(), m = std::min(sum, std::max(cap, 0));
+    if (m > 0) memcpy(out, all.data(), (size_t)m * sizeof(nv_rect));
+    if (total) *total = m;
+    if (over >= 0) { nv_set_error("image %d: more than %d motion components", over, TRK_MAX_COMPONENTS); return NV_ERR_CAPACITY; }
+    if (sum > cap) { nv_set_error("%d rectangles, caller capacity %d", sum, cap); return NV_ERR_CAPACITY; }
+    return NV_OK;
+}
+
+static int trk_batch_check(nv_ctx *ctx, const void *frames, int n, const double *timestamps_ms, const nv_tracker_params *params,
+                           nv_rect *out, int cap, int *counts)
+{
+    if (!ctx || !frames || !timestamps_ms || !params || !counts || (cap > 0 && !out)) { nv_set_error("null argument"); return NV_ERR_ARG; }
+    if (n < 1 || n > NV_BATCH_MAX) { nv_set_error("batch of %d images: 1 .. %d are supported", n, NV_BATCH_MAX); return NV_ERR_ARG; }
+    return NV_OK;
+}
+
+extern "C" int nv_tracker_process_batch(nv_ctx *ctx, const uint8_t *const *frames, int n, int width, int height, int stride_bytes,
+                                        int on_device, const double *timestamps_ms, const nv_tracker_params *params, nv_rect *out,
+                                        int cap, int *counts, int *total)
+{
+    int rc = trk_batch_check(ctx, frames, n, timestamps_ms, params, out, cap, counts);
+    if (rc != NV_OK) return rc;
+    for (int i = 0; i < n; i++) {
+        if ((rc = check_frame(ctx, frames[i], width, height, stride_bytes, 4)) != NV_OK) {
+            const std::string why = nv_last_error();
+            nv_set_error("image %d: %s", i, why.c_str());
+            return rc;
+        }
+    }
+    if (stride_bytes % 4) { nv_set_error("BGRA stride must be a multiple of 4"); return NV_ERR_ARG; }
+    std::vector<FaceSrc> srcs(n);
+    for (int i = 0; i < n; i++) srcs[i] = FaceSrc{NV_FMT_BGR, {frames[i], nullptr, nullptr}, {stride_bytes, 0, 0}, on_device != 0};
+    return tracker_batch_impl(ctx, srcs, width, height, timestamps_ms, params, out, cap, counts, total);
+}
+
+extern "C" int nv_tracker_process_batch_yuv(nv_ctx *ctx, const nv_yuv_frame *frames, int n, const double *timestamps_ms,
+                                            const nv_tracker_params *params, nv_rect *out, int cap, int *counts, int *total)
+{
+    int rc = trk_batch_check(ctx, frames, n, timestamps_ms, params, out, cap, counts);
+    if (rc != NV_OK) return rc;
+    std::vector<FaceSrc> srcs;
+    if ((rc = batch_yuv_sources(ctx, frames, n, &srcs)) != NV_OK) return rc;
+    return tracker_batch_impl(ctx, srcs, frames[0].width, frames[0].height, timestamps_ms, params, out, cap, counts, total);
+}
+
+extern "C" int nv_tracker_reset_batch(nv_ctx *ctx, int slot)
+{
+    if (!ctx) { nv_set_error("null ctx"); return NV_ERR_ARG; }
+    if (slot >= NV_BATCH_MAX) { nv_set_error("slot %d: slots are 0 .. %d", slot, NV_BATCH_MAX - 1); return NV_ERR_ARG; }
+    nv_ctx::TrkBatch &t = ctx->tb;
+    const int a = slot < 0 ? 0 : slot, b = slot < 0 ? t.cap : std::min(slot + 1, t.cap);
+    if (a >= b) return NV_OK;                                      // a slot that does not exist yet starts afresh anyway
+    for (int i = a; i < b; i++) { t.frames[i] = 0; t.val[i].fill(0.f); }
+    NV_CUDA(cudaSetDevice(ctx->gpu));
+    NV_CUDA(cudaMemsetAsync(t.d_hist + (size_t)a * t.slot_bytes, 0, (size_t)(b - a) * t.slot_bytes, ctx->stream));
+    return NV_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <array>
 #include <map>
 #include <mutex>
 #include <string>
@@ -312,6 +313,10 @@ struct PlanSlot {
 // byte offsets of the tracker's per-tile scratch inside nv_ctx::d_trk_scratch (kernels_tracker.cu)
 struct TrkLayout { int ntx, nty; size_t bbox, rects, out, bseed, parent, slotlist, bcount, keys, bslot, counters, edge_flag, zero_begin, zero_end; };
 
+// one image of a batched tracker call, in the device table of the call: its planes (BGRA: p[0]; 4:2:0: Y, U|UV|VU, V), whether it
+// only primes its slot, its threshold, the history index of its timestamp, and the live timestamps after its expiry
+struct TrkBatchImage { const uint8_t *p[3]; int first, thr, cur, pad; float val[256]; };
+
 // Source frame of the face block: interleaved BGR (p[0], s[0]) or the planes of a 4:2:0 frame.
 struct FaceSrc { int fmt; const uint8_t *p[3]; int s[3]; bool on_device; };
 
@@ -435,6 +440,21 @@ struct nv_ctx {
     float trk_val[256] = {};
     int trk_w = 0, trk_h = 0;  long long trk_frames = 0;
     uint8_t *h_trk = nullptr;
+
+    // batched tracker (nv_tracker_process_batch*): stream slots, each with the state of one tracker above; shares nothing with
+    // the single tracker or the face batch.  Device buffers are grow-only and hold cap slots at the strides below.
+    struct TrkBatch {
+        int cap = 0, w = 0, h = 0;                          // slots the buffers hold; the frame size of every slot
+        TrkLayout lo = {};
+        size_t slot_bytes = 0, scratch_bytes = 0;           // per slot: prev / hist, scratch (tracker_scratch_bytes)
+        uint8_t *d_prev = nullptr, *d_hist = nullptr, *d_scratch = nullptr;
+        uint8_t *h_out = nullptr;                           // page-locked, mapped: per slot count + 1024 rectangles (int4)
+        std::vector<std::array<float, 256>> val;            // per slot: the live timestamps (trk_val of the single tracker)
+        std::vector<long long> frames;                      // per slot: frames since creation, reset or reconfiguration
+        int frame_cap = 0;  size_t frame_bytes = 0;         // uploaded host frames: frame_cap slots of frame_bytes
+        uint8_t *d_frame = nullptr, *h_stage = nullptr;     // h_stage: page-locked staging of pageable frames (on demand)
+        TrkBatchImage *d_tab = nullptr, *h_tab = nullptr;   // per call: cap entries
+    } tb;
 };
 
 // ----------------------------------------------------------------------------------------------
@@ -563,6 +583,12 @@ cudaError_t launch_group(const PlanDev *plan, int *counters, const uint32_t *can
 size_t tracker_scratch_bytes(int w, int h, TrkLayout *lo);
 cudaError_t launch_tracker(nv_ctx *ctx, int fmt, const SrcPlanes &src, int w, int h, int first, int thr, int cur, const float *val256,
                            int *nlaunch);
+// one launch for n images: image i's table entry at d_imgs[i] (h_planes: the host copy of the 3n plane pointers), its prev / hist
+// at i * slot_stride, its scratch (layout lo) at i * scratch_stride, its mapped result block (1 + 1024 int4) at hout + i blocks;
+// strides: the plane strides of every image
+cudaError_t launch_tracker_batch(int fmt, const SrcPlanes &strides, const TrkBatchImage *d_imgs, const uint8_t *const *h_planes, int n,
+                                 int w, int h, const TrkLayout &lo, uint8_t *prev, uint8_t *hist, size_t slot_stride, uint8_t *scratch,
+                                 size_t scratch_stride, void *hout, cudaStream_t st);
 
 // ----------------------------------------------------------------------------------------------
 // device helpers shared by the ingest kernels (kernels_prep.cu, kernels_tracker.cu): cvtColor(COLOR_YUV2BGR_*) per pixel

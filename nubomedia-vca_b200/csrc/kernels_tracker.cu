@@ -74,7 +74,31 @@ struct TrkParams {
     int4 *hout;                     // the context's page-locked copy of out[0 .. 1024] (mapped host memory): written by the last block,
                                     // so that no device-to-host copy follows the launch
     float val[256];                 // timestamp of history index k after this frame's expiry (0: none / expired)
+    // batched kernel (BATCH): image blockIdx.y.  The pointers above are image 0's; image i's prev / hist lie i * slot_stride
+    // bytes further, its scratch i * scratch_stride bytes further, its mapped block at hout + i * TRK_HOUT.  src's strides are
+    // every image's; its pointers, first, thr, cur and val come from imgs[i].
+    const TrkBatchImage *imgs;
+    size_t slot_stride, scratch_stride;
 };
+#define TRK_HOUT (1 + 1024)
+
+// p moved to image blockIdx.y of a batch, whose buffers lie `stride` bytes apart; p itself when BATCH is off
+template <bool BATCH, typename T>
+__device__ __forceinline__ T *trk_img(T *p, size_t stride)
+{
+    return BATCH ? reinterpret_cast<T *>(reinterpret_cast<uintptr_t>(p) + blockIdx.y * stride) : p;
+}
+#define TRK_SLOT(p) trk_img<BATCH>(p, P.slot_stride)             // this image's prev / hist
+#define TRK_SCR(p) trk_img<BATCH>(p, P.scratch_stride)           // this image's scratch
+#define TRK_RES(p) trk_img<BATCH>(p, TRK_HOUT * sizeof(int4))    // this image's mapped result block
+
+// the planes of image blockIdx.y of a batch, with the strides every image shares
+__device__ __forceinline__ SrcPlanes trk_planes(const TrkParams &P, const TrkBatchImage *I)
+{
+    const uint8_t *p[3];
+    for (int k = 0; k < 3; k++) p[k] = reinterpret_cast<const uint8_t *>(__ldg(reinterpret_cast<const unsigned long long *>(I->p + k)));
+    return SrcPlanes{p[0], p[1], p[2], P.src.s0, P.src.s1, P.src.s2};
+}
 
 __device__ __forceinline__ bool trk_joined(float a, float b)
 {
@@ -116,6 +140,7 @@ __device__ __forceinline__ int trk_perim_px(int k)
 // stitches the edge between tile a (left / upper) and tile b (right / lower); vertical != 0: b lies below a.  Runs on the
 // first two warps of the block (an edge is at most 64 pixels long); a pixel pair that repeats its left neighbour's
 // (slot, slot) pair is skipped: along a blob that leaves one union per edge instead of one per pixel.
+template <bool BATCH>
 __device__ void trk_stitch(const TrkParams &P, const float *s_val, int a, int b, int vertical)
 {
     if (threadIdx.x >= 64) return;
@@ -127,18 +152,21 @@ __device__ void trk_stitch(const TrkParams &P, const float *s_val, int a, int b,
     unsigned sa = 0xffffu, sb = 0xffffu;
     bool joined = false;
     if (i < len && xa < P.w && xb < P.w && ya < P.h && yb < P.h) {
-        sa = __ldcg(P.bslot + (size_t)a * TRK_PERIM + ka); sb = __ldcg(P.bslot + (size_t)b * TRK_PERIM + kb);
+        sa = __ldcg(TRK_SCR(P.bslot) + (size_t)a * TRK_PERIM + ka); sb = __ldcg(TRK_SCR(P.bslot) + (size_t)b * TRK_PERIM + kb);
         if (sa != 0xffffu && sb != 0xffffu)
-            joined = trk_joined(s_val[__ldcg(P.hist + (size_t)ya * P.w + xa)], s_val[__ldcg(P.hist + (size_t)yb * P.w + xb)]);
+            joined = trk_joined(s_val[__ldcg(TRK_SLOT(P.hist) + (size_t)ya * P.w + xa)], s_val[__ldcg(TRK_SLOT(P.hist) + (size_t)yb * P.w + xb)]);
     }
     const unsigned key = joined ? (sa << 16) | sb : 0xffffffffu, left = __shfl_up_sync(0xffffffffu, key, 1);
-    if (joined && (lane == 0 || left != key)) trk_union(P.parent, a * TRK_SLOTS + (int)sa, b * TRK_SLOTS + (int)sb);
+    if (joined && (lane == 0 || left != key)) trk_union(TRK_SCR(P.parent), a * TRK_SLOTS + (int)sa, b * TRK_SLOTS + (int)sb);
 }
 
 // FMT 0: BGRA (the reference's caps, gstnubotracker.cpp:57-61); 1 / 2 / 3: I420 / NV12 / NV21 planes — the 4:2:0 ingest
 // extension: gray = BGR2GRAY(cvtColor(COLOR_YUV2BGR_*)) per pixel, the BGRA frame is never built.
-template <int FMT>
-__global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkParams P)
+// BATCH: image blockIdx.y of a batch (one tracker stream slot each), tile blockIdx.x.  Every image has its own planes, state,
+// scratch, counters and result block; no block reads or waits for anything of another image.
+// The batched instantiations ask for five blocks per SM: left to itself, ptxas holds them at 40 registers and spills.
+template <int FMT, bool BATCH>
+__global__ void __launch_bounds__(256, BATCH ? 5 : 0) k_trk_fused(const __grid_constant__ TrkParams P)
 {
     __shared__ float s_val[256];
     __shared__ union { float m[TRK_NPX]; int minx[TRK_NPX]; } s_a;          // history values, then (labels final) min x per root
@@ -148,8 +176,12 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
     const int tid = threadIdx.x, lane = tid & 31;
     const int tile = blockIdx.x, tx = tile % P.ntx, ty = tile / P.ntx;
     const int x0 = tx * TRK_TW, y0 = ty * TRK_TH;
+    // BATCH: this image's entry of the call's table, read where it is used (kept in registers, it made the kernel spill)
+    const TrkBatchImage *const I = BATCH ? P.imgs + blockIdx.y : nullptr;
+#define TRK_IMG(f) (BATCH ? __ldg(&I->f) : P.f)
+#define TRK_SRC (BATCH ? trk_planes(P, I) : P.src)
     TRK_T(0);
-    s_val[tid] = P.val[tid];
+    s_val[tid] = BATCH ? I->val[tid] : P.val[tid];
     if (tid == 0) s_nslots = 0;
     __syncthreads();
     TRK_T(1);
@@ -167,28 +199,31 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
         const bool row_ok = y < P.h;
         const bool full = row_ok && x + 3 < P.w;
         if (FMT == 0 && P.vec && full) {
-            const uint4 px = *reinterpret_cast<const uint4 *>(P.src.p0 + (size_t)y * P.src.s0 + 4 * x);
+            const uint4 px = *reinterpret_cast<const uint4 *>(TRK_SRC.p0 + (size_t)y * P.src.s0 + 4 * x);
             const unsigned w4[4] = {px.x, px.y, px.z, px.w};
 #pragma unroll
             for (int k = 0; k < 4; k++) g[k] = trk_gray(w4[k] & 255, (w4[k] >> 8) & 255, (w4[k] >> 16) & 255);
-            const unsigned p4 = *reinterpret_cast<const unsigned *>(P.prev + (size_t)y * P.w + x);
-            const unsigned h4 = P.first ? 0u : *reinterpret_cast<const unsigned *>(P.hist + (size_t)y * P.w + x);
+            const unsigned p4 = *reinterpret_cast<const unsigned *>(TRK_SLOT(P.prev) + (size_t)y * P.w + x);
+            const unsigned h4 = TRK_IMG(first) ? 0u : *reinterpret_cast<const unsigned *>(TRK_SLOT(P.hist) + (size_t)y * P.w + x);
 #pragma unroll
             for (int k = 0; k < 4; k++) { pv[k] = (p4 >> (8 * k)) & 255; hv[k] = (h4 >> (8 * k)) & 255; }
         } else if (row_ok) {
 #pragma unroll
             for (int k = 0; k < 4; k++) {
                 if (x + k >= P.w) break;
-                if (FMT == 0) {
-                    const uchar4 px = *reinterpret_cast<const uchar4 *>(P.src.p0 + (size_t)y * P.src.s0 + 4 * (x + k));
+                if (FMT == 0 && BATCH) {                                  // a caller's device frame may lie at any byte
+                    const uint8_t *px = TRK_SRC.p0 + (size_t)y * P.src.s0 + 4 * (x + k);
+                    g[k] = trk_gray(px[0], px[1], px[2]);
+                } else if (FMT == 0) {
+                    const uchar4 px = *reinterpret_cast<const uchar4 *>(TRK_SRC.p0 + (size_t)y * P.src.s0 + 4 * (x + k));
                     g[k] = trk_gray(px.x, px.y, px.z);
                 } else {
                     int c3[3];
-                    yuv_pixel(P.src, yuv_chroma<FMT == 0 ? 1 : FMT>(P.src, x + k, y), x + k, y, c3);
+                    yuv_pixel(TRK_SRC, yuv_chroma<FMT == 0 ? 1 : FMT>(TRK_SRC, x + k, y), x + k, y, c3);
                     g[k] = trk_gray(c3[0], c3[1], c3[2]);
                 }
-                pv[k] = P.prev[(size_t)y * P.w + x + k];
-                hv[k] = P.first ? 0u : P.hist[(size_t)y * P.w + x + k];
+                pv[k] = TRK_SLOT(P.prev)[(size_t)y * P.w + x + k];
+                hv[k] = TRK_IMG(first) ? 0u : TRK_SLOT(P.hist)[(size_t)y * P.w + x + k];
             }
         }
         unsigned nh[4];
@@ -196,20 +231,20 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const bool in = row_ok && x + k < P.w;
-            const bool silh = abs(g[k] - pv[k]) > P.thr;                                  // absdiff + threshold(.., BINARY)
-            nh[k] = !in ? 0u : silh ? (unsigned)P.cur : (s_val[hv[k]] != 0.f ? hv[k] : 0u);   // updateMotionHistory
+            const bool silh = abs(g[k] - pv[k]) > TRK_IMG(thr);                                  // absdiff + threshold(.., BINARY)
+            nh[k] = !in ? 0u : silh ? (unsigned)TRK_IMG(cur) : (s_val[hv[k]] != 0.f ? hv[k] : 0u);   // updateMotionHistory
             m[k] = s_val[nh[k]];
             // history index P.cur <=> mhi == ts (equal float values share an index; value 0: no seeds at all)
-            if (in && nh[k] == (unsigned)P.cur && m[k] != 0.f) seedbits[half] |= 1u << k;
+            if (in && nh[k] == (unsigned)TRK_IMG(cur) && m[k] != 0.f) seedbits[half] |= 1u << k;
         }
         if (row_ok) {
             if (P.vec && full) {
-                *reinterpret_cast<unsigned *>(P.prev + (size_t)y * P.w + x) = (unsigned)g[0] | ((unsigned)g[1] << 8) | ((unsigned)g[2] << 16) | ((unsigned)g[3] << 24);
-                if (!P.first) *reinterpret_cast<unsigned *>(P.hist + (size_t)y * P.w + x) = nh[0] | (nh[1] << 8) | (nh[2] << 16) | (nh[3] << 24);
+                *reinterpret_cast<unsigned *>(TRK_SLOT(P.prev) + (size_t)y * P.w + x) = (unsigned)g[0] | ((unsigned)g[1] << 8) | ((unsigned)g[2] << 16) | ((unsigned)g[3] << 24);
+                if (!TRK_IMG(first)) *reinterpret_cast<unsigned *>(TRK_SLOT(P.hist) + (size_t)y * P.w + x) = nh[0] | (nh[1] << 8) | (nh[2] << 16) | (nh[3] << 24);
             } else {
                 for (int k = 0; k < 4 && x + k < P.w; k++) {
-                    P.prev[(size_t)y * P.w + x + k] = (uint8_t)g[k];
-                    if (!P.first) P.hist[(size_t)y * P.w + x + k] = (uint8_t)nh[k];
+                    TRK_SLOT(P.prev)[(size_t)y * P.w + x + k] = (uint8_t)g[k];
+                    if (!TRK_IMG(first)) TRK_SLOT(P.hist)[(size_t)y * P.w + x + k] = (uint8_t)nh[k];
                 }
             }
         }
@@ -223,7 +258,7 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
             s_lab[li + k] = lab;
         }
     }
-    if (P.first) return;                                           // the first frame only primes img_prev (:360)
+    if (TRK_IMG(first)) return;                                           // the first frame only primes img_prev (:360)
     // a tile without any history (most of a frame, most of the time) has nothing to label: it only publishes an empty
     // perimeter and takes part in the edge and completion protocol
     const bool empty = !__syncthreads_or(mine);
@@ -346,7 +381,7 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
     TRK_T(5);
 
     // ---- 4. roots: final inside the tile, or a slot of the perimeter table ------------------------------------------------
-    int *const parent = P.parent + (size_t)tile * TRK_SLOTS;
+    int *const parent = TRK_SCR(P.parent) + (size_t)tile * TRK_SLOTS;
 #pragma unroll
     for (int half = 0; half < TRK_NH; half++) {
         const int ly = (tid >> 4) + half * 16, li = ly * TRK_TW + ux;
@@ -359,13 +394,13 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
             const bool edge = mnx == 0 || mxx == TRK_TW - 1 || ly == 0 || mxy == TRK_TH - 1;      // a root is its component's first row
             if (edge) {
                 const int s = atomicAdd(&s_nslots, 1);
-                P.bbox[(size_t)tile * TRK_SLOTS + s] = make_int4(x0 + mnx, y0 + ly, x0 + mxx, y0 + mxy);
-                P.bseed[(size_t)tile * TRK_SLOTS + s] = gseed;
+                TRK_SCR(P.bbox)[(size_t)tile * TRK_SLOTS + s] = make_int4(x0 + mnx, y0 + ly, x0 + mxx, y0 + mxy);
+                TRK_SCR(P.bseed)[(size_t)tile * TRK_SLOTS + s] = gseed;
                 parent[s] = tile * TRK_SLOTS + s;
                 s_maxx[i] = s;                                     // slot of this root, read back below
             } else if (gseed != TRK_NONE) {
-                const int pos = atomicAdd(&P.counters[0], 1);
-                if (pos < TRK_MAX_COMPONENTS) { P.keys[pos] = gseed; P.rects[pos] = make_int4(x0 + mnx, y0 + ly, mxx - mnx + 1, mxy - ly + 1); }
+                const int pos = atomicAdd(&TRK_SCR(P.counters)[0], 1);
+                if (pos < TRK_MAX_COMPONENTS) { TRK_SCR(P.keys)[pos] = gseed; TRK_SCR(P.rects)[pos] = make_int4(x0 + mnx, y0 + ly, mxx - mnx + 1, mxy - ly + 1); }
             }
         }
     }
@@ -373,11 +408,11 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
     } else { TRK_T(3); TRK_T(4); TRK_T(5); }
     if (tid < TRK_PERIM) {
         const int r = s_lab[trk_perim_px(tid)];
-        P.bslot[(size_t)tile * TRK_PERIM + tid] = r == TRK_NONE ? (unsigned short)0xffff : (unsigned short)s_maxx[r];
+        TRK_SCR(P.bslot)[(size_t)tile * TRK_PERIM + tid] = r == TRK_NONE ? (unsigned short)0xffff : (unsigned short)s_maxx[r];
     }
-    if (tid == 0) { P.bcount[tile] = s_nslots; s_base = s_nslots ? atomicAdd(&P.counters[2], s_nslots) : 0; }
+    if (tid == 0) { TRK_SCR(P.bcount)[tile] = s_nslots; s_base = s_nslots ? atomicAdd(&TRK_SCR(P.counters)[2], s_nslots) : 0; }
     __syncthreads();
-    for (int s2 = tid; s2 < s_nslots; s2 += blockDim.x) P.slotlist[s_base + s2] = tile * TRK_SLOTS + s2;     // for the last block
+    for (int s2 = tid; s2 < s_nslots; s2 += blockDim.x) TRK_SCR(P.slotlist)[s_base + s2] = tile * TRK_SLOTS + s2;     // for the last block
     __threadfence();
     __syncthreads();
 
@@ -390,23 +425,23 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
         if (tid == 1 && tx > 0) e = ty * (P.ntx - 1) + tx - 1;                            // left
         if (tid == 2 && ty + 1 < P.nty) e = nh_edges + ty * P.ntx + tx;                   // below
         if (tid == 3 && ty > 0) e = nh_edges + (ty - 1) * P.ntx + tx;                     // above
-        const bool second = e >= 0 && atomicAdd(&P.edge_flag[e], 1) == 1;
-        if (second) P.edge_flag[e] = 0;                            // both tiles have been here: re-armed for the next frame
+        const bool second = e >= 0 && atomicAdd(&TRK_SCR(P.edge_flag)[e], 1) == 1;
+        if (second) TRK_SCR(P.edge_flag)[e] = 0;                            // both tiles have been here: re-armed for the next frame
         s_edges[tid] = second ? 1 : 0;
     }
     __syncthreads();
     TRK_T(7);
     if (s_edges[0] || s_edges[1] || s_edges[2] || s_edges[3]) {
         __threadfence();                                           // the other tile published before it arrived at the edge
-        if (s_edges[0]) trk_stitch(P, s_val, tile, tile + 1, 0);
-        if (s_edges[1]) trk_stitch(P, s_val, tile - 1, tile, 0);
-        if (s_edges[2]) trk_stitch(P, s_val, tile, tile + P.ntx, 1);
-        if (s_edges[3]) trk_stitch(P, s_val, tile - P.ntx, tile, 1);
+        if (s_edges[0]) trk_stitch<BATCH>(P, s_val, tile, tile + 1, 0);
+        if (s_edges[1]) trk_stitch<BATCH>(P, s_val, tile - 1, tile, 0);
+        if (s_edges[2]) trk_stitch<BATCH>(P, s_val, tile, tile + P.ntx, 1);
+        if (s_edges[3]) trk_stitch<BATCH>(P, s_val, tile - P.ntx, tile, 1);
         __threadfence();
     }
     __syncthreads();
     TRK_T(8);
-    if (tid == 0) s_last = atomicAdd(&P.counters[1], 1) == P.ntx * P.nty - 1;
+    if (tid == 0) s_last = atomicAdd(&TRK_SCR(P.counters)[1], 1) == P.ntx * P.nty - 1;
     __syncthreads();
     TRK_T(9);
     if (!s_last) return;
@@ -415,52 +450,54 @@ __global__ void __launch_bounds__(256) k_trk_fused(const __grid_constant__ TrkPa
     // one block from here on: __syncthreads() orders its own global accesses, the fence below is the acquire side of the
     // other blocks' releases
     __threadfence();
-    const int nused = ((volatile int *)P.counters)[2];
+    const int nused = ((volatile int *)TRK_SCR(P.counters))[2];
     for (int i = tid; i < nused; i += blockDim.x) {
-        const int gidx = __ldcg(P.slotlist + i), r = trk_find(P.parent, gidx);
+        const int gidx = __ldcg(TRK_SCR(P.slotlist) + i), r = trk_find(TRK_SCR(P.parent), gidx);
         if (r == gidx) continue;
-        const int4 b = __ldcg(P.bbox + gidx);
-        int *rb = reinterpret_cast<int *>(P.bbox + r);
+        const int4 b = __ldcg(TRK_SCR(P.bbox) + gidx);
+        int *rb = reinterpret_cast<int *>(TRK_SCR(P.bbox) + r);
         atomicMin(rb + 0, b.x); atomicMin(rb + 1, b.y); atomicMax(rb + 2, b.z); atomicMax(rb + 3, b.w);
-        const int sd = __ldcg(P.bseed + gidx);
-        if (sd != TRK_NONE) atomicMin(P.bseed + r, sd);
+        const int sd = __ldcg(TRK_SCR(P.bseed) + gidx);
+        if (sd != TRK_NONE) atomicMin(TRK_SCR(P.bseed) + r, sd);
     }
     __syncthreads();
     for (int i = tid; i < nused; i += blockDim.x) {
-        const int gidx = __ldcg(P.slotlist + i);
-        if (((volatile int *)P.parent)[gidx] != gidx) continue;
-        const int sd = ((volatile int *)P.bseed)[gidx];
+        const int gidx = __ldcg(TRK_SCR(P.slotlist) + i);
+        if (((volatile int *)TRK_SCR(P.parent))[gidx] != gidx) continue;
+        const int sd = ((volatile int *)TRK_SCR(P.bseed))[gidx];
         if (sd == TRK_NONE) continue;
-        const int pos = atomicAdd(&P.counters[0], 1);
+        const int pos = atomicAdd(&TRK_SCR(P.counters)[0], 1);
         if (pos < TRK_MAX_COMPONENTS) {
-            const volatile int *b = reinterpret_cast<volatile int *>(P.bbox + gidx);
-            P.keys[pos] = sd;
-            P.rects[pos] = make_int4(b[0], b[1], b[2] - b[0] + 1, b[3] - b[1] + 1);
+            const volatile int *b = reinterpret_cast<volatile int *>(TRK_SCR(P.bbox) + gidx);
+            TRK_SCR(P.keys)[pos] = sd;
+            TRK_SCR(P.rects)[pos] = make_int4(b[0], b[1], b[2] - b[0] + 1, b[3] - b[1] + 1);
         }
     }
     __syncthreads();
-    const int total = ((volatile int *)P.counters)[0], n = min(total, TRK_MAX_COMPONENTS);
+    const int total = ((volatile int *)TRK_SCR(P.counters))[0], n = min(total, TRK_MAX_COMPONENTS);
     // rank by first seed pixel (keys are distinct); up to a tile's worth of keys is ranked out of shared memory
     const bool in_smem = n <= TRK_NPX;
     if (in_smem) {
-        for (int i = tid; i < n; i += blockDim.x) s_lab[i] = __ldcg(P.keys + i);
+        for (int i = tid; i < n; i += blockDim.x) s_lab[i] = __ldcg(TRK_SCR(P.keys) + i);
         __syncthreads();
     }
     for (int i = tid; i < n; i += blockDim.x) {
-        const int key = in_smem ? s_lab[i] : __ldcg(P.keys + i);
+        const int key = in_smem ? s_lab[i] : __ldcg(TRK_SCR(P.keys) + i);
         int rank = 0;
         if (in_smem) for (int j = 0; j < n; j++) rank += s_lab[j] < key;
-        else for (int j = 0; j < n; j++) rank += __ldcg(P.keys + j) < key;
-        const int4 r = __ldcg(P.rects + i);
-        P.out[1 + rank] = r;
-        if (P.hout && rank < 1024) P.hout[1 + rank] = r;
+        else for (int j = 0; j < n; j++) rank += __ldcg(TRK_SCR(P.keys) + j) < key;
+        const int4 r = __ldcg(TRK_SCR(P.rects) + i);
+        TRK_SCR(P.out)[1 + rank] = r;
+        if (TRK_RES(P.hout) && rank < 1024) TRK_RES(P.hout)[1 + rank] = r;
     }
     if (tid == 0) {
-        P.out[0] = make_int4(total, 0, 0, 0);
-        if (P.hout) P.hout[0] = make_int4(total, 0, 0, 0);
-        P.counters[0] = 0; P.counters[1] = 0; P.counters[2] = 0;
+        TRK_SCR(P.out)[0] = make_int4(total, 0, 0, 0);
+        if (TRK_RES(P.hout)) TRK_RES(P.hout)[0] = make_int4(total, 0, 0, 0);
+        TRK_SCR(P.counters)[0] = 0; TRK_SCR(P.counters)[1] = 0; TRK_SCR(P.counters)[2] = 0;
     }
     TRK_T(10);
+#undef TRK_IMG
+#undef TRK_SRC
 }
 
 size_t tracker_scratch_bytes(int w, int h, TrkLayout *lo)
@@ -485,30 +522,60 @@ size_t tracker_scratch_bytes(int w, int h, TrkLayout *lo)
     return o;
 }
 
-cudaError_t launch_tracker(nv_ctx *ctx, int fmt, const SrcPlanes &src, int w, int h, int first, int thr, int cur, const float *val256,
-                           int *nlaunch)
+// the scratch pointers of TrkParams inside one image's scratch (tracker_scratch_bytes)
+static void trk_scratch_params(TrkParams &P, const TrkLayout &lo, uint8_t *base)
 {
-    const TrkLayout &lo = ctx->trk_lo;
-    uint8_t *base = ctx->d_trk_scratch;
-    TrkParams P;
-    P.src = src; P.w = w; P.h = h; P.first = first; P.thr = thr; P.cur = cur; P.ntx = lo.ntx; P.nty = lo.nty;
-    P.vec = fmt == NV_FMT_BGR && (w % 4) == 0 && (src.s0 % 16) == 0 && ((uintptr_t)src.p0 % 16) == 0;
-    P.prev = ctx->d_trk_prev; P.hist = ctx->d_trk_hist;
+    P.ntx = lo.ntx; P.nty = lo.nty;
     P.bslot = reinterpret_cast<unsigned short *>(base + lo.bslot); P.bcount = reinterpret_cast<int *>(base + lo.bcount);
     P.bbox = reinterpret_cast<int4 *>(base + lo.bbox); P.bseed = reinterpret_cast<int *>(base + lo.bseed);
     P.slotlist = reinterpret_cast<int *>(base + lo.slotlist);
     P.parent = reinterpret_cast<int *>(base + lo.parent); P.edge_flag = reinterpret_cast<int *>(base + lo.edge_flag);
     P.counters = reinterpret_cast<int *>(base + lo.counters); P.keys = reinterpret_cast<int *>(base + lo.keys);
     P.rects = reinterpret_cast<int4 *>(base + lo.rects); P.out = reinterpret_cast<int4 *>(base + lo.out);
+}
+
+cudaError_t launch_tracker(nv_ctx *ctx, int fmt, const SrcPlanes &src, int w, int h, int first, int thr, int cur, const float *val256,
+                           int *nlaunch)
+{
+    const TrkLayout &lo = ctx->trk_lo;
+    TrkParams P;
+    P.src = src; P.w = w; P.h = h; P.first = first; P.thr = thr; P.cur = cur;
+    P.vec = fmt == NV_FMT_BGR && (w % 4) == 0 && (src.s0 % 16) == 0 && ((uintptr_t)src.p0 % 16) == 0;
+    P.prev = ctx->d_trk_prev; P.hist = ctx->d_trk_hist;
+    trk_scratch_params(P, lo, ctx->d_trk_scratch);
     P.hout = reinterpret_cast<int4 *>(ctx->h_trk);
     for (int i = 0; i < 256; i++) P.val[i] = val256[i];
+    P.imgs = nullptr; P.slot_stride = P.scratch_stride = 0;
     const int nt = lo.ntx * lo.nty;
     cudaStream_t st = ctx->stream;
-    if (fmt == NV_FMT_BGR) k_trk_fused<0><<<nt, 256, 0, st>>>(P);               // interleaved: BGRA here
-    else if (fmt == NV_FMT_I420) k_trk_fused<1><<<nt, 256, 0, st>>>(P);
-    else if (fmt == NV_FMT_NV12) k_trk_fused<2><<<nt, 256, 0, st>>>(P);
-    else if (fmt == NV_FMT_NV21) k_trk_fused<3><<<nt, 256, 0, st>>>(P);
+    if (fmt == NV_FMT_BGR) k_trk_fused<0, false><<<nt, 256, 0, st>>>(P);               // interleaved: BGRA here
+    else if (fmt == NV_FMT_I420) k_trk_fused<1, false><<<nt, 256, 0, st>>>(P);
+    else if (fmt == NV_FMT_NV12) k_trk_fused<2, false><<<nt, 256, 0, st>>>(P);
+    else if (fmt == NV_FMT_NV21) k_trk_fused<3, false><<<nt, 256, 0, st>>>(P);
     else return cudaErrorInvalidValue;
     (*nlaunch)++;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_tracker_batch(int fmt, const SrcPlanes &strides, const TrkBatchImage *d_imgs, const uint8_t *const *h_planes, int n,
+                                 int w, int h, const TrkLayout &lo, uint8_t *prev, uint8_t *hist, size_t slot_stride, uint8_t *scratch,
+                                 size_t scratch_stride, void *hout, cudaStream_t st)
+{
+    TrkParams P;
+    memset(&P, 0, sizeof P);
+    P.src = strides; P.w = w; P.h = h;
+    // the 128-bit loads only when every image qualifies (the rule of launch_tracker)
+    P.vec = fmt == NV_FMT_BGR && (w % 4) == 0 && (strides.s0 % 16) == 0;
+    for (int i = 0; i < n && P.vec; i++) P.vec = ((uintptr_t)h_planes[3 * i] % 16) == 0;
+    P.prev = prev; P.hist = hist;
+    trk_scratch_params(P, lo, scratch);
+    P.hout = reinterpret_cast<int4 *>(hout);
+    P.imgs = d_imgs; P.slot_stride = slot_stride; P.scratch_stride = scratch_stride;
+    const dim3 grid(lo.ntx * lo.nty, n);
+    if (fmt == NV_FMT_BGR) k_trk_fused<0, true><<<grid, 256, 0, st>>>(P);
+    else if (fmt == NV_FMT_I420) k_trk_fused<1, true><<<grid, 256, 0, st>>>(P);
+    else if (fmt == NV_FMT_NV12) k_trk_fused<2, true><<<grid, 256, 0, st>>>(P);
+    else if (fmt == NV_FMT_NV21) k_trk_fused<3, true><<<grid, 256, 0, st>>>(P);
+    else return cudaErrorInvalidValue;
     return cudaGetLastError();
 }

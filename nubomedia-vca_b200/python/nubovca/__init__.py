@@ -155,6 +155,11 @@ _SIGS = {
     "nv_face_detect_batch": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, C.POINTER(FaceParams), _vp, _i, _ip, _ip]),
     "nv_face_submit_batch_yuv": (_i, [_vp, _vp, C.POINTER(YuvFrame), _i, C.POINTER(FaceParams)]),
     "nv_face_detect_batch_yuv": (_i, [_vp, _vp, C.POINTER(YuvFrame), _i, C.POINTER(FaceParams), _vp, _i, _ip, _ip]),
+    "nv_tracker_process_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, C.POINTER(C.c_double), C.POINTER(TrackerParams), _vp, _i, _ip,
+                                      _ip]),
+    "nv_tracker_process_batch_yuv": (_i, [_vp, C.POINTER(YuvFrame), _i, C.POINTER(C.c_double), C.POINTER(TrackerParams), _vp, _i,
+                                          _ip, _ip]),
+    "nv_tracker_reset_batch": (_i, [_vp, _i]),
 }
 BATCH_MAX = 256           # NV_BATCH_MAX
 EXPORTS = sorted(_SIGS)
@@ -196,19 +201,19 @@ def _rects(buf, n):
 
 def _batch_frames(images, cn):
     """(pointer table, n, w, h, row stride, on_device, keep-alive) of a batch: a uint8 numpy array or CUDA torch tensor
-    [N, H, W] (cn == 1) / [N, H, W, 3] (cn == 3) whose pixels are packed within a row; rows and images may be further
-    apart than packed.  A torch tensor's stream is synchronised here, so the library reads finished frames."""
+    [N, H, W] (cn == 1) / [N, H, W, cn] (cn == 3: BGR, 4: BGRA) whose pixels are packed within a row; rows and images may
+    be further apart than packed.  A torch tensor's stream is synchronised here, so the library reads finished frames."""
     ndim = 3 if cn == 1 else 4
     if type(images).__module__.startswith("torch"):
         import torch
         if images.dtype != torch.uint8:
             raise TypeError(f"batch must be a uint8 tensor, got {images.dtype}")
-        if images.dim() != ndim or (cn == 3 and images.shape[3] != 3):
-            raise ValueError(f"batch tensor must be [N, H, W{', 3' if cn == 3 else ''}], got {tuple(images.shape)}")
+        if images.dim() != ndim or (cn > 1 and images.shape[3] != cn):
+            raise ValueError(f"batch tensor must be [N, H, W{f', {cn}' if cn > 1 else ''}], got {tuple(images.shape)}")
         if not images.is_cuda:
             images = images.numpy()
         else:
-            if images.stride(2) != cn or (cn == 3 and images.stride(3) != 1):
+            if images.stride(2) != cn or (cn > 1 and images.stride(3) != 1):
                 raise ValueError("the pixels of a row must be packed (stride(2) == channels)")
             n, h, w = images.shape[:3]
             torch.cuda.current_stream(images.device).synchronize()
@@ -218,9 +223,9 @@ def _batch_frames(images, cn):
     if not isinstance(images, np.ndarray) or images.dtype != np.uint8:
         raise TypeError("batch must be a uint8 numpy array or a CUDA torch tensor")
     shape, strides = images.shape, images.strides
-    if len(shape) != ndim or (cn == 3 and shape[3] != 3):
-        raise ValueError(f"batch array must be [N, H, W{', 3' if cn == 3 else ''}], got {shape}")
-    if strides[2] != cn or (cn == 3 and strides[3] != 1) or min(strides) < 0:
+    if len(shape) != ndim or (cn > 1 and shape[3] != cn):
+        raise ValueError(f"batch array must be [N, H, W{f', {cn}' if cn > 1 else ''}], got {shape}")
+    if strides[2] != cn or (cn > 1 and strides[3] != 1) or min(strides) < 0:
         images = np.ascontiguousarray(images)
         strides = images.strides
     n, h, w = shape[:3]
@@ -712,6 +717,46 @@ class Context:
         the BGR(A) frame at device address d_ptr (nv_draw_shapes_device)."""
         _check(_lib.nv_draw_shapes_device(self.handle, C.c_void_p(d_ptr), w, h, stride, channels, _shape_array(shapes), len(shapes)),
                "nv_draw_shapes_device")
+
+    # ---- batched tracker: slot i of this context takes frame i (see nv_tracker_process_batch).  ts_ms: N timestamps; each
+    #      parameter a scalar for every slot or a sequence of N.  Returns a list of N int32 arrays [k, 4], slot by slot.
+    @staticmethod
+    def _tracker_batch_args(n, ts_ms, threshold, min_area, max_area, distance):
+        ts = [float(t) for t in ts_ms]
+        if len(ts) != n:
+            raise ValueError(f"{len(ts)} timestamps for a batch of {n}")
+        cols = []
+        for name, v in (("threshold", threshold), ("min_area", min_area), ("max_area", max_area), ("distance", distance)):
+            v = [int(x) for x in v] if np.ndim(v) else [int(v)] * n
+            if len(v) != n:
+                raise ValueError(f"{name}: {len(v)} values for a batch of {n}")
+            cols.append(v)
+        params = (TrackerParams * max(n, 1))(*[TrackerParams(*p) for p in zip(*cols)])
+        return (C.c_double * max(n, 1))(*ts), params
+
+    def _tracker_batch_call(self, fn, where, n, args):
+        if not hasattr(self, "_bout"):
+            self._bout = (Rect * (1 << 20))()
+        counts, total = (C.c_int * max(n, 1))(), C.c_int(0)      # not _bcounts: a pending face batch collects into those
+        _check(fn(self.handle, *args, self._bout, len(self._bout), counts, C.byref(total)), where)
+        return self._batch_out(counts[:n])
+
+    def tracker_process_batch(self, frames, ts_ms, threshold=20, min_area=50, max_area=30000, distance=35):
+        """frames: a uint8 numpy array or CUDA torch tensor [N, H, W, 4] of BGRA frames (a tensor's stream is synchronised)."""
+        ptrs, n, w, h, stride, dev, keep = _batch_frames(frames, 4)
+        ts, params = self._tracker_batch_args(n, ts_ms, threshold, min_area, max_area, distance)
+        return self._tracker_batch_call(_lib.nv_tracker_process_batch, "nv_tracker_process_batch", n,
+                                        (ptrs, n, w, h, stride, dev, ts, params))
+
+    def tracker_process_batch_yuv(self, frames, fmt, ts_ms, threshold=20, min_area=50, max_area=30000, distance=35):
+        """frames: [N, H*3/2, W] packed 4:2:0 buffers, as face_detect_batch_yuv takes them."""
+        table, n, keep = _batch_yuv_frames(frames, fmt)
+        ts, params = self._tracker_batch_args(n, ts_ms, threshold, min_area, max_area, distance)
+        return self._tracker_batch_call(_lib.nv_tracker_process_batch_yuv, "nv_tracker_process_batch_yuv", n, (table, n, ts, params))
+
+    def tracker_reset_batch(self, slot=-1):
+        """Clears one slot of the batched tracker; slot < 0: every slot."""
+        _check(_lib.nv_tracker_reset_batch(self.handle, int(slot)), "nv_tracker_reset_batch")
 
     def tracker_kernel_ms(self):
         ms = C.c_float(0)
